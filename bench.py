@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """bench.py -- log-mel clips/s (5 s @ 16 kHz, 128 mels) on N B200s, with roofline and CPU baseline.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl b200|reference] [--dump-outputs DIR]
 
 Workload (BASELINE.json configs[1]): a batch of 4096 synthetic 5 s clips per GPU
 (fp32, N(0, 0.1^2), 1.31 GB -- larger than the 126 MB L2, so no L2 flush is needed between
@@ -21,6 +21,10 @@ the run EXITS NON-ZERO on a mismatch: the driver's scaling run is parity evidenc
 
 `--impl reference` times the reference's CPU implementation of the same path (the torchaudio
 glue in oracle/torchaudio_port.py, all host threads) on a bounded sample of the same workload.
+
+`--dump-outputs DIR` writes, after the timed steps, the features of rank 0's last timed step as DIR/features.npy:
+float32 [512, 1, 128, 157], the clips at a fixed seeded sample of 512 of the 4096 indices in ascending order (41 MB).
+The input clips are seeded too, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -40,6 +44,7 @@ UNIT = "clips/s"
 CFG = dict(sample_rate=16000, n_mels=128, n_fft=2048, hop_length=512, duration=5.0)
 T_LEN = 80000
 BATCH = 4096
+DUMP_CLIPS, DUMP_SEED = 512, 0   # --dump-outputs: 512 of the 4096 clips' features, 41 MB of float32
 FALLBACK_HBM_GBS = 6650.0   # /opt/skills/guides/B200_PROFILING.md fallback
 
 
@@ -160,6 +165,15 @@ def profiled_traffic():
             return json.load(f).get("dram_bytes_per_launch_b4096")
     except Exception:
         return None
+
+
+def dump_outputs(out, path: str) -> None:
+    """Writes the features of DUMP_CLIPS clips of `out` (sorted indices drawn with DUMP_SEED) to path/features.npy."""
+    import numpy as np
+    import torch
+    idx = np.sort(np.random.default_rng(DUMP_SEED).choice(out.shape[0], DUMP_CLIPS, replace=False))
+    os.makedirs(path, exist_ok=True)
+    np.save(os.path.join(path, "features.npy"), out[torch.from_numpy(idx).to(out.device)].cpu().numpy())
 
 
 def cpu_baseline(budget_s: float = 16.0) -> dict:
@@ -523,6 +537,8 @@ def run_b200(args) -> None:
     ms_per_step = ms_max / args.steps
     value = world * BATCH * args.steps / (ms_max * 1e-3)
     checksum = float(out.double().abs().mean().item())   # device->host read of the result
+    if args.dump_outputs and rank == 0:
+        dump_outputs(out, args.dump_outputs)
 
     # ---- end to end through the host API: pinned host buffers in, host features out ----------
     host_in = clips.cpu().pin_memory()
@@ -662,7 +678,13 @@ def main() -> None:
     ap.add_argument("--impl", default="b200", choices=["b200", "reference"])
     ap.add_argument("--headline-only", action="store_true",
                     help="skip the other BASELINE configs and the CPU baseline (short runs under ncu)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write a seeded 512-clip sample of the last timed step's features to DIR/features.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the features of the b200 path; the reference timing keeps none")
     if args.impl == "reference":
         run_reference(args)
     else:

@@ -1,5 +1,5 @@
-"""Multi-GPU checks that need more than one B200 (skipped on a single-GPU box): run with
-`gpurun --gpus 2 -- python -m pytest tests/test_gpu_multi.py -m gpu`."""
+"""Multi-GPU checks that need more than one B200 (skipped on a single-GPU machine): run with
+`python -m pytest tests/test_gpu_multi.py -m gpu` on a machine with two or more B200s."""
 import os
 import subprocess
 import sys
