@@ -4,7 +4,7 @@
 Every index and twiddle is a compile-time literal, so nvcc keeps whole arrays in registers.
 Three flavours of the same forward transform (sign e^{-2 pi i nk/N}), natural order in and out:
 
-  lm_fft{16,32}(float xr[N], float xi[N])
+  lm_fft{8,16,32}(float xr[N], float xi[N])
       scalar reference flavour (used by the CPU tests and as documentation of the op count).
 
   lm_fft32_aos(lm_f2 z[32])
@@ -21,6 +21,11 @@ Three flavours of the same forward transform (sign e^{-2 pi i nk/N}), natural or
       32x32 transpose deliver.  In DIT order those two points share every twiddle of stages 1-4
       (they are the even- and odd-sample 16-point sub-transforms), so stages 1-4 run packed with
       broadcast constants; stage 5 combines the halves of each register in scalar code.
+
+  lm_fft16x2_soa / lm_fft8x4_soa(const lm_f2 pr[16], const lm_f2 pi[16], float xr[32], float xi[32])
+      the same layout cut into 2 independent 16-point or 4 independent 8-point transforms (the
+      second stage of the 512- and 256-point FFTs): transform b reads pr/pi[b n/2 ..] and writes
+      xr/xi[b n ..]; all stages but the last run packed.
 
 Non-trivial butterflies use the 6-FMA (3 packed) Linzer-Feig form with the tangent
 (|c| >= |s|) or cotangent (|c| < |s|) ratio so that |ratio| <= 1:
@@ -148,73 +153,80 @@ def gen_aos(n: int, first_stage: int = 1) -> str:
 
 
 # --------------------------------------------------------------------------------------
-def gen_soa32() -> str:
-    """Stages 1-4 on (even-sample, odd-sample) register pairs, stage 5 scalar."""
+def gen_soa(n: int = 32) -> str:
+    """32 // n independent n-point transforms of the 32 points one lane holds after the transpose:
+    transform b reads pr/pi[b n/2 .. b n/2 + n/2 - 1] and writes xr/xi[b n .. b n + n - 1].
+    Stages 1 .. log2(n)-1 on (even-sample, odd-sample) register pairs, the last stage scalar."""
+    count, h = 32 // n, n // 2
+    hbits = h.bit_length() - 1
+    name = "lm_fft32_soa" if n == 32 else f"lm_fft{n}x{count}_soa"
     out, ops2, ops1, tmp = [], 0, 0, 0
     emit = out.append
-    emit("LM_HD LM_INLINE void lm_fft32_soa(const lm_f2 (&pr)[16], const lm_f2 (&pi)[16], "
+    emit(f"LM_HD LM_INLINE void {name}(const lm_f2 (&pr)[16], const lm_f2 (&pi)[16], "
          "float (&xr)[32], float (&xi)[32]) {")
-    # DIT-16 array A[i] = P[bitrev4(i)], each entry a (re pair, im pair)
-    cur = [(f"pr[{bitrev(i, 4)}]", f"pi[{bitrev(i, 4)}]") for i in range(16)]
-    for s in range(1, 5):
-        m, half = 1 << s, 1 << (s - 1)
-        for k in range(0, 16, m):
-            for j in range(half):
-                ia, ib = k + j, k + j + half
-                (ar, ai), (br, bi) = cur[ia], cur[ib]
-                p = f"s{tmp}"
-                tmp += 1
-                kind, c, sn, t = twiddle_kind(j, m)
-                if kind == "one":
-                    emit(f"  const lm_f2 {p}ar = lm_add2({ar}, {br}), {p}ai = lm_add2({ai}, {bi});")
-                    emit(f"  const lm_f2 {p}br = lm_sub2({ar}, {br}), {p}bi = lm_sub2({ai}, {bi});")
-                    ops2 += 4
-                elif kind == "mi":
-                    emit(f"  const lm_f2 {p}ar = lm_add2({ar}, {bi}), {p}ai = lm_sub2({ai}, {br});")
-                    emit(f"  const lm_f2 {p}br = lm_sub2({ar}, {bi}), {p}bi = lm_add2({ai}, {br});")
-                    ops2 += 4
-                elif kind == "tan":
-                    emit(f"  const lm_f2 {p}ur = lm_fma2(lm_bcast({lit(t)}), {bi}, {br}), "
-                         f"{p}ui = lm_fma2(lm_bcast({lit(-t)}), {br}, {bi});")
-                    emit(f"  const lm_f2 {p}ar = lm_fma2(lm_bcast({lit(c)}), {p}ur, {ar}), "
-                         f"{p}ai = lm_fma2(lm_bcast({lit(c)}), {p}ui, {ai});")
-                    emit(f"  const lm_f2 {p}br = lm_fma2(lm_bcast({lit(-c)}), {p}ur, {ar}), "
-                         f"{p}bi = lm_fma2(lm_bcast({lit(-c)}), {p}ui, {ai});")
-                    ops2 += 6
-                else:
-                    emit(f"  const lm_f2 {p}ur = lm_fma2(lm_bcast({lit(-t)}), {bi}, {br}), "
-                         f"{p}ui = lm_fma2(lm_bcast({lit(t)}), {br}, {bi});")
-                    emit(f"  const lm_f2 {p}ar = lm_fma2(lm_bcast({lit(sn)}), {p}ui, {ar}), "
-                         f"{p}ai = lm_fma2(lm_bcast({lit(-sn)}), {p}ur, {ai});")
-                    emit(f"  const lm_f2 {p}br = lm_fma2(lm_bcast({lit(-sn)}), {p}ui, {ar}), "
-                         f"{p}bi = lm_fma2(lm_bcast({lit(sn)}), {p}ur, {ai});")
-                    ops2 += 6
-                cur[ia] = (f"{p}ar", f"{p}ai")
-                cur[ib] = (f"{p}br", f"{p}bi")
-    # stage 5: X[i] = E[i] + w32^i O[i], X[i+16] = E[i] - w32^i O[i]; E = lo halves, O = hi halves
-    for i in range(16):
-        R, I = cur[i]
-        ar, ai, br, bi = f"lm_lo({R})", f"lm_lo({I})", f"lm_hi({R})", f"lm_hi({I})"
-        kind, c, sn, t = twiddle_kind(i, 32)
-        p = f"f{i}"
-        if kind == "one":
-            emit(f"  xr[{i}] = {ar} + {br}; xi[{i}] = {ai} + {bi}; xr[{i + 16}] = {ar} - {br}; xi[{i + 16}] = {ai} - {bi};")
-            ops1 += 4
-        elif kind == "mi":
-            emit(f"  xr[{i}] = {ar} + {bi}; xi[{i}] = {ai} - {br}; xr[{i + 16}] = {ar} - {bi}; xi[{i + 16}] = {ai} + {br};")
-            ops1 += 4
-        elif kind == "tan":
-            emit(f"  const float {p}ur = fmaf({lit(t)}, {bi}, {br}), {p}ui = fmaf({lit(-t)}, {br}, {bi});")
-            emit(f"  xr[{i}] = fmaf({lit(c)}, {p}ur, {ar}); xi[{i}] = fmaf({lit(c)}, {p}ui, {ai}); "
-                 f"xr[{i + 16}] = fmaf({lit(-c)}, {p}ur, {ar}); xi[{i + 16}] = fmaf({lit(-c)}, {p}ui, {ai});")
-            ops1 += 6
-        else:
-            emit(f"  const float {p}ur = fmaf({lit(-t)}, {bi}, {br}), {p}ui = fmaf({lit(t)}, {br}, {bi});")
-            emit(f"  xr[{i}] = fmaf({lit(sn)}, {p}ui, {ar}); xi[{i}] = fmaf({lit(-sn)}, {p}ur, {ai}); "
-                 f"xr[{i + 16}] = fmaf({lit(-sn)}, {p}ui, {ar}); xi[{i + 16}] = fmaf({lit(sn)}, {p}ur, {ai});")
-            ops1 += 6
+    for b in range(count):
+        # DIT-(n/2) array A[i] = P[bitrev(i)], each entry a (re pair, im pair)
+        cur = [(f"pr[{b * h + bitrev(i, hbits)}]", f"pi[{b * h + bitrev(i, hbits)}]") for i in range(h)]
+        for s in range(1, hbits + 1):
+            m, half = 1 << s, 1 << (s - 1)
+            for k in range(0, h, m):
+                for j in range(half):
+                    ia, ib = k + j, k + j + half
+                    (ar, ai), (br, bi) = cur[ia], cur[ib]
+                    p = f"s{tmp}"
+                    tmp += 1
+                    kind, c, sn, t = twiddle_kind(j, m)
+                    if kind == "one":
+                        emit(f"  const lm_f2 {p}ar = lm_add2({ar}, {br}), {p}ai = lm_add2({ai}, {bi});")
+                        emit(f"  const lm_f2 {p}br = lm_sub2({ar}, {br}), {p}bi = lm_sub2({ai}, {bi});")
+                        ops2 += 4
+                    elif kind == "mi":
+                        emit(f"  const lm_f2 {p}ar = lm_add2({ar}, {bi}), {p}ai = lm_sub2({ai}, {br});")
+                        emit(f"  const lm_f2 {p}br = lm_sub2({ar}, {bi}), {p}bi = lm_add2({ai}, {br});")
+                        ops2 += 4
+                    elif kind == "tan":
+                        emit(f"  const lm_f2 {p}ur = lm_fma2(lm_bcast({lit(t)}), {bi}, {br}), "
+                             f"{p}ui = lm_fma2(lm_bcast({lit(-t)}), {br}, {bi});")
+                        emit(f"  const lm_f2 {p}ar = lm_fma2(lm_bcast({lit(c)}), {p}ur, {ar}), "
+                             f"{p}ai = lm_fma2(lm_bcast({lit(c)}), {p}ui, {ai});")
+                        emit(f"  const lm_f2 {p}br = lm_fma2(lm_bcast({lit(-c)}), {p}ur, {ar}), "
+                             f"{p}bi = lm_fma2(lm_bcast({lit(-c)}), {p}ui, {ai});")
+                        ops2 += 6
+                    else:
+                        emit(f"  const lm_f2 {p}ur = lm_fma2(lm_bcast({lit(-t)}), {bi}, {br}), "
+                             f"{p}ui = lm_fma2(lm_bcast({lit(t)}), {br}, {bi});")
+                        emit(f"  const lm_f2 {p}ar = lm_fma2(lm_bcast({lit(sn)}), {p}ui, {ar}), "
+                             f"{p}ai = lm_fma2(lm_bcast({lit(-sn)}), {p}ur, {ai});")
+                        emit(f"  const lm_f2 {p}br = lm_fma2(lm_bcast({lit(-sn)}), {p}ui, {ar}), "
+                             f"{p}bi = lm_fma2(lm_bcast({lit(sn)}), {p}ur, {ai});")
+                        ops2 += 6
+                    cur[ia] = (f"{p}ar", f"{p}ai")
+                    cur[ib] = (f"{p}br", f"{p}bi")
+        # last stage: X[i] = E[i] + wn^i O[i], X[i+n/2] = E[i] - wn^i O[i]; E = lo halves, O = hi halves
+        for i in range(h):
+            R, I = cur[i]
+            ar, ai, br, bi = f"lm_lo({R})", f"lm_lo({I})", f"lm_hi({R})", f"lm_hi({I})"
+            kind, c, sn, t = twiddle_kind(i, n)
+            p = f"f{i}" if count == 1 else f"f{b}_{i}"
+            lo, hi = b * n + i, b * n + i + h
+            if kind == "one":
+                emit(f"  xr[{lo}] = {ar} + {br}; xi[{lo}] = {ai} + {bi}; xr[{hi}] = {ar} - {br}; xi[{hi}] = {ai} - {bi};")
+                ops1 += 4
+            elif kind == "mi":
+                emit(f"  xr[{lo}] = {ar} + {bi}; xi[{lo}] = {ai} - {br}; xr[{hi}] = {ar} - {bi}; xi[{hi}] = {ai} + {br};")
+                ops1 += 4
+            elif kind == "tan":
+                emit(f"  const float {p}ur = fmaf({lit(t)}, {bi}, {br}), {p}ui = fmaf({lit(-t)}, {br}, {bi});")
+                emit(f"  xr[{lo}] = fmaf({lit(c)}, {p}ur, {ar}); xi[{lo}] = fmaf({lit(c)}, {p}ui, {ai}); "
+                     f"xr[{hi}] = fmaf({lit(-c)}, {p}ur, {ar}); xi[{hi}] = fmaf({lit(-c)}, {p}ui, {ai});")
+                ops1 += 6
+            else:
+                emit(f"  const float {p}ur = fmaf({lit(-t)}, {bi}, {br}), {p}ui = fmaf({lit(t)}, {br}, {bi});")
+                emit(f"  xr[{lo}] = fmaf({lit(sn)}, {p}ui, {ar}); xi[{lo}] = fmaf({lit(-sn)}, {p}ur, {ai}); "
+                     f"xr[{hi}] = fmaf({lit(-sn)}, {p}ui, {ar}); xi[{hi}] = fmaf({lit(sn)}, {p}ur, {ai});")
+                ops1 += 6
     emit("}")
-    emit(f"// lm_fft32_soa: {ops2} packed f32x2 ops + {ops1} scalar ops")
+    emit(f"// {name}: {ops2} packed f32x2 ops + {ops1} scalar ops")
     return "\n".join(out)
 
 
@@ -222,15 +234,16 @@ def main() -> None:
     print("// GENERATED by gen_fft.py -- do not edit.  Register-resident forward FFTs.")
     print("#pragma once")
     print('#include "lm_f2.cuh"')
-    for n in (16, 32):
+    for n in (8, 16, 32):
         print()
         print(gen_scalar(n))
     print()
     print(gen_aos(32))
     print()
     print(gen_aos(32, first_stage=2))
-    print()
-    print(gen_soa32())
+    for n in (32, 16, 8):
+        print()
+        print(gen_soa(n))
 
 
 if __name__ == "__main__":

@@ -9,8 +9,10 @@
 
 #include <algorithm>
 #include <atomic>
+#include <map>
 #include <mutex>
 #include <new>
+#include <utility>
 #include <vector>
 
 #include <nvtx3/nvToolsExt.h>   // header-only NVTX v3: ranges are no-ops unless a profiler is attached
@@ -126,6 +128,40 @@ lm::KParams make_params(const lm_plan* p) {
     return k;
 }
 
+// Raises the dynamic shared-memory limit of every logmel_kernel instantiation a plan of this n_fft may launch.  The
+// limit belongs to the kernel on the current device, not to the plan, and plans of one n_fft with other hops or mel
+// counts need different sizes: it only ever grows, so creating a smaller plan cannot break launches of a larger one
+// made earlier.  The on-device-noise staging variant (FASTNOISE) exists for n_fft = 2048 only; the other sizes stage
+// Philox noise in the plain kernel.
+std::mutex g_smem_mu;
+std::map<std::pair<int, int>, size_t> g_smem_limit;   // (n_fft, device) -> limit set so far
+
+template <int NFFT>
+cudaError_t set_smem_limit(int device, size_t bytes) {
+    std::lock_guard<std::mutex> lock(g_smem_mu);
+    size_t& cur = g_smem_limit[std::make_pair(NFFT, device)];
+    if (bytes <= cur) return cudaSuccess;
+    const int b = static_cast<int>(bytes);
+    constexpr bool kFastNoise = (NFFT == 2048);
+    cudaError_t e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess && kFastNoise)
+        e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, false, kFastNoise>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess)
+        e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
+    if (e == cudaSuccess) cur = bytes;
+    return e;
+}
+
+template <int NFFT>
+void launch_kernel(const lm::KParams& k, int grid, size_t smem, cudaStream_t stream, bool pcm16, bool extra, bool device_noise) {
+    constexpr bool kFastNoise = (NFFT == 2048);
+    if (pcm16) lm::logmel_kernel<NFFT, false, false, true><<<grid, lm::kThreads, smem, stream>>>(k);
+    else if (extra) lm::logmel_kernel<NFFT, true><<<grid, lm::kThreads, smem, stream>>>(k);
+    else if (kFastNoise && device_noise) lm::logmel_kernel<NFFT, false, kFastNoise><<<grid, lm::kThreads, smem, stream>>>(k);
+    else lm::logmel_kernel<NFFT, false><<<grid, lm::kThreads, smem, stream>>>(k);
+}
+
 int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
            const lm_aug* aug, const float* noise, float* out_norm, float* out_db, float* out_melpow,
            int32_t normalize, cudaStream_t stream, float* const* peers = nullptr, int n_peers = 0,
@@ -166,17 +202,13 @@ int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* 
     const int grid = std::min<int>(B * k.split, cap);
     const bool extra = (out_db != nullptr) || (out_melpow != nullptr);
     const bool device_noise = (aug != nullptr) && (noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
-    if (pcm16) {   // `wave` holds 16-bit samples (lm_forward_pcm16): expanded inside the staging, no decode kernel
-        if (extra) return LM_ERR_UNSUPPORTED;
-        if (p->n_fft == 2048) lm::logmel_kernel<2048, false, false, true><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
-        else lm::logmel_kernel<1024, false, false, true><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
-    } else if (p->n_fft == 2048) {
-        if (extra) lm::logmel_kernel<2048, true><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
-        else if (device_noise) lm::logmel_kernel<2048, false, true><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
-        else lm::logmel_kernel<2048, false><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
-    } else {
-        if (extra) lm::logmel_kernel<1024, true><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
-        else lm::logmel_kernel<1024, false><<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
+    // pcm16: `wave` holds 16-bit samples (lm_forward_pcm16), expanded inside the staging, no decode kernel
+    if (pcm16 && extra) return LM_ERR_UNSUPPORTED;
+    switch (p->n_fft) {
+        case 2048: launch_kernel<2048>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
+        case 1024: launch_kernel<1024>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
+        case 512: launch_kernel<512>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
+        default: launch_kernel<256>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
     }
     LM_CUDA(cudaGetLastError());
     return LM_OK;
@@ -209,7 +241,7 @@ const char* lm_strerror(int status) {
     switch (status) {
         case LM_OK: return "ok";
         case LM_ERR_INVALID_ARG: return "invalid argument";
-        case LM_ERR_UNSUPPORTED: return "unsupported configuration (n_fft must be 1024 or 2048; hop even and <= n_fft/4; n_mels <= 256; window must be the periodic Hann window: w[n] + w[n + n_fft/2] = 1)";
+        case LM_ERR_UNSUPPORTED: return "unsupported configuration (n_fft must be 256, 512, 1024 or 2048; hop even and <= n_fft/4; n_mels <= 256; window must be the periodic Hann window: w[n] + w[n + n_fft/2] = 1)";
         case LM_ERR_FILTERBANK: return "filterbank support too wide for the on-chip table";
         case LM_ERR_CUDA: return "CUDA runtime error (see lm_last_cuda_error)";
         case LM_ERR_NO_DEVICE: return "no usable CUDA device (an sm_100 GPU is required; there is no CPU fallback)";
@@ -224,7 +256,7 @@ int lm_plan_create(const lm_config* cfg, int device, lm_plan** out_plan) {
     NvtxRange nvtx("lm_plan_create");
     if (!cfg || !out_plan || !cfg->window || !cfg->fb) return LM_ERR_INVALID_ARG;
     *out_plan = nullptr;
-    if (cfg->n_fft != 2048 && cfg->n_fft != 1024) return LM_ERR_UNSUPPORTED;
+    if (cfg->n_fft != 2048 && cfg->n_fft != 1024 && cfg->n_fft != 512 && cfg->n_fft != 256) return LM_ERR_UNSUPPORTED;
     if (cfg->hop < 2 || (cfg->hop & 1) || cfg->hop > cfg->n_fft / 4) return LM_ERR_UNSUPPORTED;
     if (cfg->n_mels < 1 || cfg->n_mels > 256) return LM_ERR_UNSUPPORTED;
     if (cfg->target_len <= cfg->n_fft / 2) return LM_ERR_TOO_SHORT;
@@ -251,7 +283,7 @@ int lm_plan_create(const lm_config* cfg, int device, lm_plan** out_plan) {
     p->n_fft = cfg->n_fft; p->hop = cfg->hop; p->n_mels = cfg->n_mels; p->T = cfg->target_len;
     p->n_freqs = cfg->n_fft / 2 + 1;
     p->frames = 1 + cfg->target_len / cfg->hop;
-    p->tile_f = (cfg->n_fft == 2048) ? lm::Geo<2048>::TILE_F : lm::Geo<1024>::TILE_F;
+    p->tile_f = lm::kGroupWarps * (2048 / cfg->n_fft);   // lm::Geo<n_fft>::TILE_F
     p->n_tiles = (p->frames + p->tile_f - 1) / p->tile_f;
     p->ns = (((p->tile_f - 1) * p->hop + p->n_fft) + 3) & ~3;
     p->db_mult = cfg->db_multiplier; p->amin = cfg->amin; p->db_offset = cfg->db_offset;
@@ -285,7 +317,9 @@ int lm_plan_create(const lm_config* cfg, int device, lm_plan** out_plan) {
         memcpy(&h, &u, 4);
         return h;
     };
-    const int row_cap = (p->n_fft == 2048) ? lm::kRowFloats : (lm::kRowFloats - lm::kPbOff);
+    // the band of the last frame of a warp row (at (FPW - 1) * OFF, lm::Geo) must end inside the row; bins past n_freqs
+    // that a padded band reads hold finite values (zeros, the next frame's spectrum, FFT scratch) and meet zero weights
+    const int fpw = 2048 / p->n_fft, row_cap = lm::kRowFloats - (fpw - 1) * (p->n_fft / 2 + 16);
     for (int mt = 0; mt < n_mt; ++mt) {
         int lo = -1, hi = -1;
         for (int k = 0; k < p->n_freqs; ++k)
@@ -333,13 +367,17 @@ int lm_plan_create(const lm_config* cfg, int device, lm_plan** out_plan) {
     }
 
     // ---- twiddles ---------------------------------------------------------------------------
+    // W_nc^(k1 n2) between the two FFT stages: nc = 1024 complex points for n_fft 2048 / 1024, nc = n_fft for the
+    // small sizes, where lane = s * (nc / 32) + n2 carries point n2 of sub-FFT s
     std::vector<float2> tw(32 * lm::kTwRows), utw(512);
     const double two_pi = 6.283185307179586476925286766559;
+    const int nc = std::min(p->n_fft, 1024);
     for (int r = 0; r < lm::kTwRows; ++r) {
         const int k1 = (lm::kTwRows == 31) ? r + 1 : (r < 3 ? r + 1 : 4 * (r - 2));   // 1..31, or 1, 2, 3, 4, 8, ..., 28
-        for (int n2 = 0; n2 < 32; ++n2) {
-            const double a = two_pi * static_cast<double>(k1 * n2) / 1024.0;
-            tw[r * 32 + n2] = make_float2(static_cast<float>(cos(a)), static_cast<float>(-sin(a)));
+        for (int lane = 0; lane < 32; ++lane) {
+            const int n2 = lane % (nc / 32);
+            const double a = two_pi * static_cast<double>(k1 * n2) / static_cast<double>(nc);
+            tw[r * 32 + lane] = make_float2(static_cast<float>(cos(a)), static_cast<float>(-sin(a)));
         }
     }
     for (int k = 0; k < 512; ++k) {
@@ -369,33 +407,18 @@ int lm_plan_create(const lm_config* cfg, int device, lm_plan** out_plan) {
 
     // ---- shared memory --------------------------------------------------------------------
     cudaError_t e;
-    {
-        const size_t want = (p->n_fft == 2048) ? lm::Smem<2048>::total(p->ns, p->n_dk) : lm::Smem<1024>::total(p->ns, p->n_dk);
-        if (want > prop.sharedMemPerBlockOptin) { free_plan(p); return LM_ERR_FILTERBANK; }
+    switch (p->n_fft) {
+        case 2048: p->smem_bytes = lm::Smem<2048>::total(p->ns, p->n_dk); break;
+        case 1024: p->smem_bytes = lm::Smem<1024>::total(p->ns, p->n_dk); break;
+        case 512: p->smem_bytes = lm::Smem<512>::total(p->ns, p->n_dk); break;
+        default: p->smem_bytes = lm::Smem<256>::total(p->ns, p->n_dk); break;
     }
-    if (p->n_fft == 2048) {
-        p->smem_bytes = lm::Smem<2048>::total(p->ns, p->n_dk);
-        e = cudaFuncSetAttribute(lm::logmel_kernel<2048, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 static_cast<int>(p->smem_bytes));
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(lm::logmel_kernel<2048, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     static_cast<int>(p->smem_bytes));
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(lm::logmel_kernel<2048, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     static_cast<int>(p->smem_bytes));
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(lm::logmel_kernel<2048, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     static_cast<int>(p->smem_bytes));
-    } else {
-        p->smem_bytes = lm::Smem<1024>::total(p->ns, p->n_dk);
-        e = cudaFuncSetAttribute(lm::logmel_kernel<1024, false>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                 static_cast<int>(p->smem_bytes));
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(lm::logmel_kernel<1024, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     static_cast<int>(p->smem_bytes));
-        if (e == cudaSuccess)
-            e = cudaFuncSetAttribute(lm::logmel_kernel<1024, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                     static_cast<int>(p->smem_bytes));
+    if (p->smem_bytes > prop.sharedMemPerBlockOptin) { free_plan(p); return LM_ERR_FILTERBANK; }
+    switch (p->n_fft) {
+        case 2048: e = set_smem_limit<2048>(device, p->smem_bytes); break;
+        case 1024: e = set_smem_limit<1024>(device, p->smem_bytes); break;
+        case 512: e = set_smem_limit<512>(device, p->smem_bytes); break;
+        default: e = set_smem_limit<256>(device, p->smem_bytes); break;
     }
     if (e != cudaSuccess) { free_plan(p); return cuda_fail(e, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)"); }
     *out_plan = p;

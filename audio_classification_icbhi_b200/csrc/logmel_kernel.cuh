@@ -9,7 +9,9 @@
 // CTA whose warps all sit in the same phase (DESIGN.md section 5: the relative phase of the groups
 // does not matter, `stagger_ns` is kept as an experiment knob only).
 //
-// A tile is 8 frames (16 for n_fft = 1024); one warp = one frame.  Per item, inside a group:
+// A tile is 8 frames (16 / 32 / 64 for n_fft = 1024 / 512 / 256); one warp = one frame at n_fft = 2048, two frames
+// packed as a + i b into one complex FFT at 1024, and 1024 / n_fft such FFTs side by side below (Geo).  Per item,
+// inside a group:
 //
 //   stage   (one item ahead, into the group's single buffer as soon as every warp has pulled its
 //           frame into registers) the tile's samples -> shared memory, once per sample although
@@ -309,9 +311,14 @@ __device__ __forceinline__ void warp_twiddle(lm_f2 (&z)[32], const float2* __res
         z[4 * a + 3] = cmul(z[4 * a + 3], cmul(A, B3));
     }
 }
-__device__ __forceinline__ void warp_cfft1024_part2(lm_f2 (&z)[32], float (&xr)[32], float (&xi)[32],
-                                                    float* __restrict__ scr, const float2* __restrict__ tw, int lane,
-                                                    bool do_twiddle = true) {
+// n_fft = 512 / 256 (R = 16 / 8): lane s R + n2 holds z_s[R n1 + n2] of sub-FFT s in z[n1].  Part 1 is the same
+// radix-32 FFT over n1; the twiddle is W_n_fft^(n2 k1) (the table is built per n_fft, the code is the same); after
+// the transpose lane k1 holds the R values n2 of each sub-FFT side by side, and the second stage is 32 / R
+// radix-R FFTs: lane k1 ends with Z_s[k1 + 32 k2] in (xr[s R + k2], xi[s R + k2]).
+template <int NFFT>
+__device__ __forceinline__ void warp_cfft_part2(lm_f2 (&z)[32], float (&xr)[32], float (&xi)[32],
+                                                float* __restrict__ scr, const float2* __restrict__ tw, int lane,
+                                                bool do_twiddle = true) {
     if (do_twiddle) warp_twiddle(z, tw, lane);
     lm_f2 pr[16], pi[16];
 #pragma unroll
@@ -334,7 +341,9 @@ __device__ __forceinline__ void warp_cfft1024_part2(lm_f2 (&z)[32], float (&xr)[
         pi[2 * q + 1] = lm_pack(v.z, v.w);
     }
     __syncwarp();
-    lm_fft32_soa(pr, pi, xr, xi);
+    if (NFFT == 512) lm_fft16x2_soa(pr, pi, xr, xi);
+    else if (NFFT == 256) lm_fft8x4_soa(pr, pi, xr, xi);
+    else lm_fft32_soa(pr, pi, xr, xi);
 }
 
 // The four normals of one Philox block: z[j] == philox_normal(seed, 4 * blk + j), bit for bit (same operations),
@@ -369,12 +378,22 @@ struct ClipCtx;
 // path and must not change the register allocation or the code layout of the kernel's main loop.
 __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restrict__ sb, int ns, int need, int j0, int T, int gtid);
 
+// n_fft = 2048: one real frame per warp (a 1024-point complex FFT of its even / odd samples).  n_fft <= 1024: the
+// warp's 1024 complex points are P = 1024 / n_fft independent n_fft-point FFTs, each carrying two real frames as
+// a + i b, so FPW = 2 P frames per warp.  Frame j of a warp leaves its power spectrum at j * OFF in the warp's row.
 template <int NFFT>
 struct Geo {
-    static constexpr int FPW = (NFFT == 2048) ? 1 : 2;   // frames per warp pass
+    static_assert(NFFT == 2048 || NFFT == 1024 || NFFT == 512 || NFFT == 256, "n_fft");
+    static constexpr int FPW = 2048 / NFFT;              // frames per warp pass
     static constexpr int TILE_F = kGroupWarps * FPW;     // frames per item
     static constexpr int NB = TILE_F / 8;                // 8-frame MMA column blocks per tile
+    // spectrum pitch inside a row: >= n_fft/2 + 1 bins, == 16 (mod 32) so that the two frames g, g+1 that one
+    // quarter-warp's LDS.128 B-operand loads touch sit 16 banks apart (1024: kPbOff, 512: 272, 256: 144)
+    static constexpr int OFF = NFFT / 2 + 16;
+    static constexpr int R = (NFFT >= 1024 ? 1024 : NFFT) / 32;   // points per lane of one complex FFT (second radix)
+    static_assert(OFF % 32 == 16 && (FPW - 1) * OFF + NFFT / 2 + 1 <= kRowFloats, "row layout");
 };
+static_assert(Geo<1024>::OFF == kPbOff, "n_fft = 1024 row layout");
 
 // Shared-memory carve-up, shared by host (size) and device (pointers).  Everything of fixed size
 // comes first so that its addresses are compile-time constants (no registers spent on pointers);
@@ -475,7 +494,7 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     // skipped (ICBHI cycles average 2.7 s of the 5 s target).  Silence is monotone in the tile index.
     int silent_from = p.n_tiles;
     if (LM_SILENT && c->plain) {
-        const int tile_f = (nfft == 2048) ? 8 : 16;
+        const int tile_f = kGroupWarps * (2048 / nfft);   // Geo<nfft>::TILE_F
         for (int t = p.n_tiles - 1; t >= 0; --t) {
             const int tf = t * tile_f;
             const int nf = (p.frames - tf) < tile_f ? (p.frames - tf) : tile_f;
@@ -498,6 +517,8 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
     using G = Geo<NFFT>;
     constexpr int TILE_F = G::TILE_F;
     constexpr int HALF = NFFT / 2;
+    constexpr int NBC = G::NB < 4 ? G::NB : 4;   // MMA column blocks per walk of a mel tile's band
+    constexpr int DUNROLL = G::NB > 2 ? 1 : 2;     // unroll of the band walk (n_fft <= 512: 4 blocks per step are enough)
 
     extern __shared__ __align__(128) unsigned char smem_raw[];
     using L = Smem<NFFT>;
@@ -768,7 +789,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                     z[r] = lm_fma2(lm_sub2(V1, V2), W, V2);
                     z[r + 16] = lm_fma2(lm_add2(V1, V2), W, lm_pack(-v2.x, -v2.y));
                 }
-            } else {
+            } else if (NFFT == 1024) {
                 // n_fft = 1024: two frames per warp as one complex signal z = a + i b
                 const float* __restrict__ sa = sb + (2 * gw) * hop;
                 const float* __restrict__ sbb = sa + hop;
@@ -777,6 +798,21 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                     const float a1 = sa[32 * r + lane], a2 = sa[32 * (r + 16) + lane];
                     const float b1 = sbb[32 * r + lane], b2 = sbb[32 * (r + 16) + lane];
                     const lm_f2 V1 = lm_pack(a1, b1), V2 = lm_pack(a2, b2), W = lm_bcast(s_win[32 * r + lane]);
+                    z[r] = lm_fma2(lm_sub2(V1, V2), W, V2);
+                    z[r + 16] = lm_fma2(lm_add2(V1, V2), W, lm_pack(-a2, -b2));
+                }
+            } else {
+                // n_fft = 512 / 256: sub-FFT s = lane / R of the warp carries frames 2s (re) and 2s + 1 (im); lane
+                // s R + n2 takes samples n = R n1 + n2, so z[r] and z[r + 16] are n and n + n_fft/2 as above
+                constexpr int R = G::R;
+                const int n2 = lane & (R - 1);
+                const float* __restrict__ sa = sb + (G::FPW * gw + 2 * (lane / R)) * hop + n2;
+                const float* __restrict__ sbb = sa + hop;
+#pragma unroll
+                for (int r = 0; r < 16; ++r) {
+                    const float a1 = sa[R * r], a2 = sa[R * (r + 16)];
+                    const float b1 = sbb[R * r], b2 = sbb[R * (r + 16)];
+                    const lm_f2 V1 = lm_pack(a1, b1), V2 = lm_pack(a2, b2), W = lm_bcast(s_win[R * r + n2]);
                     z[r] = lm_fma2(lm_sub2(V1, V2), W, V2);
                     z[r + 16] = lm_fma2(lm_add2(V1, V2), W, lm_pack(-a2, -b2));
                 }
@@ -802,7 +838,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
             const int lane = launder(lane_), gw = launder(gwarp_);
             float* const scr = rows + gw * kRowFloats;
             float xr[32], xi[32];
-            warp_cfft1024_part2(z, xr, xi, scr, s_tw, lane, !(LM_SKEW && (gw & 1)));
+            warp_cfft_part2<NFFT>(z, xr, xi, scr, s_tw, lane, !(LM_SKEW && (gw & 1)));
             const int srcl = (32 - lane) & 31;
             const bool l0 = (lane == 0);
             if (NFFT == 2048) {
@@ -845,6 +881,31 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                     if (l0) {
                         scr[256] = fmaf(ur, ur, ui * ui);
                         scr[768] = fmaf(vr, vr, vi * vi);
+                    }
+                }
+            } else if (NFFT < 1024) {
+                // per sub-FFT s, as the 1024 case below with R slots per lane: Z_s[k] = (xr, xi)[s R + k2] at
+                // k = lane + 32 k2, its partner Z_s[n_fft - k] in lane (32 - lane) & 31 at slot R - 1 - k2 (lane 0:
+                // its own slot (R - k2) mod R).  Frames 2s and 2s + 1 go to 2s OFF and (2s + 1) OFF in the row.
+                constexpr int R = G::R;
+#pragma unroll
+                for (int s = 0; s < 32 / R; ++s) {
+                    float* Pa = scr + (2 * s) * G::OFF;
+                    float* Pb = Pa + G::OFF;
+#pragma unroll
+                    for (int k2 = 0; k2 < R / 2; ++k2) {
+                        float br = __shfl_sync(0xffffffffu, xr[s * R + R - 1 - k2], srcl);
+                        float bi = __shfl_sync(0xffffffffu, xi[s * R + R - 1 - k2], srcl);
+                        if (l0) { br = xr[s * R + ((R - k2) & (R - 1))]; bi = xi[s * R + ((R - k2) & (R - 1))]; }
+                        const float ar = xr[s * R + k2], ai = xi[s * R + k2];
+                        const float ur = ar + br, ui = ai - bi, vr = ar - br, vi = ai + bi;
+                        Pa[lane + 32 * k2] = fmaf(ur, ur, ui * ui);
+                        Pb[lane + 32 * k2] = fmaf(vr, vr, vi * vi);
+                    }
+                    if (l0) {   // k = n_fft/2 pairs with itself
+                        const float zr = xr[s * R + R / 2], zi = xi[s * R + R / 2];
+                        Pa[NFFT / 2] = 4.0f * zr * zr;
+                        Pb[NFFT / 2] = 4.0f * zi * zi;
                     }
                 }
             } else {
@@ -890,61 +951,65 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                 if (mt < 0 || LM_EXP == 1) break;
                 const int kb = s_tab->kb[mt], ndk = s_tab->ndk[mt];
                 const float4* __restrict__ wp = s_melw + static_cast<size_t>(s_tab->off[mt]) * 64 + lane;
-                // B operand: frame n = g of column block nb lives in warp row (8 nb + g) / FPW
-                // (+ kPbOff for the odd frame); this lane reads bins kb + 16 d + 4 tg .. +3 of it
-                const float* rp[G::NB];
-                float acc_h[G::NB][4], acc_l[G::NB][4];   // products with the head / the residual of the power
+                // B operand: frame n = g of column block nb lives in warp row (8 nb + g) / FPW at ((8 nb + g) % FPW) OFF;
+                // this lane reads bins kb + 16 d + 4 tg .. +3 of it.  The band is walked once per NBC column blocks: at
+                // n_fft = 256 (NB = 8) all accumulators at once would not fit in the registers beside the rest.
+#pragma unroll 1
+                for (int nb0 = 0; nb0 < G::NB; nb0 += NBC) {
+                    const float* rp[NBC];
+                    float acc_h[NBC][4], acc_l[NBC][4];   // products with the head / the residual of the power
 #pragma unroll
-                for (int nb = 0; nb < G::NB; ++nb) {
-                    const int f = 8 * nb + g;
-                    rp[nb] = rows + (f / G::FPW) * kRowFloats + (f % G::FPW) * kPbOff + kb + 4 * tg;
+                    for (int nb = 0; nb < NBC; ++nb) {
+                        const int f = 8 * (nb0 + nb) + g;
+                        rp[nb] = rows + (f / G::FPW) * kRowFloats + (f % G::FPW) * G::OFF + kb + 4 * tg;
 #pragma unroll
-                    for (int q = 0; q < 4; ++q) { acc_h[nb][q] = 0.f; acc_l[nb][q] = 0.f; }
-                }
-#pragma unroll 2
-                for (int d = 0; d < ndk; ++d) {
-                    // A operand rows 0-7: TF32 head of fb[., mel g], rows 8-15: its residual; one LDS.128 is one
-                    // k-step's fragment.  k-step 1: logical k = tg -> bin 4tg, k = tg+4 -> bin 4tg+1; k-step 2: bins 4tg+2, 4tg+3
-                    const float4 w1 = wp[64 * d], w2 = wp[64 * d + 32];
-#pragma unroll
-                    for (int nb = 0; nb < G::NB; ++nb) {
-                        const float4 pv = *reinterpret_cast<const float4*>(rp[nb] + 16 * d);
-                        const uint32_t p0 = tf32_hi(pv.x), p1 = tf32_hi(pv.y), p2 = tf32_hi(pv.z), p3 = tf32_hi(pv.w);
-                        const lm_f2 r01 = lm_sub2(lm_pack(pv.x, pv.y), lm_pack(__uint_as_float(p0), __uint_as_float(p1)));
-                        const lm_f2 r23 = lm_sub2(lm_pack(pv.z, pv.w), lm_pack(__uint_as_float(p2), __uint_as_float(p3)));
-                        mma_tf32(acc_h[nb], __float_as_uint(w1.x), __float_as_uint(w1.y), __float_as_uint(w1.z), __float_as_uint(w1.w), p0, p1);
-                        mma_tf32(acc_l[nb], __float_as_uint(w1.x), __float_as_uint(w1.y), __float_as_uint(w1.z), __float_as_uint(w1.w),
-                                 __float_as_uint(lm_lo(r01)), __float_as_uint(lm_hi(r01)));
-                        mma_tf32(acc_h[nb], __float_as_uint(w2.x), __float_as_uint(w2.y), __float_as_uint(w2.z), __float_as_uint(w2.w), p2, p3);
-                        mma_tf32(acc_l[nb], __float_as_uint(w2.x), __float_as_uint(w2.y), __float_as_uint(w2.z), __float_as_uint(w2.w),
-                                 __float_as_uint(lm_lo(r23)), __float_as_uint(lm_hi(r23)));
+                        for (int q = 0; q < 4; ++q) { acc_h[nb][q] = 0.f; acc_l[nb][q] = 0.f; }
                     }
-                }
-                // epilogue: c0:(head row, frame 2tg) c1:(head, 2tg+1) c2:(residual row, 2tg) c3:(residual, 2tg+1)
-                const int m = mt * 8 + g;
-                const bool ok_m = m < n_mels;
-                const bool mk_m = (m >= cf0) && (m < cf1);
+#pragma unroll DUNROLL
+                    for (int d = 0; d < ndk; ++d) {
+                        // A operand rows 0-7: TF32 head of fb[., mel g], rows 8-15: its residual; one LDS.128 is one
+                        // k-step's fragment.  k-step 1: logical k = tg -> bin 4tg, k = tg+4 -> bin 4tg+1; k-step 2: bins 4tg+2, 4tg+3
+                        const float4 w1 = wp[64 * d], w2 = wp[64 * d + 32];
 #pragma unroll
-                for (int nb = 0; nb < G::NB; ++nb) {
-                    const lm_f2 mp2 = lm_add2(lm_add2(lm_pack(acc_h[nb][0], acc_h[nb][1]), lm_pack(acc_h[nb][2], acc_h[nb][3])),
-                                              lm_add2(lm_pack(acc_l[nb][0], acc_l[nb][1]), lm_pack(acc_l[nb][2], acc_l[nb][3])));
-                    const int fl = 8 * nb + 2 * tg, tt = tf + fl;
-                    const int o = m * frames + tt;
-                    const float mp0 = lm_lo(mp2), mp1 = lm_hi(mp2);
-                    float v0 = (mp0 <= p.amin) ? p.floor_db : fmaf(p.db_scale, lg2_ftz(mp0), -p.db_offset);
-                    float v1 = (mp1 <= p.amin) ? p.floor_db : fmaf(p.db_scale, lg2_ftz(mp1), -p.db_offset);
-                    if (mk_m || ((tt >= ct0) && (tt < ct1))) v0 = 0.0f;
-                    if (mk_m || ((tt + 1 >= ct0) && (tt + 1 < ct1))) v1 = 0.0f;
-                    const bool ok0 = ok_m && (fl < nf), ok1 = ok_m && (fl + 1 < nf);
-                    if (ok0) out[o] = v0;
-                    if (ok1) out[o + 1] = v1;
-                    if (EXTRA_OUT) {
-                        if (odb) { if (ok0) odb[o] = v0; if (ok1) odb[o + 1] = v1; }
-                        if (omp) { if (ok0) omp[o] = mp0; if (ok1) omp[o + 1] = mp1; }
+                        for (int nb = 0; nb < NBC; ++nb) {
+                            const float4 pv = *reinterpret_cast<const float4*>(rp[nb] + 16 * d);
+                            const uint32_t p0 = tf32_hi(pv.x), p1 = tf32_hi(pv.y), p2 = tf32_hi(pv.z), p3 = tf32_hi(pv.w);
+                            const lm_f2 r01 = lm_sub2(lm_pack(pv.x, pv.y), lm_pack(__uint_as_float(p0), __uint_as_float(p1)));
+                            const lm_f2 r23 = lm_sub2(lm_pack(pv.z, pv.w), lm_pack(__uint_as_float(p2), __uint_as_float(p3)));
+                            mma_tf32(acc_h[nb], __float_as_uint(w1.x), __float_as_uint(w1.y), __float_as_uint(w1.z), __float_as_uint(w1.w), p0, p1);
+                            mma_tf32(acc_l[nb], __float_as_uint(w1.x), __float_as_uint(w1.y), __float_as_uint(w1.z), __float_as_uint(w1.w),
+                                     __float_as_uint(lm_lo(r01)), __float_as_uint(lm_hi(r01)));
+                            mma_tf32(acc_h[nb], __float_as_uint(w2.x), __float_as_uint(w2.y), __float_as_uint(w2.z), __float_as_uint(w2.w), p2, p3);
+                            mma_tf32(acc_l[nb], __float_as_uint(w2.x), __float_as_uint(w2.y), __float_as_uint(w2.z), __float_as_uint(w2.w),
+                                     __float_as_uint(lm_lo(r23)), __float_as_uint(lm_hi(r23)));
+                        }
                     }
-                    const float u0 = ok0 ? v0 : 0.0f, u1 = ok1 ? v1 : 0.0f;
-                    ssum += u0 + u1;
-                    qsum = fmaf(u0, u0, fmaf(u1, u1, qsum));
+                    // epilogue: c0:(head row, frame 2tg) c1:(head, 2tg+1) c2:(residual row, 2tg) c3:(residual, 2tg+1)
+                    const int m = mt * 8 + g;
+                    const bool ok_m = m < n_mels;
+                    const bool mk_m = (m >= cf0) && (m < cf1);
+#pragma unroll
+                    for (int nb = 0; nb < NBC; ++nb) {
+                        const lm_f2 mp2 = lm_add2(lm_add2(lm_pack(acc_h[nb][0], acc_h[nb][1]), lm_pack(acc_h[nb][2], acc_h[nb][3])),
+                                                  lm_add2(lm_pack(acc_l[nb][0], acc_l[nb][1]), lm_pack(acc_l[nb][2], acc_l[nb][3])));
+                        const int fl = 8 * (nb0 + nb) + 2 * tg, tt = tf + fl;
+                        const int o = m * frames + tt;
+                        const float mp0 = lm_lo(mp2), mp1 = lm_hi(mp2);
+                        float v0 = (mp0 <= p.amin) ? p.floor_db : fmaf(p.db_scale, lg2_ftz(mp0), -p.db_offset);
+                        float v1 = (mp1 <= p.amin) ? p.floor_db : fmaf(p.db_scale, lg2_ftz(mp1), -p.db_offset);
+                        if (mk_m || ((tt >= ct0) && (tt < ct1))) v0 = 0.0f;
+                        if (mk_m || ((tt + 1 >= ct0) && (tt + 1 < ct1))) v1 = 0.0f;
+                        const bool ok0 = ok_m && (fl < nf), ok1 = ok_m && (fl + 1 < nf);
+                        if (ok0) out[o] = v0;
+                        if (ok1) out[o + 1] = v1;
+                        if (EXTRA_OUT) {
+                            if (odb) { if (ok0) odb[o] = v0; if (ok1) odb[o + 1] = v1; }
+                            if (omp) { if (ok0) omp[o] = mp0; if (ok1) omp[o + 1] = mp1; }
+                        }
+                        const float u0 = ok0 ? v0 : 0.0f, u1 = ok1 ? v1 : 0.0f;
+                        ssum += u0 + u1;
+                        qsum = fmaf(u0, u0, fmaf(u1, u1, qsum));
+                    }
                 }
             }
             stat_add(&s_stat[tid], ssum, qsum);

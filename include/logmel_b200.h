@@ -52,7 +52,7 @@ extern "C" {
 typedef enum lm_status {
     LM_OK = 0,
     LM_ERR_INVALID_ARG = -1,   /* NULL pointer, negative size, ...                         */
-    LM_ERR_UNSUPPORTED = -2,   /* n_fft not in {1024, 2048}, odd hop, hop > n_fft/4, ...   */
+    LM_ERR_UNSUPPORTED = -2,   /* n_fft not in {256, 512, 1024, 2048}, odd hop, ...        */
     LM_ERR_FILTERBANK = -3,    /* fb support too wide for the on-chip table                */
     LM_ERR_CUDA = -4,          /* a CUDA runtime call failed (see lm_last_cuda_error)      */
     LM_ERR_NO_DEVICE = -5,     /* no CUDA device / wrong architecture                      */
@@ -64,7 +64,7 @@ typedef enum lm_status {
  * (torch.hann_window(n_fft); torchaudio.functional.melscale_fbanks(n_fft/2+1, 0, sr/2, n_mels,
  * sr, None, "htk")). */
 typedef struct lm_config {
-    int32_t n_fft;        /* 2048 or 1024                                              */
+    int32_t n_fft;        /* 2048, 1024, 512 or 256                                    */
     int32_t hop;          /* even, 1 <= hop <= n_fft/4                                 */
     int32_t n_mels;       /* 1..256                                                    */
     int32_t target_len;   /* int(sample_rate * duration): every clip is padded/cropped */
