@@ -9,6 +9,7 @@
 
 #include <algorithm>
 #include <atomic>
+#include <iterator>
 #include <map>
 #include <mutex>
 #include <new>
@@ -34,18 +35,27 @@ int cuda_fail(cudaError_t e, const char* what) {
         if (_e != cudaSuccess) return cuda_fail(_e, #call);  \
     } while (0)
 
-// The companion entry points take raw device pointers and a stream but no plan: make the device that owns the
-// pointer current for the launch (a caller on cuda:0 may hold tensors of cuda:1) and restore it afterwards.
+// Makes a device current for the guard's lifetime and restores the caller's device afterwards, so that every entry
+// point returns with the caller's device current.  DeviceOf(ptr) picks the device that owns a pointer: the companion
+// entry points take raw device pointers and a stream but no plan (a caller on cuda:0 may hold tensors of cuda:1).
 struct DeviceOf {
-    int prev = -1, dev = -1;
+    int prev = -1, dev = -1;   // dev >= 0: switched away from prev
+    cudaError_t err = cudaSuccess;
+    explicit DeviceOf(int device) { enter(device); }
     explicit DeviceOf(const void* ptr) {
         cudaPointerAttributes a{};
-        if (cudaGetDevice(&prev) != cudaSuccess) prev = -1;
-        if (ptr && cudaPointerGetAttributes(&a, ptr) == cudaSuccess && a.type == cudaMemoryTypeDevice) dev = a.device;
+        if (ptr && cudaPointerGetAttributes(&a, ptr) == cudaSuccess && a.type == cudaMemoryTypeDevice) enter(a.device);
         cudaGetLastError();
-        if (dev >= 0 && dev != prev) cudaSetDevice(dev); else dev = -1;
     }
-    ~DeviceOf() { if (dev >= 0 && prev >= 0) cudaSetDevice(prev); }
+    ~DeviceOf() { if (dev >= 0) cudaSetDevice(prev); }
+    DeviceOf(const DeviceOf&) = delete;
+    DeviceOf& operator=(const DeviceOf&) = delete;
+
+  private:
+    void enter(int device) {
+        if ((err = cudaGetDevice(&prev)) != cudaSuccess || device == prev) return;
+        if ((err = cudaSetDevice(device)) == cudaSuccess) dev = device;
+    }
 };
 
 // NVTX range around a C-ABI entry point (SURVEY.md section 5: ranges around plan / execute), visible in Nsight Systems / Compute
@@ -74,6 +84,43 @@ struct HostSlot {
     int cap_clips = 0;
 };
 
+// The logmel_kernel instantiations a plan may launch, by what the call needs.
+enum Variant { kPlain, kExtraOut, kPcm16, kDeviceNoise, kVariants };
+using KernelFn = void (*)(lm::KParams);
+
+// What a plan of one n_fft and hop needs from the kernel's compile-time layout (lm::Geo, lm::Smem).
+struct Geometry {
+    int tile_f;    // frames per item
+    int ns;        // staged floats per item: (tile_f - 1) * hop + n_fft, rounded up to 4
+    int row_cap;   // a mel band of the last frame of a warp row (at (FPW - 1) * OFF) must end before this row offset
+    int nc;        // points of one complex FFT: the twiddle between its two stages is W_nc^(k1 n2)
+    size_t (*smem_total)(int ns, int n_dk);
+    KernelFn kernels[kVariants];
+};
+
+template <int NFFT>
+Geometry geometry(int hop) {
+    using G = lm::Geo<NFFT>;
+    // Philox noise drawn in the kernel has its own staging instantiation (FASTNOISE) at n_fft = 2048 only; the other
+    // sizes stage it in the plain kernel.
+    KernelFn device_noise = lm::logmel_kernel<NFFT, false>;
+    if constexpr (NFFT == 2048) device_noise = lm::logmel_kernel<NFFT, false, true>;
+    return {G::TILE_F, ((G::TILE_F - 1) * hop + NFFT + 3) & ~3, lm::kRowFloats - (G::FPW - 1) * G::OFF, 32 * G::R,
+            &lm::Smem<NFFT>::total,
+            {lm::logmel_kernel<NFFT, false>, lm::logmel_kernel<NFFT, true>, lm::logmel_kernel<NFFT, false, false, true>,
+             device_noise}};
+}
+
+// The one place where a run-time n_fft (validated by lm_plan_create) becomes a compile-time size.
+Geometry geometry(int n_fft, int hop) {
+    switch (n_fft) {
+        case 2048: return geometry<2048>(hop);
+        case 1024: return geometry<1024>(hop);
+        case 512: return geometry<512>(hop);
+        default: return geometry<256>(hop);
+    }
+}
+
 }  // namespace
 
 struct lm_plan {
@@ -83,6 +130,7 @@ struct lm_plan {
     int sm_count = 0, max_ctas = 0, use_tma = 1, stagger_ns = 0;
     int host_chunk_clips = 0;   // lm_forward_host chunk size; 0 = automatic
     size_t smem_bytes = 0;
+    KernelFn kernels[kVariants] = {};
     float db_mult = 10.f, amin = 1e-10f, db_offset = 0.f, floor_db = -100.f, norm_eps = 1e-8f;
     // device constants
     float* d_window = nullptr;
@@ -105,7 +153,7 @@ namespace {
 
 int free_plan(lm_plan* p) {
     if (!p) return LM_OK;
-    cudaSetDevice(p->device);
+    DeviceOf on(p->device);
     cudaFree(p->d_window); cudaFree(p->d_tw); cudaFree(p->d_utw); cudaFree(p->d_melw); cudaFree(p->d_tab); cudaFree(p->d_counters); cudaFree(p->d_split);
     for (auto& s : p->slots) {
         if (s.stream) cudaStreamDestroy(s.stream);
@@ -128,38 +176,37 @@ lm::KParams make_params(const lm_plan* p) {
     return k;
 }
 
-// Raises the dynamic shared-memory limit of every logmel_kernel instantiation a plan of this n_fft may launch.  The
-// limit belongs to the kernel on the current device, not to the plan, and plans of one n_fft with other hops or mel
-// counts need different sizes: it only ever grows, so creating a smaller plan cannot break launches of a larger one
-// made earlier.  The on-device-noise staging variant (FASTNOISE) exists for n_fft = 2048 only; the other sizes stage
-// Philox noise in the plain kernel.
+// Raises the dynamic shared-memory limit of a plan's kernel instantiations.  The limit belongs to the kernel on the
+// current device, not to the plan, and plans of one n_fft with other hops or mel counts need different sizes: it only
+// ever grows, so creating a smaller plan cannot break launches of a larger one made earlier.
 std::mutex g_smem_mu;
-std::map<std::pair<int, int>, size_t> g_smem_limit;   // (n_fft, device) -> limit set so far
+std::map<std::pair<const void*, int>, size_t> g_smem_limit;   // (kernel, device) -> limit set so far
 
-template <int NFFT>
-cudaError_t set_smem_limit(int device, size_t bytes) {
+cudaError_t set_smem_limit(const KernelFn (&kernels)[kVariants], int device, size_t bytes) {
     std::lock_guard<std::mutex> lock(g_smem_mu);
-    size_t& cur = g_smem_limit[std::make_pair(NFFT, device)];
-    if (bytes <= cur) return cudaSuccess;
-    const int b = static_cast<int>(bytes);
-    constexpr bool kFastNoise = (NFFT == 2048);
-    cudaError_t e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess && kFastNoise)
-        e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, false, kFastNoise>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(lm::logmel_kernel<NFFT, false, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, b);
-    if (e == cudaSuccess) cur = bytes;
-    return e;
+    for (KernelFn f : kernels) {
+        size_t& cur = g_smem_limit[std::make_pair(reinterpret_cast<const void*>(f), device)];
+        if (bytes <= cur) continue;
+        const cudaError_t e = cudaFuncSetAttribute(f, cudaFuncAttributeMaxDynamicSharedMemorySize, static_cast<int>(bytes));
+        if (e != cudaSuccess) return e;
+        cur = bytes;
+    }
+    return cudaSuccess;
 }
 
-template <int NFFT>
-void launch_kernel(const lm::KParams& k, int grid, size_t smem, cudaStream_t stream, bool pcm16, bool extra, bool device_noise) {
-    constexpr bool kFastNoise = (NFFT == 2048);
-    if (pcm16) lm::logmel_kernel<NFFT, false, false, true><<<grid, lm::kThreads, smem, stream>>>(k);
-    else if (extra) lm::logmel_kernel<NFFT, true><<<grid, lm::kThreads, smem, stream>>>(k);
-    else if (kFastNoise && device_noise) lm::logmel_kernel<NFFT, false, kFastNoise><<<grid, lm::kThreads, smem, stream>>>(k);
-    else lm::logmel_kernel<NFFT, false><<<grid, lm::kThreads, smem, stream>>>(k);
+// Small batches: fewer clips than 8-warp groups on the GPU.  Cut every clip into `split` chunks of `tiles_per_chunk`
+// whole tiles so that (almost) every group gets one chunk, and at most `split_override` chunks when that is > 1.  When
+// normalising, the chunks' statistics are combined with integer atomics (logmel_kernel.cuh) in a scratch block that
+// holds kMaxSplitClips clips.
+void choose_split(const lm_plan* p, int B, int groups, bool normalize, int* split, int* tiles_per_chunk) {
+    *split = 1;
+    *tiles_per_chunk = p->n_tiles;
+    if (p->split_override == 1 || B >= groups || p->n_tiles < 2 || (normalize && B > kMaxSplitClips)) return;
+    int want = groups / B;
+    if (p->split_override > 1) want = std::min(want, p->split_override);
+    want = std::max(1, std::min(want, p->n_tiles));
+    *tiles_per_chunk = (p->n_tiles + want - 1) / want;
+    *split = (p->n_tiles + *tiles_per_chunk - 1) / *tiles_per_chunk;
 }
 
 int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
@@ -176,23 +223,7 @@ int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* 
     const long long seq = p->launches.fetch_add(1);
     k.work_counter = p->d_counters + 2 * (seq % kCounters);   // zero now, left at zero by the kernel (no memset per launch)
     const int cap = p->max_ctas > 0 ? p->max_ctas : p->sm_count;
-    // Small batches: fewer clips than 8-warp groups on the GPU.  Cut every clip into chunks of whole tiles so that
-    // (almost) every group gets one chunk; statistics are combined with integer atomics (logmel_kernel.cuh).
-    k.split = 1; k.tiles_per_chunk = p->n_tiles;
-    const int groups = cap * lm::kGroups;
-    if (normalize && p->split_override != 1 && B < groups && B <= kMaxSplitClips && p->n_tiles > 1) {
-        int want = groups / B;
-        if (p->split_override > 1) want = std::min(want, p->split_override);
-        want = std::max(1, std::min(want, p->n_tiles));
-        const int tpc = (p->n_tiles + want - 1) / want;
-        k.tiles_per_chunk = tpc;
-        k.split = (p->n_tiles + tpc - 1) / tpc;
-    }
-    if (!normalize && p->split_override != 1 && B < groups && p->n_tiles > 1) {   // nothing to combine: split freely
-        const int want = std::max(1, std::min(groups / B, p->n_tiles));
-        k.tiles_per_chunk = (p->n_tiles + want - 1) / want;
-        k.split = (p->n_tiles + k.tiles_per_chunk - 1) / k.tiles_per_chunk;
-    }
+    choose_split(p, B, cap * lm::kGroups, normalize != 0, &k.split, &k.tiles_per_chunk);
     if (k.split > 1 && normalize) {
         unsigned char* blk = p->d_split + static_cast<size_t>(seq % kCounters) * (kMaxSplitClips * 20);
         k.clip_stats = reinterpret_cast<unsigned long long*>(blk);
@@ -204,12 +235,8 @@ int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* 
     const bool device_noise = (aug != nullptr) && (noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
     // pcm16: `wave` holds 16-bit samples (lm_forward_pcm16), expanded inside the staging, no decode kernel
     if (pcm16 && extra) return LM_ERR_UNSUPPORTED;
-    switch (p->n_fft) {
-        case 2048: launch_kernel<2048>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
-        case 1024: launch_kernel<1024>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
-        case 512: launch_kernel<512>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
-        default: launch_kernel<256>(k, grid, p->smem_bytes, stream, pcm16, extra, device_noise); break;
-    }
+    const Variant v = pcm16 ? kPcm16 : extra ? kExtraOut : device_noise ? kDeviceNoise : kPlain;
+    p->kernels[v]<<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
     LM_CUDA(cudaGetLastError());
     return LM_OK;
 }
@@ -228,6 +255,157 @@ int grow(Tp** ptr, size_t* cap, size_t want) {
     *ptr = nullptr; *cap = 0;
     LM_CUDA(cudaMalloc(reinterpret_cast<void**>(ptr), want * sizeof(Tp)));
     *cap = want;
+    return LM_OK;
+}
+
+// ---- plan creation steps ------------------------------------------------------------------------------------------
+
+// The checks of lm_plan_create that need no device, in the order the status codes are returned.
+int validate_config(const lm_config& cfg) {
+    if (cfg.n_fft != 2048 && cfg.n_fft != 1024 && cfg.n_fft != 512 && cfg.n_fft != 256) return LM_ERR_UNSUPPORTED;
+    if (cfg.hop < 2 || (cfg.hop & 1) || cfg.hop > cfg.n_fft / 4) return LM_ERR_UNSUPPORTED;
+    if (cfg.n_mels < 1 || cfg.n_mels > 256) return LM_ERR_UNSUPPORTED;
+    if (cfg.target_len <= cfg.n_fft / 2) return LM_ERR_TOO_SHORT;
+    if (!(cfg.amin > 0.f)) return LM_ERR_INVALID_ARG;
+    // The kernel keeps half of the window and fuses it with the first butterfly through w[n + N/2] = 1 - w[n], which
+    // holds for the periodic Hann window of the reference (torch.hann_window, TA/transforms/_transforms.py:86-87) and
+    // for nothing else in common use: refuse other windows instead of computing wrong spectra.
+    for (int n = 0; n < cfg.n_fft / 2; ++n)
+        if (!(fabsf(cfg.window[n] + cfg.window[n + cfg.n_fft / 2] - 1.0f) <= 2e-6f)) return LM_ERR_UNSUPPORTED;
+    return LM_OK;
+}
+
+int check_device(int device, cudaDeviceProp* prop) {
+    int n_dev = 0;
+    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev) {
+        cudaGetLastError();
+        return LM_ERR_NO_DEVICE;
+    }
+    LM_CUDA(cudaGetDeviceProperties(prop, device));
+    if (prop->major != 10) return LM_ERR_NO_DEVICE;   // the fatbin holds sm_100a code only
+    return LM_OK;
+}
+
+// Banded filterbank as mma.sync A fragments (scaled by 1/4: the kernel produces 4 |X|^2).
+// Mel tile mt = filters [8mt, 8mt+8).  Its band starts at kb (first non-zero bin, rounded down to
+// 4) and is walked in steps of 16 bins = two MMA k-steps.  For step d and k-step s, lane
+// (g = lane/4, tg = lane%4) holds one float4 = the A fragment (a0, a1, a2, a3) =
+// (head w0, residual w0, head w1, residual w1) with w_j = fb[kb + 16d + 4tg + 2s + j][8mt + g]:
+// MMA rows 0-7 carry the TF32 head (low 13 mantissa bits cleared), rows 8-15 the residual w - head
+// (13 significant bits, of which the tensor core keeps 11), and the k-permutation matches the
+// kernel's LDS.128 loads of the power rows.  Fills the bands of `tab` (kb, ndk, off), `melw` and the
+// filterbank's non-zero count.
+int pack_filterbank(const lm_config& cfg, int row_cap, lm::MelTable* tab, std::vector<float4>* melw, int* nnz) {
+    const int n_freqs = cfg.n_fft / 2 + 1, n_mels = cfg.n_mels, n_mt = (n_mels + 7) / 8;
+    *nnz = 0;
+    for (int k = 0; k < n_freqs; ++k)
+        for (int m = 0; m < n_mels; ++m) *nnz += cfg.fb[static_cast<size_t>(k) * n_mels + m] != 0.0f;
+    auto fbv = [&](int k, int m) -> float {
+        return (k < n_freqs && m < n_mels) ? 0.25f * cfg.fb[static_cast<size_t>(k) * n_mels + m] : 0.0f;
+    };
+    auto head = [](float w) -> float {
+        uint32_t u;
+        memcpy(&u, &w, 4);
+        u &= 0xffffe000u;
+        float h;
+        memcpy(&h, &u, 4);
+        return h;
+    };
+    // bins past n_freqs that a padded band reads hold finite values (zeros, the next frame's spectrum, FFT scratch)
+    // and meet zero weights
+    for (int mt = 0; mt < n_mt; ++mt) {
+        int lo = -1, hi = -1;
+        for (int k = 0; k < n_freqs; ++k)
+            for (int g = 0; g < 8; ++g)
+                if (fbv(k, 8 * mt + g) != 0.0f) { if (lo < 0) lo = k; hi = k; }
+        int kb = 0, ndk = 0;
+        if (lo >= 0) { kb = lo & ~3; ndk = (hi + 1 - kb + 15) / 16; }
+        while (ndk > 0 && kb > 0 && kb + 16 * ndk > row_cap) kb -= 4;   // keep the padded band inside the row
+        if (kb + 16 * ndk > row_cap) return LM_ERR_FILTERBANK;
+        tab->kb[mt] = kb; tab->ndk[mt] = ndk; tab->off[mt] = static_cast<int>(melw->size() / 64);
+        for (int d = 0; d < ndk; ++d)
+            for (int s = 0; s < 2; ++s)
+                for (int lane = 0; lane < 32; ++lane) {
+                    const int g = lane >> 2, tg = lane & 3, k0 = kb + 16 * d + 4 * tg + 2 * s, m = 8 * mt + g;
+                    const float w0 = fbv(k0, m), w1 = fbv(k0 + 1, m);
+                    melw->push_back(make_float4(head(w0), w0 - head(w0), head(w1), w1 - head(w1)));
+                }
+    }
+    if (melw->empty()) melw->assign(64, make_float4(0.f, 0.f, 0.f, 0.f));
+    return melw->size() / 64 > static_cast<size_t>(lm::kMaxDk) ? LM_ERR_FILTERBANK : LM_OK;
+}
+
+// Longest-processing-time assignment of the n_mt mel tiles of `tab` to the 8 warps of a group (both groups use the
+// same table); warps 2s and 2s+1... of one scheduler are warp % 4, balanced too.
+void assign_mel_tiles(int n_mt, lm::MelTable* tab) {
+    for (auto& w : tab->warp_tile)
+        for (int& t : w) t = -1;
+    std::vector<int> order(n_mt);
+    for (int i = 0; i < n_mt; ++i) order[i] = i;
+    std::sort(order.begin(), order.end(), [&](int a, int b) { return tab->ndk[a] > tab->ndk[b]; });
+    int load_w[lm::kGroupWarps] = {0}, load_s[4] = {0, 0, 0, 0}, cnt_w[lm::kGroupWarps] = {0};
+    for (int mt : order) {
+        int best = -1;
+        for (int w = 0; w < lm::kGroupWarps; ++w) {
+            if (cnt_w[w] >= lm::kTileSlots) continue;
+            if (best < 0) { best = w; continue; }
+            const int a = load_w[w] * 64 + load_s[w & 3];
+            const int b = load_w[best] * 64 + load_s[best & 3];
+            // lightest warp first, then lightest scheduler
+            if (a < b) best = w;
+        }
+        tab->warp_tile[best][cnt_w[best]++] = mt;
+        load_w[best] += tab->ndk[mt] + 4;      // a tile's fixed cost (setup + epilogue) is worth ~4 steps
+        load_s[best & 3] += tab->ndk[mt] + 4;
+    }
+}
+
+constexpr double kTwoPi = 6.283185307179586476925286766559;
+
+// W_nc^(k1 n2) between the two FFT stages (warp_twiddle): nc points per complex FFT, lane = s * (nc / 32) + n2
+// carries point n2 of sub-FFT s.  Rows k1 = 1, 2, 3, 4, 8, ..., 28; the kernel forms the others as products.
+std::vector<float2> fft_twiddles(int nc) {
+    std::vector<float2> tw(32 * lm::kTwRows);
+    for (int r = 0; r < lm::kTwRows; ++r) {
+        const int k1 = r < 3 ? r + 1 : 4 * (r - 2);
+        for (int lane = 0; lane < 32; ++lane) {
+            const int n2 = lane % (nc / 32);
+            const double a = kTwoPi * static_cast<double>(k1 * n2) / static_cast<double>(nc);
+            tw[r * 32 + lane] = make_float2(static_cast<float>(cos(a)), static_cast<float>(-sin(a)));
+        }
+    }
+    return tw;
+}
+
+// (cos, sin)(2 pi k / 2048), k < 512: the real-FFT untangle at n_fft = 2048
+std::vector<float2> untangle_twiddles() {
+    std::vector<float2> utw(512);
+    for (int k = 0; k < 512; ++k) {
+        const double a = kTwoPi * static_cast<double>(k) / 2048.0;
+        utw[k] = make_float2(static_cast<float>(cos(a)), static_cast<float>(sin(a)));
+    }
+    return utw;
+}
+
+// The plan's constant tables to the device, and its scheduling counters and small-batch scratch, zeroed.
+int upload_tables(lm_plan* p, const float* window, const std::vector<float2>& tw, const std::vector<float2>& utw,
+                  const std::vector<float4>& melw, const lm::MelTable& tab) {
+    auto up = [&](void** dst, const void* src, size_t bytes) -> int {
+        LM_CUDA(cudaMalloc(dst, bytes));
+        LM_CUDA(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
+        return LM_OK;
+    };
+    int rc = LM_OK;
+    if ((rc = up(reinterpret_cast<void**>(&p->d_window), window, sizeof(float) * p->n_fft)) ||
+        (rc = up(reinterpret_cast<void**>(&p->d_tw), tw.data(), sizeof(float2) * tw.size())) ||
+        (rc = up(reinterpret_cast<void**>(&p->d_utw), utw.data(), sizeof(float2) * utw.size())) ||
+        (rc = up(reinterpret_cast<void**>(&p->d_melw), melw.data(), sizeof(float4) * melw.size())) ||
+        (rc = up(reinterpret_cast<void**>(&p->d_tab), &tab, sizeof(tab))))
+        return rc;
+    LM_CUDA(cudaMalloc(&p->d_counters, sizeof(int) * 2 * kCounters));
+    LM_CUDA(cudaMemset(p->d_counters, 0, sizeof(int) * 2 * kCounters));
+    LM_CUDA(cudaMalloc(&p->d_split, static_cast<size_t>(kCounters) * kMaxSplitClips * 20));
+    LM_CUDA(cudaMemset(p->d_split, 0, static_cast<size_t>(kCounters) * kMaxSplitClips * 20));
     return LM_OK;
 }
 
@@ -256,171 +434,40 @@ int lm_plan_create(const lm_config* cfg, int device, lm_plan** out_plan) {
     NvtxRange nvtx("lm_plan_create");
     if (!cfg || !out_plan || !cfg->window || !cfg->fb) return LM_ERR_INVALID_ARG;
     *out_plan = nullptr;
-    if (cfg->n_fft != 2048 && cfg->n_fft != 1024 && cfg->n_fft != 512 && cfg->n_fft != 256) return LM_ERR_UNSUPPORTED;
-    if (cfg->hop < 2 || (cfg->hop & 1) || cfg->hop > cfg->n_fft / 4) return LM_ERR_UNSUPPORTED;
-    if (cfg->n_mels < 1 || cfg->n_mels > 256) return LM_ERR_UNSUPPORTED;
-    if (cfg->target_len <= cfg->n_fft / 2) return LM_ERR_TOO_SHORT;
-    if (!(cfg->amin > 0.f)) return LM_ERR_INVALID_ARG;
-    // The kernel keeps half of the window and fuses it with the first butterfly through w[n + N/2] = 1 - w[n], which
-    // holds for the periodic Hann window of the reference (torch.hann_window, TA/transforms/_transforms.py:86-87) and
-    // for nothing else in common use: refuse other windows instead of computing wrong spectra.
-    for (int n = 0; n < cfg->n_fft / 2; ++n)
-        if (!(fabsf(cfg->window[n] + cfg->window[n + cfg->n_fft / 2] - 1.0f) <= 2e-6f)) return LM_ERR_UNSUPPORTED;
-
-    int n_dev = 0;
-    if (cudaGetDeviceCount(&n_dev) != cudaSuccess || device < 0 || device >= n_dev) {
-        cudaGetLastError();
-        return LM_ERR_NO_DEVICE;
-    }
+    int rc = validate_config(*cfg);
     cudaDeviceProp prop{};
-    LM_CUDA(cudaGetDeviceProperties(&prop, device));
-    if (prop.major != 10) return LM_ERR_NO_DEVICE;   // the fatbin holds sm_100a code only
-    LM_CUDA(cudaSetDevice(device));
+    if (rc || (rc = check_device(device, &prop))) return rc;
+    DeviceOf on(device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
 
     lm_plan* p = new (std::nothrow) lm_plan();
     if (!p) return LM_ERR_INVALID_ARG;
+    auto fail = [p](int status) { free_plan(p); return status; };
+    const Geometry geo = geometry(cfg->n_fft, cfg->hop);
     p->device = device;
     p->n_fft = cfg->n_fft; p->hop = cfg->hop; p->n_mels = cfg->n_mels; p->T = cfg->target_len;
     p->n_freqs = cfg->n_fft / 2 + 1;
     p->frames = 1 + cfg->target_len / cfg->hop;
-    p->tile_f = lm::kGroupWarps * (2048 / cfg->n_fft);   // lm::Geo<n_fft>::TILE_F
+    p->tile_f = geo.tile_f;
     p->n_tiles = (p->frames + p->tile_f - 1) / p->tile_f;
-    p->ns = (((p->tile_f - 1) * p->hop + p->n_fft) + 3) & ~3;
+    p->ns = geo.ns;
+    std::copy(std::begin(geo.kernels), std::end(geo.kernels), p->kernels);
     p->db_mult = cfg->db_multiplier; p->amin = cfg->amin; p->db_offset = cfg->db_offset;
     p->norm_eps = cfg->norm_eps;
     p->floor_db = cfg->db_multiplier * log10f(cfg->amin) - cfg->db_offset;
     p->sm_count = prop.multiProcessorCount;
 
-    // ---- banded filterbank as mma.sync A fragments (scaled by 1/4: the kernel produces 4 |X|^2) ----
-    // Mel tile mt = filters [8mt, 8mt+8).  Its band starts at kb (first non-zero bin, rounded down to
-    // 4) and is walked in steps of 16 bins = two MMA k-steps.  For step d and k-step s, lane
-    // (g = lane/4, tg = lane%4) holds one float4 = the A fragment (a0, a1, a2, a3) =
-    // (head w0, residual w0, head w1, residual w1) with w_j = fb[kb + 16d + 4tg + 2s + j][8mt + g]:
-    // MMA rows 0-7 carry the TF32 head (low 13 mantissa bits cleared), rows 8-15 the residual w - head
-    // (13 significant bits, of which the tensor core keeps 11), and the k-permutation matches the
-    // kernel's LDS.128 loads of the power rows.
-    const int n_mt = (p->n_mels + 7) / 8;
     lm::MelTable tab{};
     std::vector<float4> melw;
-    int nnz = 0;
-    for (int k = 0; k < p->n_freqs; ++k)
-        for (int m = 0; m < p->n_mels; ++m) nnz += cfg->fb[static_cast<size_t>(k) * p->n_mels + m] != 0.0f;
-    p->fb_nnz = nnz;
-    auto fbv = [&](int k, int m) -> float {
-        return (k < p->n_freqs && m < p->n_mels) ? 0.25f * cfg->fb[static_cast<size_t>(k) * p->n_mels + m] : 0.0f;
-    };
-    auto head = [](float w) -> float {
-        uint32_t u;
-        memcpy(&u, &w, 4);
-        u &= 0xffffe000u;
-        float h;
-        memcpy(&h, &u, 4);
-        return h;
-    };
-    // the band of the last frame of a warp row (at (FPW - 1) * OFF, lm::Geo) must end inside the row; bins past n_freqs
-    // that a padded band reads hold finite values (zeros, the next frame's spectrum, FFT scratch) and meet zero weights
-    const int fpw = 2048 / p->n_fft, row_cap = lm::kRowFloats - (fpw - 1) * (p->n_fft / 2 + 16);
-    for (int mt = 0; mt < n_mt; ++mt) {
-        int lo = -1, hi = -1;
-        for (int k = 0; k < p->n_freqs; ++k)
-            for (int g = 0; g < 8; ++g)
-                if (fbv(k, 8 * mt + g) != 0.0f) { if (lo < 0) lo = k; hi = k; }
-        int kb = 0, ndk = 0;
-        if (lo >= 0) { kb = lo & ~3; ndk = (hi + 1 - kb + 15) / 16; }
-        while (ndk > 0 && kb > 0 && kb + 16 * ndk > row_cap) kb -= 4;   // keep the padded band inside the row
-        if (kb + 16 * ndk > row_cap) { free_plan(p); return LM_ERR_FILTERBANK; }
-        tab.kb[mt] = kb; tab.ndk[mt] = ndk; tab.off[mt] = static_cast<int>(melw.size() / 64);
-        for (int d = 0; d < ndk; ++d)
-            for (int s = 0; s < 2; ++s)
-                for (int lane = 0; lane < 32; ++lane) {
-                    const int g = lane >> 2, tg = lane & 3, k0 = kb + 16 * d + 4 * tg + 2 * s, m = 8 * mt + g;
-                    const float w0 = fbv(k0, m), w1 = fbv(k0 + 1, m);
-                    melw.push_back(make_float4(head(w0), w0 - head(w0), head(w1), w1 - head(w1)));
-                }
-    }
-    if (melw.empty()) melw.assign(64, make_float4(0.f, 0.f, 0.f, 0.f));
+    if ((rc = pack_filterbank(*cfg, geo.row_cap, &tab, &melw, &p->fb_nnz))) return fail(rc);
+    assign_mel_tiles((cfg->n_mels + 7) / 8, &tab);
     p->n_dk = static_cast<int>(melw.size() / 64);
-    if (p->n_dk > lm::kMaxDk) { free_plan(p); return LM_ERR_FILTERBANK; }
-    // longest-processing-time assignment of mel tiles to the 8 warps of a group (both groups use the
-    // same table); warps 2s and 2s+1... of one scheduler are warp % 4, balanced too
-    {
-        for (auto& w : tab.warp_tile)
-            for (int& t : w) t = -1;
-        std::vector<int> order(n_mt);
-        for (int i = 0; i < n_mt; ++i) order[i] = i;
-        std::sort(order.begin(), order.end(), [&](int a, int b) { return tab.ndk[a] > tab.ndk[b]; });
-        int load_w[lm::kGroupWarps] = {0}, load_s[4] = {0, 0, 0, 0}, cnt_w[lm::kGroupWarps] = {0};
-        for (int mt : order) {
-            int best = -1;
-            for (int w = 0; w < lm::kGroupWarps; ++w) {
-                if (cnt_w[w] >= lm::kTileSlots) continue;
-                if (best < 0) { best = w; continue; }
-                const int a = load_w[w] * 64 + load_s[w & 3];
-                const int b = load_w[best] * 64 + load_s[best & 3];
-                // lightest warp first, then lightest scheduler
-                if (a < b) best = w;
-            }
-            tab.warp_tile[best][cnt_w[best]++] = mt;
-            load_w[best] += tab.ndk[mt] + 4;      // a tile's fixed cost (setup + epilogue) is worth ~4 steps
-            load_s[best & 3] += tab.ndk[mt] + 4;
-        }
-    }
+    if ((rc = upload_tables(p, cfg->window, fft_twiddles(geo.nc), untangle_twiddles(), melw, tab))) return fail(rc);
 
-    // ---- twiddles ---------------------------------------------------------------------------
-    // W_nc^(k1 n2) between the two FFT stages: nc = 1024 complex points for n_fft 2048 / 1024, nc = n_fft for the
-    // small sizes, where lane = s * (nc / 32) + n2 carries point n2 of sub-FFT s
-    std::vector<float2> tw(32 * lm::kTwRows), utw(512);
-    const double two_pi = 6.283185307179586476925286766559;
-    const int nc = std::min(p->n_fft, 1024);
-    for (int r = 0; r < lm::kTwRows; ++r) {
-        const int k1 = (lm::kTwRows == 31) ? r + 1 : (r < 3 ? r + 1 : 4 * (r - 2));   // 1..31, or 1, 2, 3, 4, 8, ..., 28
-        for (int lane = 0; lane < 32; ++lane) {
-            const int n2 = lane % (nc / 32);
-            const double a = two_pi * static_cast<double>(k1 * n2) / static_cast<double>(nc);
-            tw[r * 32 + lane] = make_float2(static_cast<float>(cos(a)), static_cast<float>(-sin(a)));
-        }
-    }
-    for (int k = 0; k < 512; ++k) {
-        const double a = two_pi * static_cast<double>(k) / 2048.0;
-        utw[k] = make_float2(static_cast<float>(cos(a)), static_cast<float>(sin(a)));
-    }
-
-    auto up = [&](void** dst, const void* src, size_t bytes) -> int {
-        LM_CUDA(cudaMalloc(dst, bytes));
-        LM_CUDA(cudaMemcpy(*dst, src, bytes, cudaMemcpyHostToDevice));
-        return LM_OK;
-    };
-    int rc = LM_OK;
-    if ((rc = up(reinterpret_cast<void**>(&p->d_window), cfg->window, sizeof(float) * p->n_fft)) ||
-        (rc = up(reinterpret_cast<void**>(&p->d_tw), tw.data(), sizeof(float2) * tw.size())) ||
-        (rc = up(reinterpret_cast<void**>(&p->d_utw), utw.data(), sizeof(float2) * utw.size())) ||
-        (rc = up(reinterpret_cast<void**>(&p->d_melw), melw.data(), sizeof(float4) * melw.size())) ||
-        (rc = up(reinterpret_cast<void**>(&p->d_tab), &tab, sizeof(tab))) ||
-        (rc = (cudaMalloc(&p->d_counters, sizeof(int) * 2 * kCounters) == cudaSuccess &&
-               cudaMemset(p->d_counters, 0, sizeof(int) * 2 * kCounters) == cudaSuccess &&
-               cudaMalloc(&p->d_split, static_cast<size_t>(kCounters) * kMaxSplitClips * 20) == cudaSuccess &&
-               cudaMemset(p->d_split, 0, static_cast<size_t>(kCounters) * kMaxSplitClips * 20) == cudaSuccess)
-                  ? LM_OK : cuda_fail(cudaGetLastError(), "work counters"))) {
-        free_plan(p);
-        return rc;
-    }
-
-    // ---- shared memory --------------------------------------------------------------------
-    cudaError_t e;
-    switch (p->n_fft) {
-        case 2048: p->smem_bytes = lm::Smem<2048>::total(p->ns, p->n_dk); break;
-        case 1024: p->smem_bytes = lm::Smem<1024>::total(p->ns, p->n_dk); break;
-        case 512: p->smem_bytes = lm::Smem<512>::total(p->ns, p->n_dk); break;
-        default: p->smem_bytes = lm::Smem<256>::total(p->ns, p->n_dk); break;
-    }
-    if (p->smem_bytes > prop.sharedMemPerBlockOptin) { free_plan(p); return LM_ERR_FILTERBANK; }
-    switch (p->n_fft) {
-        case 2048: e = set_smem_limit<2048>(device, p->smem_bytes); break;
-        case 1024: e = set_smem_limit<1024>(device, p->smem_bytes); break;
-        case 512: e = set_smem_limit<512>(device, p->smem_bytes); break;
-        default: e = set_smem_limit<256>(device, p->smem_bytes); break;
-    }
-    if (e != cudaSuccess) { free_plan(p); return cuda_fail(e, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)"); }
+    p->smem_bytes = geo.smem_total(p->ns, p->n_dk);
+    if (p->smem_bytes > prop.sharedMemPerBlockOptin) return fail(LM_ERR_FILTERBANK);
+    const cudaError_t e = set_smem_limit(p->kernels, device, p->smem_bytes);
+    if (e != cudaSuccess) return fail(cuda_fail(e, "cudaFuncSetAttribute(MaxDynamicSharedMemorySize)"));
     *out_plan = p;
     return LM_OK;
 }
@@ -470,13 +517,10 @@ int lm_forward(lm_plan* plan, const float* wave, const int64_t* offset, const in
     if (B == 0) return LM_OK;
     if (!wave || !offset || !length || !out_norm) return LM_ERR_INVALID_ARG;
     NvtxRange nvtx("lm_forward");
-    int dev = -1;
-    LM_CUDA(cudaGetDevice(&dev));
-    if (dev != plan->device) LM_CUDA(cudaSetDevice(plan->device));
-    const int rc = launch(plan, wave, offset, length, B, aug, noise, out_norm, out_db, out_melpow, normalize,
-                          static_cast<cudaStream_t>(cuda_stream));
-    if (dev != plan->device) cudaSetDevice(dev);
-    return rc;
+    DeviceOf on(plan->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
+    return launch(plan, wave, offset, length, B, aug, noise, out_norm, out_db, out_melpow, normalize,
+                  static_cast<cudaStream_t>(cuda_stream));
 }
 
 int lm_forward_pcm16(lm_plan* plan, const int16_t* pcm, const int64_t* offset, const int32_t* length, int32_t B,
@@ -485,13 +529,10 @@ int lm_forward_pcm16(lm_plan* plan, const int16_t* pcm, const int64_t* offset, c
     if (B == 0) return LM_OK;
     if (!pcm || !offset || !length || !out_norm) return LM_ERR_INVALID_ARG;
     NvtxRange nvtx("lm_forward_pcm16");
-    int dev = -1;
-    LM_CUDA(cudaGetDevice(&dev));
-    if (dev != plan->device) LM_CUDA(cudaSetDevice(plan->device));
-    const int rc = launch(plan, reinterpret_cast<const float*>(pcm), offset, length, B, aug, noise, out_norm, nullptr, nullptr, normalize,
-                          static_cast<cudaStream_t>(cuda_stream), nullptr, 0, nullptr, true);
-    if (dev != plan->device) cudaSetDevice(dev);
-    return rc;
+    DeviceOf on(plan->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
+    return launch(plan, reinterpret_cast<const float*>(pcm), offset, length, B, aug, noise, out_norm, nullptr, nullptr, normalize,
+                  static_cast<cudaStream_t>(cuda_stream), nullptr, 0, nullptr, true);
 }
 
 int lm_forward_gather(lm_plan* plan, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
@@ -505,13 +546,10 @@ int lm_forward_gather(lm_plan* plan, const float* wave, const int64_t* offset, c
     if ((reinterpret_cast<uintptr_t>(out_slice) & 15u) || (reinterpret_cast<uintptr_t>(mc_slice) & 15u)) return LM_ERR_INVALID_ARG;
     for (int r = 0; r < n_peers; ++r)
         if (!peer_slices[r] || (reinterpret_cast<uintptr_t>(peer_slices[r]) & 15u)) return LM_ERR_INVALID_ARG;
-    int dev = -1;
-    LM_CUDA(cudaGetDevice(&dev));
-    if (dev != plan->device) LM_CUDA(cudaSetDevice(plan->device));
-    const int rc = launch(plan, wave, offset, length, B, aug, noise, out_slice, nullptr, nullptr, 1,
-                          static_cast<cudaStream_t>(cuda_stream), peer_slices, n_peers, mc_slice);
-    if (dev != plan->device) cudaSetDevice(dev);
-    return rc;
+    DeviceOf on(plan->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
+    return launch(plan, wave, offset, length, B, aug, noise, out_slice, nullptr, nullptr, 1,
+                  static_cast<cudaStream_t>(cuda_stream), peer_slices, n_peers, mc_slice);
 }
 
 int lm_resize_finish(const float* in, int32_t B, int32_t n_mels, int32_t frames_in, int32_t frames_out,
@@ -557,7 +595,8 @@ int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resa
         cudaGetLastError();
         return LM_ERR_NO_DEVICE;
     }
-    LM_CUDA(cudaSetDevice(device));
+    DeviceOf on(device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
     int a = orig_freq, b = new_freq;
     while (b) { const int t = a % b; a = b; b = t; }
     const int o = orig_freq / a, q = new_freq / a;
@@ -630,7 +669,7 @@ int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resa
 
 int lm_resampler_destroy(lm_resampler* r) {
     if (!r) return LM_OK;
-    cudaSetDevice(r->device);
+    DeviceOf on(r->device);
     cudaFree(r->d_taps); cudaFree(r->d_k0); cudaFree(r->d_taps4);
     delete r;
     return LM_OK;
@@ -725,9 +764,8 @@ static int forward_host_impl(lm_plan* plan, const void* wave_any, bool pcm16, in
         if (length[i] < 0 || offset[i] < 0 || offset[i] + length[i] > total_samples) return LM_ERR_INVALID_ARG;
     NvtxRange nvtx(pcm16 ? "lm_forward_host_pcm16" : "lm_forward_host");
     std::lock_guard<std::mutex> one_caller(plan->host_mu);   // the staging slots belong to the plan
-    int dev = -1;
-    LM_CUDA(cudaGetDevice(&dev));
-    LM_CUDA(cudaSetDevice(plan->device));
+    DeviceOf on(plan->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
     int rc = ensure_slots(plan);
     if (rc) return rc;
 
@@ -795,7 +833,6 @@ static int forward_host_impl(lm_plan* plan, const void* wave_any, bool pcm16, in
         const cudaError_t e = cudaStreamSynchronize(s.stream);
         if (e != cudaSuccess && rc == LM_OK) rc = cuda_fail(e, "pipeline drain");
     }
-    cudaSetDevice(dev);
     return rc;
 }
 

@@ -9,9 +9,9 @@
 // CTA whose warps all sit in the same phase (DESIGN.md section 5: the relative phase of the groups
 // does not matter, `stagger_ns` is kept as an experiment knob only).
 //
-// A tile is 8 frames (16 / 32 / 64 for n_fft = 1024 / 512 / 256); one warp = one frame at n_fft = 2048, two frames
-// packed as a + i b into one complex FFT at 1024, and 1024 / n_fft such FFTs side by side below (Geo).  Per item,
-// inside a group:
+// A tile is 8 frames (16 / 32 / 64 for n_fft = 1024 / 512 / 256).  Two frame layouts (Geo): one real frame per warp at
+// n_fft = 2048; below that, 1024 / n_fft complex FFTs side by side in the warp, each carrying two real frames packed
+// as a + i b.  Per item, inside a group:
 //
 //   stage   (one item ahead, into the group's single buffer as soon as every warp has pulled its
 //           frame into registers) the tile's samples -> shared memory, once per sample although
@@ -69,16 +69,6 @@
 #ifndef LM_TIMING
 #define LM_TIMING 0
 #endif
-#ifndef LM_SILENT
-#define LM_SILENT 1   // 1: tiles that lie entirely in a plain clip's zero padding skip FFT and mel and write the floor
-#endif
-#ifndef LM_SKEW
-#define LM_SKEW 0   // 1: odd warps of a group apply the twiddle before barrier (A), even warps after it: the two
-                    //    halves then hit the shared-memory pipe (transposes) and the FMA pipe out of step
-#endif
-#ifndef LM_TW2
-#define LM_TW2 1   // 1: twiddle = product of two table entries (10 table rows); 0: full table (31 rows, 8 KB)
-#endif
 #if LM_TIMING
 #define LM_T(slot) do { const long long t_now_ = clock64(); t_acc[slot] += t_now_ - t_last; t_last = t_now_; } while (0)
 #else
@@ -98,7 +88,6 @@ constexpr int kWarps = kGroups * kGroupWarps;
 constexpr int kThreads = kWarps * 32;
 constexpr int kScrPitch = 36;                 // transpose rows: 32 + 4 (16 B aligned, LDS.128 conflict-free)
 constexpr int kRowFloats = 1168;              // per-warp row: >= 32*36 and == 16 (mod 32) for the MMA loads
-constexpr int kPbOff = 528;                   // n_fft=1024: second frame's spectrum inside the row (== 16 mod 32)
 constexpr int kMaxMelTiles = 32;              // n_mels <= 256
 constexpr int kMaxPeers = 7;                  // other GPUs of one NVSwitch domain
 constexpr int kTileSlots = kMaxMelTiles / kGroupWarps;   // mel tiles per warp, at most
@@ -273,20 +262,8 @@ __device__ __forceinline__ float philox_normal(uint64_t seed, uint32_t idx) {
 //           separately; the LDS.128 reads hand the second FFT register pairs of neighbouring
 //           points, the layout its packed stages 1-4 want -- see gen_fft.py) + second radix-32 FFT.
 // ---------------------------------------------------------------------------------------
-#if LM_TW2
 constexpr int kTwRows = 10;   // twiddle table rows kept on chip: k1 = 1, 2, 3, 4, 8, 12, ..., 28
-#else
-constexpr int kTwRows = 31;   // k1 = 1 .. 31
-#endif
 __device__ __forceinline__ void warp_twiddle(lm_f2 (&z)[32], const float2* __restrict__ tw, int lane) {
-#if !LM_TW2
-#pragma unroll
-    for (int k1 = 1; k1 < 32; ++k1) {
-        const float2 w = tw[(k1 - 1) * 32 + lane];   // (cos, -sin): (r + i m)(wx + i wy) = (r wx - m wy, m wx + r wy)
-        z[k1] = lm_fma2(lm_swap(z[k1]), lm_pack(-w.y, w.y), lm_mul2(z[k1], lm_bcast(w.x)));
-    }
-    return;
-#endif
     // Twiddle W1024^(lane*k1), k1 = 4a + b, as the product of two table entries W^(4a*lane) * W^(b*lane):
     // 10 shared-memory loads instead of 31 (the shared-memory pipe is the tighter resource here, and
     // 31 loads in flight on top of z do not fit the register file), one extra rounding per twiddle.
@@ -317,9 +294,8 @@ __device__ __forceinline__ void warp_twiddle(lm_f2 (&z)[32], const float2* __res
 // radix-R FFTs: lane k1 ends with Z_s[k1 + 32 k2] in (xr[s R + k2], xi[s R + k2]).
 template <int NFFT>
 __device__ __forceinline__ void warp_cfft_part2(lm_f2 (&z)[32], float (&xr)[32], float (&xi)[32],
-                                                float* __restrict__ scr, const float2* __restrict__ tw, int lane,
-                                                bool do_twiddle = true) {
-    if (do_twiddle) warp_twiddle(z, tw, lane);
+                                                float* __restrict__ scr, const float2* __restrict__ tw, int lane) {
+    warp_twiddle(z, tw, lane);
     lm_f2 pr[16], pi[16];
 #pragma unroll
     for (int k1 = 0; k1 < 32; ++k1) scr[k1 * kScrPitch + lane] = lm_lo(z[k1]);
@@ -378,9 +354,10 @@ struct ClipCtx;
 // path and must not change the register allocation or the code layout of the kernel's main loop.
 __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restrict__ sb, int ns, int need, int j0, int T, int gtid);
 
-// n_fft = 2048: one real frame per warp (a 1024-point complex FFT of its even / odd samples).  n_fft <= 1024: the
-// warp's 1024 complex points are P = 1024 / n_fft independent n_fft-point FFTs, each carrying two real frames as
-// a + i b, so FPW = 2 P frames per warp.  Frame j of a warp leaves its power spectrum at j * OFF in the warp's row.
+// The two frame layouts.  n_fft = 2048: one real frame per warp (a 1024-point complex FFT of its even / odd samples).
+// n_fft <= 1024: the warp's 1024 complex points are P = 1024 / n_fft independent n_fft-point FFTs of R points per lane
+// (one FFT over the whole warp at 1024), each carrying two real frames as a + i b, so FPW = 2 P frames per warp.
+// Frame j of a warp leaves its power spectrum at j * OFF in the warp's row.
 template <int NFFT>
 struct Geo {
     static_assert(NFFT == 2048 || NFFT == 1024 || NFFT == 512 || NFFT == 256, "n_fft");
@@ -388,12 +365,11 @@ struct Geo {
     static constexpr int TILE_F = kGroupWarps * FPW;     // frames per item
     static constexpr int NB = TILE_F / 8;                // 8-frame MMA column blocks per tile
     // spectrum pitch inside a row: >= n_fft/2 + 1 bins, == 16 (mod 32) so that the two frames g, g+1 that one
-    // quarter-warp's LDS.128 B-operand loads touch sit 16 banks apart (1024: kPbOff, 512: 272, 256: 144)
+    // quarter-warp's LDS.128 B-operand loads touch sit 16 banks apart (1024: 528, 512: 272, 256: 144)
     static constexpr int OFF = NFFT / 2 + 16;
     static constexpr int R = (NFFT >= 1024 ? 1024 : NFFT) / 32;   // points per lane of one complex FFT (second radix)
     static_assert(OFF % 32 == 16 && (FPW - 1) * OFF + NFFT / 2 + 1 <= kRowFloats, "row layout");
 };
-static_assert(Geo<1024>::OFF == kPbOff, "n_fft = 1024 row layout");
 
 // Shared-memory carve-up, shared by host (size) and device (pointers).  Everything of fixed size
 // comes first so that its addresses are compile-time constants (no registers spent on pointers);
@@ -466,7 +442,10 @@ __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restric
 constexpr int kCtxSlot = 80;
 static_assert(sizeof(ClipCtx) <= kCtxSlot && kCtxSlot % 16 == 0, "ClipCtx slot size");
 
-__device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* __restrict__ c, int nfft, bool pcm16 = false) {
+// `nfft` is NFFT passed as a value: with the compile-time constant in the padded-signal bounds below, the compiler
+// reassociates them and the churn that follows through the whole kernel measured 0.1-0.2 % slower at n_fft = 512.
+template <int NFFT, bool PCM16>
+__device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* __restrict__ c, int nfft) {
     const int clip = vclip / p.split, chunk = vclip - clip * p.split;
     c->t_begin = chunk * p.tiles_per_chunk;
     c->t_end = (c->t_begin + p.tiles_per_chunk < p.n_tiles) ? c->t_begin + p.tiles_per_chunk : p.n_tiles;
@@ -475,7 +454,7 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     const int crop = len > p.T ? (len - p.T) / 2 : 0;       // centre crop
     c->clip = clip;
     c->lc = len < p.T ? len : p.T;
-    c->src = pcm16 ? reinterpret_cast<const float*>(reinterpret_cast<const short*>(p.wave) + off + crop) : p.wave + off + crop;
+    c->src = PCM16 ? reinterpret_cast<const float*>(reinterpret_cast<const short*>(p.wave) + off + crop) : p.wave + off + crop;
     int shift = 0, f0 = 0, f1 = 0, t0 = 0, t1 = 0;
     float nscale = 0.0f, gain = 1.0f;
     uint64_t seed = 0;
@@ -493,8 +472,8 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     // plain clip: its power spectrum is exactly 0 and every feature sits at the dB floor, so FFT and mel are
     // skipped (ICBHI cycles average 2.7 s of the 5 s target).  Silence is monotone in the tile index.
     int silent_from = p.n_tiles;
-    if (LM_SILENT && c->plain) {
-        const int tile_f = kGroupWarps * (2048 / nfft);   // Geo<nfft>::TILE_F
+    if (c->plain) {
+        constexpr int tile_f = Geo<NFFT>::TILE_F;
         for (int t = p.n_tiles - 1; t >= 0; --t) {
             const int tf = t * tile_f;
             const int nf = (p.frames - tf) < tile_f ? (p.frames - tf) : tile_f;
@@ -600,7 +579,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
         cnt = (hi - lo) & ~3;
     };
     auto tile_silent = [&](const ClipCtx* __restrict__ c, int tile_) -> bool {   // group-uniform
-        return LM_SILENT && tile_ >= c->silent_from;
+        return tile_ >= c->silent_from;
     };
     auto stage_bulk = [&](const ClipCtx* __restrict__ c, int tile_) {   // ONE thread of the group
         int e_lo, cnt;
@@ -694,7 +673,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
 
     // ---- prologue: item 0 is staged before the loop; item it+1 is staged during item it ----------------
     if (gtid == 0) {
-        load_clip(p, clip0, &s_ctx[0], NFFT, PCM16);
+        load_clip<NFFT, PCM16>(p, clip0, &s_ctx[0], NFFT);
         stage_bulk(&s_ctx[0], s_ctx[0].t_begin);
     }
     group_bar(group);
@@ -736,7 +715,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                 if (wrap) {   // fetch the group's next (virtual) clip
                     const int nxt = nv + atomicAdd(p.work_counter, 1);
                     if (nxt < n_virtual) {
-                        load_clip(p, nxt, cn, NFFT, PCM16);
+                        load_clip<NFFT, PCM16>(p, nxt, cn, NFFT);
                         stage_bulk(cn, cn->t_begin);
                     } else {
                         cn->clip = -1;
@@ -789,24 +768,13 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                     z[r] = lm_fma2(lm_sub2(V1, V2), W, V2);
                     z[r + 16] = lm_fma2(lm_add2(V1, V2), W, lm_pack(-v2.x, -v2.y));
                 }
-            } else if (NFFT == 1024) {
-                // n_fft = 1024: two frames per warp as one complex signal z = a + i b
-                const float* __restrict__ sa = sb + (2 * gw) * hop;
-                const float* __restrict__ sbb = sa + hop;
-#pragma unroll
-                for (int r = 0; r < 16; ++r) {
-                    const float a1 = sa[32 * r + lane], a2 = sa[32 * (r + 16) + lane];
-                    const float b1 = sbb[32 * r + lane], b2 = sbb[32 * (r + 16) + lane];
-                    const lm_f2 V1 = lm_pack(a1, b1), V2 = lm_pack(a2, b2), W = lm_bcast(s_win[32 * r + lane]);
-                    z[r] = lm_fma2(lm_sub2(V1, V2), W, V2);
-                    z[r + 16] = lm_fma2(lm_add2(V1, V2), W, lm_pack(-a2, -b2));
-                }
             } else {
-                // n_fft = 512 / 256: sub-FFT s = lane / R of the warp carries frames 2s (re) and 2s + 1 (im); lane
-                // s R + n2 takes samples n = R n1 + n2, so z[r] and z[r + 16] are n and n + n_fft/2 as above
+                // n_fft <= 1024: sub-FFT s = lane / R of the warp carries frames 2s (re) and 2s + 1 (im) as one complex
+                // signal z = a + i b; lane s R + n2 takes samples n = R n1 + n2, so z[r] and z[r + 16] are n and
+                // n + n_fft/2 as above.  (lane is laundered: at R = 32 the compiler cannot fold lane / R to 0 itself.)
                 constexpr int R = G::R;
-                const int n2 = lane & (R - 1);
-                const float* __restrict__ sa = sb + (G::FPW * gw + 2 * (lane / R)) * hop + n2;
+                const int n2 = R == 32 ? lane : lane & (R - 1), sub = R == 32 ? 0 : lane / R;
+                const float* __restrict__ sa = sb + (G::FPW * gw + 2 * sub) * hop + n2;
                 const float* __restrict__ sbb = sa + hop;
 #pragma unroll
                 for (int r = 0; r < 16; ++r) {
@@ -818,7 +786,6 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                 }
             }
             lm_fft32_aos_from2(z);
-            if (LM_SKEW && (gw & 1)) warp_twiddle(z, s_tw, lane);
         }
         LM_T(1);   // FFT part 1
         group_bar(group);   // (A) every warp of the group is done with the mel phase of the previous item
@@ -838,7 +805,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
             const int lane = launder(lane_), gw = launder(gwarp_);
             float* const scr = rows + gw * kRowFloats;
             float xr[32], xi[32];
-            warp_cfft_part2<NFFT>(z, xr, xi, scr, s_tw, lane, !(LM_SKEW && (gw & 1)));
+            warp_cfft_part2<NFFT>(z, xr, xi, scr, s_tw, lane);
             const int srcl = (32 - lane) & 31;
             const bool l0 = (lane == 0);
             if (NFFT == 2048) {
@@ -883,10 +850,11 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                         scr[768] = fmaf(vr, vr, vi * vi);
                     }
                 }
-            } else if (NFFT < 1024) {
-                // per sub-FFT s, as the 1024 case below with R slots per lane: Z_s[k] = (xr, xi)[s R + k2] at
-                // k = lane + 32 k2, its partner Z_s[n_fft - k] in lane (32 - lane) & 31 at slot R - 1 - k2 (lane 0:
-                // its own slot (R - k2) mod R).  Frames 2s and 2s + 1 go to 2s OFF and (2s + 1) OFF in the row.
+            } else {
+                // Per sub-FFT s, with R slots per lane: Z_s[k] = (xr, xi)[s R + k2] at k = lane + 32 k2, its partner
+                // B = Z_s[n_fft - k] in lane (32 - lane) & 31 at slot R - 1 - k2 (lane 0: its own slot (R - k2) mod R).
+                // A = Z_s[k]:  |Xa|^2 = |A + conj B|^2 / 4, |Xb|^2 = |A - conj B|^2 / 4.  Frames 2s and 2s + 1 go to
+                // 2s OFF and (2s + 1) OFF in the row.
                 constexpr int R = G::R;
 #pragma unroll
                 for (int s = 0; s < 32 / R; ++s) {
@@ -902,30 +870,11 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                         Pa[lane + 32 * k2] = fmaf(ur, ur, ui * ui);
                         Pb[lane + 32 * k2] = fmaf(vr, vr, vi * vi);
                     }
-                    if (l0) {   // k = n_fft/2 pairs with itself
+                    if (l0) {   // k = n_fft/2 pairs with itself: A = B
                         const float zr = xr[s * R + R / 2], zi = xi[s * R + R / 2];
                         Pa[NFFT / 2] = 4.0f * zr * zr;
                         Pb[NFFT / 2] = 4.0f * zi * zi;
                     }
-                }
-            } else {
-                // A = Z[k], B = Z[1024-k]:  |Xa|^2 = |A + conj B|^2 / 4, |Xb|^2 = |A - conj B|^2 / 4
-                const float z16r = xr[16], z16i = xi[16];
-                float* Pa = scr;
-                float* Pb = scr + kPbOff;
-#pragma unroll
-                for (int k2 = 0; k2 < 16; ++k2) {
-                    float br = __shfl_sync(0xffffffffu, xr[31 - k2], srcl);
-                    float bi = __shfl_sync(0xffffffffu, xi[31 - k2], srcl);
-                    if (l0) { br = xr[(32 - k2) & 31]; bi = xi[(32 - k2) & 31]; }
-                    const float ar = xr[k2], ai = xi[k2];
-                    const float ur = ar + br, ui = ai - bi, vr = ar - br, vi = ai + bi;
-                    Pa[lane + 32 * k2] = fmaf(ur, ur, ui * ui);
-                    Pb[lane + 32 * k2] = fmaf(vr, vr, vi * vi);
-                }
-                if (l0) {   // k = 512 pairs with itself: A = B
-                    Pa[512] = 4.0f * z16r * z16r;
-                    Pb[512] = 4.0f * z16i * z16i;
                 }
             }
         }

@@ -125,6 +125,28 @@ class LogMelPlan:
         return (batch, 1, self.n_mels, self.frames)
 
     # -- device path -----------------------------------------------------------------------
+    def _check_device_inputs(self, samples: Tuple[str, torch.Tensor, torch.dtype], offset: torch.Tensor,
+                             length: torch.Tensor, aug: Optional[torch.Tensor], noise: Optional[torch.Tensor],
+                             outs=()) -> int:
+        """Raises ValueError unless the tensors of one device call fit this plan; returns the batch size B.
+        `samples` is (name, tensor, dtype) of the packed clips, `outs` (name, tensor or None) of the outputs."""
+        B = int(offset.numel())
+        for name, t, dt in (samples, ("offset", offset, torch.int64), ("length", length, torch.int32)):
+            if t.device != self.device or t.dtype != dt or not t.is_contiguous():
+                raise ValueError(f"{name} must be a contiguous {dt} tensor on {self.device}")
+        if length.numel() != B:
+            raise ValueError("offset / length size mismatch")
+        for name, t in outs:
+            if t is not None and (t.device != self.device or t.dtype != torch.float32 or not t.is_contiguous()
+                                  or t.numel() != B * self.n_mels * self.frames):
+                raise ValueError(f"{name} must be contiguous fp32 [B,1,n_mels,frames] on {self.device}")
+        if aug is not None and (aug.device != self.device or aug.numel() * aug.element_size() != 40 * B):
+            raise ValueError("aug must hold B lm_aug records (40 bytes each) on the plan's device")
+        if noise is not None and (noise.device != self.device or noise.dtype != torch.float32
+                                  or noise.numel() != B * self.target_length or not noise.is_contiguous()):
+            raise ValueError("noise must be contiguous fp32 [B, target_length] on the plan's device")
+        return B
+
     def forward(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor,
                 aug: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None,
                 normalize: bool = True, out: Optional[torch.Tensor] = None,
@@ -135,23 +157,10 @@ class LogMelPlan:
         wave: fp32 1-D packed samples; offset int64 [B]; length int32 [B];
         aug: uint8 [B*40] device tensor holding ``lm_aug`` records (see ``upload_aug``);
         noise: fp32 [B, target_length].  Returns ``out`` = [B, 1, n_mels, frames] fp32."""
-        B = int(offset.numel())
-        for name, t, dt in (("wave", wave, torch.float32), ("offset", offset, torch.int64), ("length", length, torch.int32)):
-            if t.device != self.device or t.dtype != dt or not t.is_contiguous():
-                raise ValueError(f"{name} must be a contiguous {dt} tensor on {self.device}")
-        if length.numel() != B:
-            raise ValueError("offset / length size mismatch")
+        B = self._check_device_inputs(("wave", wave, torch.float32), offset, length, aug, noise,
+                                      (("out", out), ("out_db", out_db), ("out_melpow", out_melpow)))
         if out is None:
             out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
-        for name, t in (("out", out), ("out_db", out_db), ("out_melpow", out_melpow)):
-            if t is not None and (t.device != self.device or t.dtype != torch.float32 or not t.is_contiguous()
-                                  or t.numel() != B * self.n_mels * self.frames):
-                raise ValueError(f"{name} must be contiguous fp32 [B,1,n_mels,frames] on {self.device}")
-        if aug is not None and (aug.device != self.device or aug.numel() * aug.element_size() != 40 * B):
-            raise ValueError("aug must hold B lm_aug records (40 bytes each) on the plan's device")
-        if noise is not None and (noise.device != self.device or noise.dtype != torch.float32
-                                  or noise.numel() != B * self.target_length or not noise.is_contiguous()):
-            raise ValueError("noise must be contiguous fp32 [B, target_length] on the plan's device")
         s = torch.cuda.current_stream(self.device) if stream is None else stream
         _lib.check(self._lib.lm_forward(self._h, wave.data_ptr(), offset.data_ptr(), length.data_ptr(), B,
                                         _ptr(aug), _ptr(noise), out.data_ptr(), _ptr(out_db), _ptr(out_melpow),
@@ -165,20 +174,9 @@ class LogMelPlan:
         """`forward` on packed int16 samples (the ICBHI wav sample format; R/src/data/preprocessing.py:55-68 is
         torchaudio.load, i.e. x / 32768): one kernel, 2 bytes per sample across HBM, bit-identical to decoding
         first.  Clip starts that are multiples of 8 samples take the bulk-copy staging path."""
-        B = int(offset.numel())
-        for name, t, dt in (("pcm", pcm, torch.int16), ("offset", offset, torch.int64), ("length", length, torch.int32)):
-            if t.device != self.device or t.dtype != dt or not t.is_contiguous():
-                raise ValueError(f"{name} must be a contiguous {dt} tensor on {self.device}")
+        B = self._check_device_inputs(("pcm", pcm, torch.int16), offset, length, aug, noise, (("out", out),))
         if out is None:
             out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
-        elif (out.device != self.device or out.dtype != torch.float32 or not out.is_contiguous()
-              or out.numel() != B * self.n_mels * self.frames):
-            raise ValueError(f"out must be contiguous fp32 [B,1,n_mels,frames] on {self.device}")
-        if aug is not None and (aug.device != self.device or aug.numel() * aug.element_size() != 40 * B):
-            raise ValueError("aug must hold B lm_aug records (40 bytes each) on the plan's device")
-        if noise is not None and (noise.device != self.device or noise.dtype != torch.float32
-                                  or noise.numel() != B * self.target_length or not noise.is_contiguous()):
-            raise ValueError("noise must be contiguous fp32 [B, target_length] on the plan's device")
         s = torch.cuda.current_stream(self.device) if stream is None else stream
         _lib.check(self._lib.lm_forward_pcm16(self._h, pcm.data_ptr(), offset.data_ptr(), length.data_ptr(), B,
                                               _ptr(aug), _ptr(noise), out.data_ptr(), 1 if normalize else 0,
@@ -192,10 +190,7 @@ class LogMelPlan:
         the other ranks' gathered buffers (`peer_slice_ptrs`: device addresses mapped into this process, e.g.
         `torch.distributed._symmetric_memory` buffer pointers + slice offset) or through the multicast address
         `mc_slice_ptr`.  See `sharding.FusedGather`."""
-        B = int(offset.numel())
-        for name, t, dt in (("wave", wave, torch.float32), ("offset", offset, torch.int64), ("length", length, torch.int32)):
-            if t.device != self.device or t.dtype != dt or not t.is_contiguous():
-                raise ValueError(f"{name} must be a contiguous {dt} tensor on {self.device}")
+        B = self._check_device_inputs(("wave", wave, torch.float32), offset, length, aug, noise)
         peers = [int(x) for x in peer_slice_ptrs]
         arr = (C.c_void_p * max(len(peers), 1))(*peers) if peers else None
         s = torch.cuda.current_stream(self.device) if stream is None else stream

@@ -312,6 +312,23 @@ def test_forward_gather_stores_are_bit_identical():
     assert torch.equal(own, want) and all(torch.equal(p, want) for p in peers)
 
 
+def test_forward_gather_checks_aug_and_noise():
+    """forward_gather refuses aug / noise tensors that do not cover the batch, as forward does (the kernel would read
+    past them)."""
+    plan = get_plan(*GEOMETRIES[4])
+    dev = plan.device
+    T, B = plan.target_length, 4
+    wave = torch.zeros(B * T, device=dev)
+    offset = torch.arange(B, device=dev, dtype=torch.int64) * T
+    length = torch.full((B,), T, device=dev, dtype=torch.int32)
+    own = torch.empty(plan.out_shape(B), device=dev)
+    short_aug = plan.upload_aug(A.make_aug_array(B - 1))
+    with pytest.raises(ValueError, match="aug"):
+        plan.forward_gather(wave, offset, length, own.data_ptr(), aug=short_aug)
+    with pytest.raises(ValueError, match="noise"):
+        plan.forward_gather(wave, offset, length, own.data_ptr(), noise=torch.zeros(B - 1, T, device=dev))
+
+
 @pytest.mark.skipif(torch.cuda.device_count() < 2, reason="needs at least two GPUs")
 def test_fused_gather_across_gpus_small_fft():
     n = min(torch.cuda.device_count(), 8)

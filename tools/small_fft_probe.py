@@ -1,5 +1,5 @@
 #!/usr/bin/env python3
-"""Throughput of the 512- / 256-point STFT paths against the 2048 / 512 headline, and the same batches through
+"""Throughput of the 1024- / 512- / 256-point STFT paths against the 2048 / 512 headline, and the same batches through
 torchaudio on the same GPU (T.MelSpectrogram(...).cuda() -> T.AmplitudeToDB() -> per-clip (x - mean) / (std + eps)).
 
 4096 five-second clips of N(0, 0.1^2) per configuration, resident in HBM (0.33 .. 1.31 GB, above the 126 MB L2).
@@ -23,6 +23,7 @@ from audio_classification_icbhi_b200.plan import LogMelPlan  # noqa: E402
 
 # (label, sample_rate, n_fft, hop, n_mels)
 CONFIGS = [
+    ("16k_1024_256_m128", 16000, 1024, 256, 128),
     ("16k_512_128_m128", 16000, 512, 128, 128),
     ("8k_512_128_m64", 8000, 512, 128, 64),
     ("4k_256_64_m64", 4000, 256, 64, 64),
