@@ -12,6 +12,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(PKG_DIR, "liblogmel_b200.so")
 
 LM_OK = 0
+LM_MAX_RESAMPLERS = 8   # rate pairs of one lm_forward_resampled call
 
 
 class LmConfig(C.Structure):
@@ -75,6 +76,8 @@ EXPORTS = {
                                         C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),
     "lm_forward_pcm16": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p,
                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "lm_forward_resampled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                       C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
 }
 
 _lib = None

@@ -85,7 +85,7 @@ struct HostSlot {
 };
 
 // The logmel_kernel instantiations a plan may launch, by what the call needs.
-enum Variant { kPlain, kExtraOut, kPcm16, kDeviceNoise, kVariants };
+enum Variant { kPlain, kExtraOut, kPcm16, kDeviceNoise, kResampled, kVariants };
 using KernelFn = void (*)(lm::KParams);
 
 // What a plan of one n_fft and hop needs from the kernel's compile-time layout (lm::Geo, lm::Smem).
@@ -108,7 +108,7 @@ Geometry geometry(int hop) {
     return {G::TILE_F, ((G::TILE_F - 1) * hop + NFFT + 3) & ~3, lm::kRowFloats - (G::FPW - 1) * G::OFF, 32 * G::R,
             &lm::Smem<NFFT>::total,
             {lm::logmel_kernel<NFFT, false>, lm::logmel_kernel<NFFT, true>, lm::logmel_kernel<NFFT, false, false, true>,
-             device_noise}};
+             device_noise, lm::logmel_kernel<NFFT, false, false, false, true>}};
 }
 
 // The one place where a run-time n_fft (validated by lm_plan_create) becomes a compile-time size.
@@ -122,6 +122,19 @@ Geometry geometry(int n_fft, int hop) {
 }
 
 }  // namespace
+
+// ---- polyphase sinc resampler (torchaudio.transforms.Resample defaults) ---------------------------------------
+struct lm_resampler {
+    int device = 0, orig = 1, neu = 1;   // after division by the gcd
+    int width = 0, ntaps = 0;
+    float* d_taps = nullptr;
+    int* d_k0 = nullptr;
+    // tiled kernel: taps padded to nt4 float4 per phase; shared memory for the widest input span of a 1024-output chunk
+    // (lm_forward_resampled walks the same padded taps inside the log-mel staging)
+    float4* d_taps4 = nullptr;
+    int nt4 = 0, k0max = 0;
+    size_t tile_smem = 0;     // 0 = the span does not fit: the untiled kernel is used
+};
 
 struct lm_plan {
     int device = 0;
@@ -212,7 +225,8 @@ void choose_split(const lm_plan* p, int B, int groups, bool normalize, int* spli
 int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
            const lm_aug* aug, const float* noise, float* out_norm, float* out_db, float* out_melpow,
            int32_t normalize, cudaStream_t stream, float* const* peers = nullptr, int n_peers = 0,
-           float* mc_out = nullptr, bool pcm16 = false) {
+           float* mc_out = nullptr, bool pcm16 = false, const int32_t* source = nullptr,
+           const lm_resampler* const* resamplers = nullptr, int n_resamplers = 0) {
     if (B == 0) return LM_OK;
     lm::KParams k = make_params(p);
     for (int r = 0; r < n_peers; ++r) k.peer[r] = peers[r];
@@ -220,6 +234,14 @@ int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* 
     k.wave = wave; k.offset = reinterpret_cast<const long long*>(offset); k.length = length;
     k.aug = aug; k.noise = noise; k.out_norm = out_norm; k.out_db = out_db; k.out_melpow = out_melpow;
     k.B = B; k.normalize = normalize;
+    // lm_forward_resampled: every clip through the resampling staging, the sample format a run-time flag
+    const bool resampled = source != nullptr;
+    k.source = source; k.pcm16 = pcm16 ? 1 : 0; k.n_rs = n_resamplers;
+    for (int r = 0; r < n_resamplers; ++r) {
+        const lm_resampler* rs = resamplers[r];
+        k.rs_taps4[r] = rs->d_taps4; k.rs_k0[r] = rs->d_k0;
+        k.rs_o[r] = rs->orig; k.rs_q[r] = rs->neu; k.rs_nt4[r] = rs->nt4; k.rs_width[r] = rs->width;
+    }
     const long long seq = p->launches.fetch_add(1);
     k.work_counter = p->d_counters + 2 * (seq % kCounters);   // zero now, left at zero by the kernel (no memset per launch)
     const int cap = p->max_ctas > 0 ? p->max_ctas : p->sm_count;
@@ -235,7 +257,8 @@ int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* 
     const bool device_noise = (aug != nullptr) && (noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
     // pcm16: `wave` holds 16-bit samples (lm_forward_pcm16), expanded inside the staging, no decode kernel
     if (pcm16 && extra) return LM_ERR_UNSUPPORTED;
-    const Variant v = pcm16 ? kPcm16 : extra ? kExtraOut : device_noise ? kDeviceNoise : kPlain;
+    if (resampled && extra) return LM_ERR_UNSUPPORTED;
+    const Variant v = resampled ? kResampled : pcm16 ? kPcm16 : extra ? kExtraOut : device_noise ? kDeviceNoise : kPlain;
     p->kernels[v]<<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
     LM_CUDA(cudaGetLastError());
     return LM_OK;
@@ -552,6 +575,26 @@ int lm_forward_gather(lm_plan* plan, const float* wave, const int64_t* offset, c
                   static_cast<cudaStream_t>(cuda_stream), peer_slices, n_peers, mc_slice);
 }
 
+int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, int32_t n_resamplers, const void* wave,
+                         int32_t pcm16, const int64_t* offset, const int32_t* length, const int32_t* source, int32_t B,
+                         const lm_aug* aug, const float* noise, float* out_norm, int32_t normalize, void* cuda_stream) {
+    // every check that needs no device comes before the plan is dereferenced
+    if (!plan || B < 0 || n_resamplers < 0 || n_resamplers > LM_MAX_RESAMPLERS || (n_resamplers > 0 && !resamplers) ||
+        (pcm16 != 0 && pcm16 != 1))
+        return LM_ERR_INVALID_ARG;
+    for (int r = 0; r < n_resamplers; ++r)
+        if (!resamplers[r]) return LM_ERR_INVALID_ARG;
+    if (B == 0) return LM_OK;
+    if (!wave || !offset || !length || !source || !out_norm) return LM_ERR_INVALID_ARG;
+    for (int r = 0; r < n_resamplers; ++r)
+        if (resamplers[r]->device != plan->device) return LM_ERR_INVALID_ARG;
+    NvtxRange nvtx("lm_forward_resampled");
+    DeviceOf on(plan->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
+    return launch(plan, static_cast<const float*>(wave), offset, length, B, aug, noise, out_norm, nullptr, nullptr, normalize,
+                  static_cast<cudaStream_t>(cuda_stream), nullptr, 0, nullptr, pcm16 != 0, source, resamplers, n_resamplers);
+}
+
 int lm_resize_finish(const float* in, int32_t B, int32_t n_mels, int32_t frames_in, int32_t frames_out,
                      const lm_aug* aug, float* out, int32_t normalize, float norm_eps, void* cuda_stream) {
     if (B < 0 || n_mels < 1 || frames_in < 1 || frames_out < 1) return LM_ERR_INVALID_ARG;
@@ -574,18 +617,6 @@ int lm_pcm16_roundtrip(const float* in, float* out, int64_t n, void* cuda_stream
     LM_CUDA(cudaGetLastError());
     return LM_OK;
 }
-
-// ---- polyphase sinc resampler (torchaudio.transforms.Resample defaults) ---------------------------------------
-struct lm_resampler {
-    int device = 0, orig = 1, neu = 1;   // after division by the gcd
-    int width = 0, ntaps = 0;
-    float* d_taps = nullptr;
-    int* d_k0 = nullptr;
-    // tiled kernel: taps padded to nt4 float4 per phase; shared memory for the widest input span of a 1024-output chunk
-    float4* d_taps4 = nullptr;
-    int nt4 = 0, k0max = 0;
-    size_t tile_smem = 0;     // 0 = the span does not fit: the untiled kernel is used
-};
 
 int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resampler** out) {
     if (!out || orig_freq < 1 || new_freq < 1) return LM_ERR_INVALID_ARG;

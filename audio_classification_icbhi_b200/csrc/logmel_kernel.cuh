@@ -145,6 +145,15 @@ struct KParams {
     const float2* __restrict__ utw;     // [512]    (cos, sin)(2 pi k / 2048)
     const float4* __restrict__ melw;    // [n_dk][2 k-steps][32 lanes]: mma A fragments (head, residual, head, residual)
     const MelTable* __restrict__ mel_table;
+    // lm_forward_resampled (RESAMPLE instantiation): clip i is at the rate of rate pair source[i] (-1: the plan's rate)
+    // and is resampled inside the staging; `wave` holds int16 samples when pcm16 is set.  Per rate pair the tables of
+    // the tiled resampler (logmel_aux.cuh resample_tiled_kernel): nt4 float4 taps per phase, first tap k0 per phase.
+    const int* __restrict__ source;
+    int pcm16;
+    int n_rs;
+    const float4* rs_taps4[LM_MAX_RESAMPLERS];
+    const int* rs_k0[LM_MAX_RESAMPLERS];
+    int rs_o[LM_MAX_RESAMPLERS], rs_q[LM_MAX_RESAMPLERS], rs_nt4[LM_MAX_RESAMPLERS], rs_width[LM_MAX_RESAMPLERS];
 };
 
 // ---------------------------------------------------------------------------------------
@@ -442,9 +451,105 @@ __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restric
 constexpr int kCtxSlot = 80;
 static_assert(sizeof(ClipCtx) <= kCtxSlot && kCtxSlot % 16 == 0, "ClipCtx slot size");
 
+// ---------------------------------------------------------------------------------------
+// Resampling inside the staging (RESAMPLE instantiation, lm_forward_resampled).  Clip i holds len native samples;
+// its resampled signal y has L' = ceil(q len / o) samples and is padded / centre-cropped like any clip, so staged
+// sample i (after reflect and roll, i < lc = min(L', T)) is y[crop + i], crop = (L' - T) / 2 when L' > T.  y[m q + ph]
+// is the tiled resampler's chain: acc = fmaf(taps4[ph][t], x[m o + k0[ph] - width + t], acc) for t < 4 nt4, x = 0
+// outside [0, len) -- the same taps, the same order and the same zero-padded tail, hence bit-identical to lm_resample.
+// ClipCtx has no room for the rate pair: the staging reads source / length / offset of the clip again per tile.
+// ---------------------------------------------------------------------------------------
+struct RsClip {
+    const float4* taps4;
+    const int* k0;
+    long long len;    // native samples (0 for a source index outside [-1, n_rs))
+    long long lp;     // L': samples of y (len when the clip is at the plan's rate)
+    long long crop;   // first sample of y kept by the centre crop
+    int o, q, nt4, width;   // q == 0: the clip is at the plan's rate (src already points past its crop)
+};
+__device__ __forceinline__ RsClip rs_clip(const KParams& p, int clip) {
+    RsClip r{nullptr, nullptr, p.length[clip], 0, 0, 1, 0, 0, 0};
+    const int s = p.source[clip];
+    r.lp = r.len;
+    if (s < -1 || s >= p.n_rs) {   // device data: an invalid index makes an empty clip, nothing is read
+        r.len = 0; r.lp = 0;
+    } else if (s >= 0) {
+        r.taps4 = p.rs_taps4[s]; r.k0 = p.rs_k0[s];
+        r.o = p.rs_o[s]; r.q = p.rs_q[s]; r.nt4 = p.rs_nt4[s]; r.width = p.rs_width[s];
+        r.lp = (static_cast<long long>(r.q) * r.len + r.o - 1) / r.o;   // 64-bit: q len overflows int for long recordings
+    }
+    r.crop = r.lp > p.T ? (r.lp - p.T) / 2 : 0;
+    return r;
+}
+template <bool PCM>
+__device__ __forceinline__ float rs_in(const void* x, long long k) {
+    return PCM ? static_cast<float>(__ldg(static_cast<const short*>(x) + k)) * (1.0f / 32768.0f) : __ldg(static_cast<const float*>(x) + k);
+}
+template <bool PCM>
+__device__ __forceinline__ float rs_sample(const RsClip& r, const void* x, long long mp) {
+    const long long m = mp / r.q;
+    const int ph = static_cast<int>(mp - m * r.q);
+    const long long base = m * r.o + __ldg(r.k0 + ph) - r.width;   // native index of tap 0
+    const float4* __restrict__ w = r.taps4 + static_cast<size_t>(ph) * r.nt4;
+    float acc = 0.0f;
+    if (base >= 0 && base + 4 * r.nt4 <= r.len) {   // the whole (padded) span inside the clip: no bounds checks
+        for (int t = 0; t < r.nt4; ++t) {
+            const float4 wv = __ldg(w + t);
+            const long long k = base + 4 * t;
+            acc = fmaf(wv.x, rs_in<PCM>(x, k), acc);
+            acc = fmaf(wv.y, rs_in<PCM>(x, k + 1), acc);
+            acc = fmaf(wv.z, rs_in<PCM>(x, k + 2), acc);
+            acc = fmaf(wv.w, rs_in<PCM>(x, k + 3), acc);
+        }
+    } else {
+        auto at = [&](long long k) { return (k >= 0 && k < r.len) ? rs_in<PCM>(x, k) : 0.0f; };
+        for (int t = 0; t < r.nt4; ++t) {
+            const float4 wv = __ldg(w + t);
+            const long long k = base + 4 * t;
+            acc = fmaf(wv.x, at(k), acc);
+            acc = fmaf(wv.y, at(k + 1), acc);
+            acc = fmaf(wv.z, at(k + 2), acc);
+            acc = fmaf(wv.w, at(k + 3), acc);
+        }
+    }
+    return acc;
+}
+// One tile of a clip of lm_forward_resampled: the steps of stage_gather (reflect, roll, i < lc, gain, noise), with the
+// source value computed by rs_sample.  Kept out of line like stage_noisy_tile.
+template <bool PCM>
+__device__ __forceinline__ void stage_resampled_impl(const ClipCtx& c, const RsClip& r, float* __restrict__ sb, int ns, int need,
+                                                     int j0, int T, int gtid) {
+    const void* x = c.src;
+    const int shift = c.shift, lc = c.lc;
+    for (int e = gtid; e < ns; e += kGroupThreads) {
+        int j = j0 + e;
+        if (j < 0) j = -j;
+        else if (j >= T) j = 2 * (T - 1) - j;
+        float v = 0.0f;
+        if (e < need && j >= 0 && j < T) {
+            int i = j - shift;               // torch.roll: out[j] = in[(j - shift) mod T]
+            if (i < 0) i += T;
+            else if (i >= T) i -= T;
+            if (i < lc) v = (r.q ? rs_sample<PCM>(r, x, r.crop + i) : rs_in<PCM>(x, i)) * c.gain;
+            if (c.nscale != 0.0f) {
+                const float z = c.nz ? __ldg(c.nz + i) : philox_normal(c.seed, static_cast<uint32_t>(i));
+                v = fmaf(z, c.nscale, v);
+            }
+        }
+        sb[e] = v;
+    }
+}
+__device__ __noinline__ void stage_resampled_tile(const ClipCtx& c, const RsClip r, int pcm16, float* __restrict__ sb, int ns,
+                                                  int need, int j0, int T, int gtid) {
+    if (pcm16) stage_resampled_impl<true>(c, r, sb, ns, need, j0, T, gtid);
+    else stage_resampled_impl<false>(c, r, sb, ns, need, j0, T, gtid);
+}
+
 // `nfft` is NFFT passed as a value: with the compile-time constant in the padded-signal bounds below, the compiler
 // reassociates them and the churn that follows through the whole kernel measured 0.1-0.2 % slower at n_fft = 512.
-template <int NFFT, bool PCM16>
+// RESAMPLE: lc = min(L', T) and src is the clip's first native sample, or its first sample after the crop for a clip at
+// the plan's rate (rs_clip); `plain` then only decides silent tiles, the staging never takes the bulk-copy path.
+template <int NFFT, bool PCM16, bool RESAMPLE = false>
 __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* __restrict__ c, int nfft) {
     const int clip = vclip / p.split, chunk = vclip - clip * p.split;
     c->t_begin = chunk * p.tiles_per_chunk;
@@ -455,6 +560,12 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     c->clip = clip;
     c->lc = len < p.T ? len : p.T;
     c->src = PCM16 ? reinterpret_cast<const float*>(reinterpret_cast<const short*>(p.wave) + off + crop) : p.wave + off + crop;
+    if (RESAMPLE) {   // overrides the lines above rather than replacing them: an if / else moved the register allocation of every other instantiation
+        const RsClip r = rs_clip(p, clip);
+        const long long start = off + (r.q ? 0 : r.crop);
+        c->lc = r.lp < p.T ? static_cast<int>(r.lp) : p.T;
+        c->src = p.pcm16 ? reinterpret_cast<const float*>(reinterpret_cast<const short*>(p.wave) + start) : p.wave + start;
+    }
     int shift = 0, f0 = 0, f1 = 0, t0 = 0, t1 = 0;
     float nscale = 0.0f, gain = 1.0f;
     uint64_t seed = 0;
@@ -490,9 +601,12 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
 // FASTNOISE: tiles of clips with on-device Philox noise are staged four samples per thread (stage_noisy_tile).  The call
 // costs the main loop ~3 % (registers live across it), so the host launches this instantiation only when the batch can
 // contain such clips (augmentation records given, no host-drawn noise tensor); the headline path keeps FASTNOISE = false.
-template <int NFFT, bool EXTRA_OUT, bool FASTNOISE = false, bool PCM16 = false>
+// RESAMPLE: lm_forward_resampled.  Every tile goes through stage_resampled_tile (no bulk copy; fp32 or 16-bit samples by
+// p.pcm16 at run time, Philox noise drawn per sample); silent tiles still apply to un-augmented clips.
+template <int NFFT, bool EXTRA_OUT, bool FASTNOISE = false, bool PCM16 = false, bool RESAMPLE = false>
 __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
     static_assert(!(PCM16 && (FASTNOISE || EXTRA_OUT)), "the 16-bit instantiation is the plain one");
+    static_assert(!(RESAMPLE && (PCM16 || FASTNOISE || EXTRA_OUT)), "the resampling instantiation is the plain one");
     using G = Geo<NFFT>;
     constexpr int TILE_F = G::TILE_F;
     constexpr int HALF = NFFT / 2;
@@ -559,7 +673,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
     // bulk part: [e_lo, e_lo + cnt) of the tile is src[j0 + e_lo ...] verbatim (plain clips only)
     auto bulk_range = [&](const ClipCtx* __restrict__ c, int tile_, int& e_lo, int& cnt) {
         e_lo = 0; cnt = 0;
-        if (!p.use_tma || !c->plain) return;
+        if (RESAMPLE || !p.use_tma || !c->plain) return;
         const int tf = tile_ * TILE_F;
         const int nf = (frames - tf) < TILE_F ? (frames - tf) : TILE_F;
         const int need = (nf - 1) * hop + NFFT;
@@ -643,6 +757,10 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
         const int nf = (frames - tf) < TILE_F ? (frames - tf) : TILE_F;
         const int need = (nf - 1) * hop + NFFT;
         const int j0 = tf * hop - HALF;
+        if (RESAMPLE) {
+            stage_resampled_tile(*cc, rs_clip(p, c.clip), p.pcm16, sb, p.ns, need, j0, T, gtid);
+            return true;
+        }
         // reflect (torch.stft center=True) -> roll -> pad/crop -> gain, + noise; slots past `need`
         // feed only frames >= `frames` and are zeroed
         if (FASTNOISE && c.nscale != 0.0f && c.nz == nullptr && cnt == 0) {   // on-device noise (training batches): out of line
@@ -673,7 +791,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
 
     // ---- prologue: item 0 is staged before the loop; item it+1 is staged during item it ----------------
     if (gtid == 0) {
-        load_clip<NFFT, PCM16>(p, clip0, &s_ctx[0], NFFT);
+        load_clip<NFFT, PCM16, RESAMPLE>(p, clip0, &s_ctx[0], NFFT);
         stage_bulk(&s_ctx[0], s_ctx[0].t_begin);
     }
     group_bar(group);
@@ -715,7 +833,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                 if (wrap) {   // fetch the group's next (virtual) clip
                     const int nxt = nv + atomicAdd(p.work_counter, 1);
                     if (nxt < n_virtual) {
-                        load_clip<NFFT, PCM16>(p, nxt, cn, NFFT);
+                        load_clip<NFFT, PCM16, RESAMPLE>(p, nxt, cn, NFFT);
                         stage_bulk(cn, cn->t_begin);
                     } else {
                         cn->clip = -1;

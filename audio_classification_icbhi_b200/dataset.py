@@ -16,6 +16,7 @@ from typing import List, Sequence, Tuple
 import torch
 from torch.utils.data import Dataset
 
+from . import _lib
 from .preprocessing import AudioPreprocessor
 
 __all__ = ["ICBHIDataset", "ICBHISegmentedDataset", "GpuCollate", "GpuLoader", "raw_collate"]
@@ -65,8 +66,9 @@ class RawView(Dataset):
 
 class GpuCollate:
     """collate_fn for raw items: list of (waveform, sample_rate, label) -- or (waveform, label) for waveforms already
-    at the target rate -- -> (features [B,1,n_mels,frames] on the GPU, labels int64 on the GPU).  Recordings at
-    another rate are resampled here, on the GPU (`lm_resample`), then the whole batch is ONE `lm_forward` launch.
+    at the target rate -- -> (features [B,1,n_mels,frames] on the GPU, labels int64 on the GPU).  The whole batch is
+    ONE log-mel launch; recordings at other rates are resampled inside it (`lm_forward_resampled`).  A batch with more
+    than LM_MAX_RESAMPLERS distinct foreign rates is resampled item by item first (`lm_resample`), then packed.
     It must run in the process that owns the CUDA context.  A DataLoader calls its collate_fn INSIDE the worker
     processes, so with `num_workers > 0` give the loader `raw_collate` (workers hand back plain lists) and wrap it in
     `GpuLoader(loader, GpuCollate(...))`, which collates in the training process; with `num_workers=0` it can be
@@ -77,16 +79,17 @@ class GpuCollate:
         self.fast_augment = fast_augment
 
     def __call__(self, batch: Sequence[tuple]):
-        waves, labels = [], []
+        pre = self.preprocessor
+        waves, rates, labels = [], [], []
         for item in batch:
-            if len(item) == 3:
-                w, sr, y = item
-                w = self.preprocessor.resample_to_target(w, sr)
-            else:
-                w, y = item
+            w, sr, y = item if len(item) == 3 else (item[0], pre.sample_rate, item[1])
             waves.append(w)
+            rates.append(int(sr))
             labels.append(int(y))
-        feats = self.preprocessor.preprocess_batch(waves, fast_augment=self.fast_augment)
+        if len({r for r in rates if r != int(pre.sample_rate)}) > _lib.LM_MAX_RESAMPLERS:
+            waves = [pre.resample_to_target(w, sr) for w, sr in zip(waves, rates)]
+            rates = None
+        feats = pre.preprocess_batch(waves, fast_augment=self.fast_augment, sample_rates=rates)
         return feats, torch.tensor(labels, dtype=torch.int64).to(feats.device, non_blocking=True)
 
 

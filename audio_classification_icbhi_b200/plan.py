@@ -183,6 +183,45 @@ class LogMelPlan:
                                               C.c_void_p(s.cuda_stream)))
         return out
 
+    def forward_resampled(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor, source: torch.Tensor,
+                          resamplers: Sequence["Resampler"], aug: Optional[torch.Tensor] = None,
+                          noise: Optional[torch.Tensor] = None, normalize: bool = True, out: Optional[torch.Tensor] = None,
+                          stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """`forward` on clips at their own sample rates, resampled to the plan's rate inside the kernel: one launch for
+        a batch that mixes rates.  `wave` is fp32 or int16 (x / 32768) packed samples; `offset` / `length` count
+        samples at the clip's own rate; `source` int32 [B] (on the host or on the plan's device) holds each clip's
+        index into `resamplers` (`Resampler(clip_rate, plan.sample_rate)`, at most LM_MAX_RESAMPLERS), or -1 for a clip
+        already at the plan's rate.  Bit-identical to resampling each clip with its `Resampler`, packing the results
+        and calling `forward` (`forward_pcm16` for int16 clips with source -1)."""
+        if wave.dtype not in (torch.float32, torch.int16):
+            raise ValueError("wave must be fp32 samples or int16 PCM")
+        B = self._check_device_inputs(("wave", wave, wave.dtype), offset, length, aug, noise, (("out", out),))
+        resamplers = list(resamplers)
+        if len(resamplers) > _lib.LM_MAX_RESAMPLERS:
+            raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} resamplers per call")
+        for r in resamplers:
+            if r.new_freq != self.sample_rate:
+                raise ValueError(f"resampler {r.orig_freq} -> {r.new_freq} Hz does not produce the plan's {self.sample_rate} Hz")
+            if torch.device("cuda", r.device.index or 0) != self.device:
+                raise ValueError(f"resampler on {r.device}, plan on {self.device}")
+        if source.dtype != torch.int32 or source.numel() != B or source.dim() != 1 or source.device.type not in ("cpu", "cuda") \
+                or (source.is_cuda and source.device != self.device):
+            raise ValueError(f"source must be an int32 [B] tensor on the host or on {self.device}")
+        if B and (int(source.min()) < -1 or int(source.max()) >= len(resamplers)):
+            raise ValueError(f"source values must lie in [-1, {len(resamplers)})")
+        if not source.is_cuda:
+            source = source.contiguous().to(self.device, non_blocking=True)
+        source = source.contiguous()
+        if out is None:
+            out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
+        handles = (C.c_void_p * max(len(resamplers), 1))(*[r._h.value for r in resamplers])
+        s = torch.cuda.current_stream(self.device) if stream is None else stream
+        _lib.check(self._lib.lm_forward_resampled(self._h, handles, len(resamplers), wave.data_ptr(),
+                                                  1 if wave.dtype == torch.int16 else 0, offset.data_ptr(), length.data_ptr(),
+                                                  source.data_ptr(), B, _ptr(aug), _ptr(noise), out.data_ptr(),
+                                                  1 if normalize else 0, C.c_void_p(s.cuda_stream)))
+        return out
+
     def forward_gather(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor, out_slice_ptr: int,
                        peer_slice_ptrs=(), mc_slice_ptr: int = 0, aug: Optional[torch.Tensor] = None,
                        noise: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> None:

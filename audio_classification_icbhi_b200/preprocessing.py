@@ -264,16 +264,24 @@ class AudioPreprocessor:
             noise_d.index_copy_(0, ix.to(plan.device), noise.index_select(0, ix).to(plan.device, non_blocking=True))
         return noise_d
 
-    def _finish(self, plan: LogMelPlan, wave, offset, length, aug, noise, B: int) -> torch.Tensor:
-        """Runs the kernel(s).  Overridden by FlexibleAudioPreprocessor when a resize is needed."""
+    def _finish(self, plan: LogMelPlan, wave, offset, length, aug, noise, B: int, forward=None) -> torch.Tensor:
+        """Runs the kernel(s).  Overridden by FlexibleAudioPreprocessor when a resize is needed.  `forward` is
+        `plan.forward` or a stand-in with its signature (`plan.forward_resampled` with the rate pairs bound)."""
+        forward = plan.forward if forward is None else forward
         aug_d = plan.upload_aug(aug) if aug is not None else None
-        return plan.forward(wave, offset, length, aug=aug_d, noise=self._upload_noise(plan, aug, noise))
+        return forward(wave, offset, length, aug=aug_d, noise=self._upload_noise(plan, aug, noise))
 
     def preprocess_batch(self, waveforms: Union[Sequence[Wave], torch.Tensor],
-                         lengths: Optional[Sequence[int]] = None, fast_augment: bool = False) -> torch.Tensor:
+                         lengths: Optional[Sequence[int]] = None, fast_augment: bool = False,
+                         sample_rates: Optional[Sequence[int]] = None) -> torch.Tensor:
         """Batched hot path.  `waveforms`: list of 1-D / [C, len] waveforms of any lengths (host
         or device), or a dense `[B, len]` tensor (optionally with per-row `lengths`).
+        `sample_rates`: optional rate of each clip.  Clips at other rates than `sample_rate` are resampled inside the
+        log-mel kernel (`LogMelPlan.forward_resampled`, at most LM_MAX_RESAMPLERS distinct foreign rates per batch),
+        with the same result as `resample_to_target` on each of them first.
         Returns `[B, 1, n_mels, frames]` float32 on the GPU."""
+        if sample_rates is not None and any(int(r) != int(self.sample_rate) for r in sample_rates):
+            return self._preprocess_resampled(waveforms, lengths, fast_augment, sample_rates)
         plan = self.plan
         dev = plan.device
         if isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2:
@@ -287,32 +295,65 @@ class AudioPreprocessor:
         else:
             clips = [_as_mono_1d(w) for w in waveforms]
             B = len(clips)
-            lens = [int(c.numel()) for c in clips]
-            starts, pos = [], 0
-            for n in lens:           # 16-byte aligned clip starts: interior tiles go through TMA
-                starts.append(pos)
-                pos += (n + 3) & ~3
-            packed = torch.empty(max(pos, 4), dtype=torch.float32, device=dev)   # alignment gaps are never read
-            # host clips: packed into ONE pinned staging buffer (kept on the object, grow-only) and sent with ONE
-            # asynchronous copy; clips that already live on the device (e.g. resampled by GpuCollate) are copied in place
-            host_ix = [i for i, c in enumerate(clips) if not c.is_cuda]
-            if host_ix:
-                lo, hi = starts[host_ix[0]], starts[host_ix[-1]] + lens[host_ix[-1]]
-                stage = self._pinned_stage(hi - lo)
-                for i in host_ix:
-                    if lens[i]:
-                        stage[starts[i] - lo:starts[i] - lo + lens[i]].copy_(clips[i])
-                if hi > lo:
-                    packed[lo:hi].copy_(stage[:hi - lo], non_blocking=True)
-                self._stage_release()
-            for i, c in enumerate(clips):        # after the block copy: it also covered their (stale) slots
-                if c.is_cuda and lens[i]:
-                    packed[starts[i]:starts[i] + lens[i]].copy_(c, non_blocking=True)
-            wave = packed
-            offset = torch.tensor(starts, dtype=torch.int64).to(dev, non_blocking=True)
-            length = torch.tensor(lens, dtype=torch.int32).to(dev, non_blocking=True)
+            wave, offset, length = self._pack(clips)
         aug, noise = self._draw(B, fast_augment)
         return self._finish(plan, wave, offset, length, aug, noise, B)
+
+    def _pack(self, clips: List[torch.Tensor]):
+        """1-D fp32 clips (host or device) -> (packed device samples, offset int64, length int32) on the plan's device."""
+        dev = self.plan.device
+        lens = [int(c.numel()) for c in clips]
+        starts, pos = [], 0
+        for n in lens:           # 16-byte aligned clip starts: interior tiles go through TMA
+            starts.append(pos)
+            pos += (n + 3) & ~3
+        packed = torch.empty(max(pos, 4), dtype=torch.float32, device=dev)   # alignment gaps are never read
+        # host clips: packed into ONE pinned staging buffer (kept on the object, grow-only) and sent with ONE
+        # asynchronous copy; clips that already live on the device (e.g. resampled by GpuCollate) are copied in place
+        host_ix = [i for i, c in enumerate(clips) if not c.is_cuda]
+        if host_ix:
+            lo, hi = starts[host_ix[0]], starts[host_ix[-1]] + lens[host_ix[-1]]
+            stage = self._pinned_stage(hi - lo)
+            for i in host_ix:
+                if lens[i]:
+                    stage[starts[i] - lo:starts[i] - lo + lens[i]].copy_(clips[i])
+            if hi > lo:
+                packed[lo:hi].copy_(stage[:hi - lo], non_blocking=True)
+            self._stage_release()
+        for i, c in enumerate(clips):        # after the block copy: it also covered their (stale) slots
+            if c.is_cuda and lens[i]:
+                packed[starts[i]:starts[i] + lens[i]].copy_(c, non_blocking=True)
+        offset = torch.tensor(starts, dtype=torch.int64).to(dev, non_blocking=True)
+        length = torch.tensor(lens, dtype=torch.int32).to(dev, non_blocking=True)
+        return packed, offset, length
+
+    def _preprocess_resampled(self, waveforms, lengths, fast_augment: bool, sample_rates) -> torch.Tensor:
+        """`preprocess_batch` for a batch with clips at other rates: native-rate clips packed as usual, then ONE
+        `forward_resampled` launch (through `_finish`, so the flexible resize path applies too)."""
+        from functools import partial
+        from .resample import get_resampler
+        plan = self.plan
+        if isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2:
+            n = waveforms.shape[1]
+            lens = [n] * waveforms.shape[0] if lengths is None else [int(x) for x in lengths]
+            if max(lens, default=0) > n:
+                raise ValueError("lengths exceed the row length")
+            clips = [waveforms[i, :lens[i]].to(torch.float32) for i in range(waveforms.shape[0])]
+        else:
+            clips = [_as_mono_1d(w) for w in waveforms]
+        B = len(clips)
+        rates = [int(r) for r in sample_rates]
+        if len(rates) != B:
+            raise ValueError("sample_rates must give one rate per waveform")
+        foreign = sorted({r for r in rates if r != int(self.sample_rate)})
+        if len(foreign) > _lib.LM_MAX_RESAMPLERS:
+            raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} sample rates other than {self.sample_rate} per batch")
+        resamplers = [get_resampler(r, int(self.sample_rate), plan.device) for r in foreign]
+        source = torch.tensor([foreign.index(r) if r != int(self.sample_rate) else -1 for r in rates], dtype=torch.int32)
+        wave, offset, length = self._pack(clips)
+        aug, noise = self._draw(B, fast_augment)
+        forward = partial(plan.forward_resampled, source=source, resamplers=resamplers)
+        return self._finish(plan, wave, offset, length, aug, noise, B, forward=forward)
 
     def preprocess_waveform(self, waveform: Wave) -> torch.Tensor:
         """One in-memory waveform -> `[1, n_mels, frames]` float32 CPU tensor (what `preprocess`

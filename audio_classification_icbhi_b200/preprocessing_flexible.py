@@ -73,10 +73,11 @@ class FlexibleAudioPreprocessor(AudioPreprocessor):
                                         1 if normalize else 0, 1e-8, C.c_void_p(stream)))
         return out
 
-    def _finish(self, plan: LogMelPlan, wave, offset, length, aug, noise, B: int) -> torch.Tensor:
+    def _finish(self, plan: LogMelPlan, wave, offset, length, aug, noise, B: int, forward=None) -> torch.Tensor:
         fout = self.target_time_steps()
         if plan.frames == fout:
-            return super()._finish(plan, wave, offset, length, aug, noise, B)
+            return super()._finish(plan, wave, offset, length, aug, noise, B, forward=forward)
+        forward = plan.forward if forward is None else forward
         # fused kernel up to dB with the waveform augmentation only; masks act on the resized map
         aug_d = plan.upload_aug(aug) if aug is not None else None
         wave_aug_d = None
@@ -85,5 +86,5 @@ class FlexibleAudioPreprocessor(AudioPreprocessor):
             wa["f0"] = wa["f1"] = wa["t0"] = wa["t1"] = 0
             wave_aug_d = plan.upload_aug(wa)
         noise_d = self._upload_noise(plan, aug, noise)
-        db = plan.forward(wave, offset, length, aug=wave_aug_d, noise=noise_d, normalize=False)
+        db = forward(wave, offset, length, aug=wave_aug_d, noise=noise_d, normalize=False)
         return self._resize_finish(db, fout, aug_d, normalize=True)

@@ -48,6 +48,7 @@ extern "C" {
 #endif
 
 #define LM_ABI_VERSION 1
+#define LM_MAX_RESAMPLERS 8   /* rate pairs of one lm_forward_resampled call */
 
 typedef enum lm_status {
     LM_OK = 0,
@@ -113,7 +114,7 @@ int lm_plan_info(const lm_plan* plan, lm_info* info);
 /* Tuning knobs for experiments: key "tma" (0/1), "max_ctas" (0 = SM count), "split" (small-batch mode:
  * 0 = automatic, 1 = off, k = at most k tile ranges per clip), "host_chunk_clips", "stagger_ns". */
 int lm_plan_set(lm_plan* plan, const char* key, int value);
-/* Number of kernels this plan has launched since creation (lm_forward: 1 per call,
+/* Number of kernels this plan has launched since creation (lm_forward, lm_forward_resampled: 1 per call,
  * lm_forward_host / lm_forward_host_pcm16: 1 per chunk). */
 int64_t lm_plan_launch_count(const lm_plan* plan);
 
@@ -189,6 +190,30 @@ int lm_resample(const lm_resampler* r, const float* in, int64_t in_len, float* o
  * in + i * in_stride and goes to out + i * out_stride (strides in floats). */
 int lm_resample_rows(const lm_resampler* r, const float* in, int64_t in_len, int64_t in_stride, int32_t n_rows,
                      float* out, int64_t out_stride, void* cuda_stream);
+
+/*
+ * lm_forward for clips recorded at other sample rates (ICBHI: 4, 10 and 44.1 kHz), resampled to the plan's rate
+ * inside the log-mel kernel's staging: one launch for a batch that mixes rates, no resampled copy in memory.
+ *   resamplers  HOST array of n_resamplers (0..LM_MAX_RESAMPLERS) handles from lm_resampler_create(clip_rate,
+ *               plan_rate, plan_device), on the plan's device.  The caller guarantees that each one's new rate is
+ *               the rate the plan's filterbank was built for: lm_config carries no rate, so the library cannot check.
+ *               They must outlive the launch in stream order.
+ *   wave        DEVICE pointer to packed samples: fp32 when pcm16 == 0, 16-bit PCM (x / 32768) when pcm16 == 1
+ *   offset, length  [B] int64 / int32, in samples at the clip's OWN rate
+ *   source      [B] int32 DEVICE array: index into `resamplers` of the clip's rate pair, -1 for a clip already at the
+ *               plan's rate.  An index outside [-1, n_resamplers) makes the clip a zero-length clip (nothing is read).
+ *   aug, noise, out_norm, normalize  as lm_forward (noise rows hold target_len draws at the plan's rate); there are no
+ *               extra outputs.  normalize == 0 leaves dB (the input of lm_resize_finish).
+ * Output is bit-identical to: y_i = lm_resample(resamplers[source[i]], clip i) (ceil(q len / o) samples), the y_i
+ * packed, then lm_forward (fp32) with the same aug, noise and normalize -- pad or centre crop, roll, gain and noise
+ * act on y_i.  A clip with source -1 gives exactly what lm_forward (fp32) or lm_forward_pcm16 (pcm16) gives.
+ * Returns LM_ERR_INVALID_ARG for NULL pointers or handles, a bad n_resamplers or pcm16, or a resampler on
+ * another device.
+ */
+int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, int32_t n_resamplers,
+                         const void* wave, int32_t pcm16, const int64_t* offset, const int32_t* length,
+                         const int32_t* source, int32_t B, const lm_aug* aug, const float* noise,
+                         float* out_norm, int32_t normalize, void* cuda_stream);
 
 /*
  * T.AmplitudeToDB() as a stand-alone transform (R/src/data/preprocessing.py:46; torchaudio/functional/functional.py:390-391,
