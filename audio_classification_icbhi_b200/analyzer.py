@@ -11,6 +11,7 @@ clips would be.  There is no 15 s cap (:126).
 from __future__ import annotations
 
 import ctypes as C
+from functools import partial
 from typing import List, Optional, Tuple, Union
 
 import numpy as np
@@ -81,5 +82,5 @@ class SlidingWindowLogMel:
         length = torch.from_numpy(lengths).to(plan.device)
         if rec.numel() < 4:
             rec = torch.nn.functional.pad(rec, (0, 4 - rec.numel()))
-        feats = self.preprocessor._finish(plan, rec.contiguous(), offset, length, None, None, len(starts))
+        feats = self.preprocessor._finish(plan, partial(plan.forward, rec.contiguous(), offset, length), None, None)
         return feats, times

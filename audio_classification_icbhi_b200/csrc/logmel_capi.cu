@@ -72,8 +72,7 @@ constexpr int kMaxSplitClips = 512;  // small-batch mode is used below 2 * SM co
 
 struct HostSlot {
     cudaStream_t stream = nullptr;
-    float* d_wave = nullptr;      size_t cap_wave = 0;     // floats
-    int16_t* d_pcm = nullptr;     size_t cap_pcm = 0;      // 16-bit samples (lm_forward_host_pcm16)
+    unsigned char* d_wave = nullptr;  size_t cap_wave = 0; // bytes of fp32 or 16-bit samples
     float* d_noise = nullptr;     size_t cap_noise = 0;
     float* d_out = nullptr;       size_t cap_out = 0;
     // per-chunk metadata, one pinned staging block and one device block: [offset int64 x n][aug 40 B x n][length int32 x n]
@@ -170,7 +169,7 @@ int free_plan(lm_plan* p) {
     cudaFree(p->d_window); cudaFree(p->d_tw); cudaFree(p->d_utw); cudaFree(p->d_melw); cudaFree(p->d_tab); cudaFree(p->d_counters); cudaFree(p->d_split);
     for (auto& s : p->slots) {
         if (s.stream) cudaStreamDestroy(s.stream);
-        cudaFree(s.d_wave); cudaFree(s.d_pcm); cudaFree(s.d_noise); cudaFree(s.d_out);
+        cudaFree(s.d_wave); cudaFree(s.d_noise); cudaFree(s.d_out);
         cudaFree(s.d_meta);
         if (s.h_meta) cudaFreeHost(s.h_meta);
     }
@@ -222,46 +221,67 @@ void choose_split(const lm_plan* p, int B, int groups, bool normalize, int* spli
     *split = (p->n_tiles + *tiles_per_chunk - 1) / *tiles_per_chunk;
 }
 
-int launch(lm_plan* p, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
-           const lm_aug* aug, const float* noise, float* out_norm, float* out_db, float* out_melpow,
-           int32_t normalize, cudaStream_t stream, float* const* peers = nullptr, int n_peers = 0,
-           float* mc_out = nullptr, bool pcm16 = false, const int32_t* source = nullptr,
-           const lm_resampler* const* resamplers = nullptr, int n_resamplers = 0) {
-    if (B == 0) return LM_OK;
+// A batch as the kernel reads it: clip i is samples [offset[i], offset[i] + length[i]), fp32 or, when pcm16, 16-bit PCM
+// expanded to x / 32768 inside the staging (no decode kernel).  lm_forward_resampled adds the rate of each clip: that of
+// resamplers[source[i]], or the plan's rate for -1.
+struct Batch {
+    const void* samples; bool pcm16;
+    const int64_t* offset; const int32_t* length; int32_t B;
+    const lm_aug* aug; const float* noise;
+    const int32_t* source = nullptr; const lm_resampler* const* resamplers = nullptr; int n_resamplers = 0;
+};
+
+// Where the features go: `norm` always, dB and mel power when given.  lm_forward_gather also stores the normalised
+// features into the other ranks' gathered buffers (`peers`) or through a multicast address (`mc`).
+struct Outputs {
+    float* norm; float* db = nullptr; float* melpow = nullptr;
+    float* const* peers = nullptr; int n_peers = 0; float* mc = nullptr;
+};
+
+int launch(lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, cudaStream_t stream) {
+    if (b.B == 0) return LM_OK;
     lm::KParams k = make_params(p);
-    for (int r = 0; r < n_peers; ++r) k.peer[r] = peers[r];
-    k.n_peer = n_peers; k.mc_out = mc_out;
-    k.wave = wave; k.offset = reinterpret_cast<const long long*>(offset); k.length = length;
-    k.aug = aug; k.noise = noise; k.out_norm = out_norm; k.out_db = out_db; k.out_melpow = out_melpow;
-    k.B = B; k.normalize = normalize;
+    for (int r = 0; r < o.n_peers; ++r) k.peer[r] = o.peers[r];
+    k.n_peer = o.n_peers; k.mc_out = o.mc;
+    k.wave = b.samples; k.offset = reinterpret_cast<const long long*>(b.offset); k.length = b.length;
+    k.aug = b.aug; k.noise = b.noise; k.out_norm = o.norm; k.out_db = o.db; k.out_melpow = o.melpow;
+    k.B = b.B; k.normalize = normalize;
     // lm_forward_resampled: every clip through the resampling staging, the sample format a run-time flag
-    const bool resampled = source != nullptr;
-    k.source = source; k.pcm16 = pcm16 ? 1 : 0; k.n_rs = n_resamplers;
-    for (int r = 0; r < n_resamplers; ++r) {
-        const lm_resampler* rs = resamplers[r];
+    const bool resampled = b.source != nullptr;
+    k.source = b.source; k.pcm16 = b.pcm16 ? 1 : 0; k.n_rs = b.n_resamplers;
+    for (int r = 0; r < b.n_resamplers; ++r) {
+        const lm_resampler* rs = b.resamplers[r];
         k.rs_taps4[r] = rs->d_taps4; k.rs_k0[r] = rs->d_k0;
         k.rs_o[r] = rs->orig; k.rs_q[r] = rs->neu; k.rs_nt4[r] = rs->nt4; k.rs_width[r] = rs->width;
     }
     const long long seq = p->launches.fetch_add(1);
     k.work_counter = p->d_counters + 2 * (seq % kCounters);   // zero now, left at zero by the kernel (no memset per launch)
     const int cap = p->max_ctas > 0 ? p->max_ctas : p->sm_count;
-    choose_split(p, B, cap * lm::kGroups, normalize != 0, &k.split, &k.tiles_per_chunk);
+    choose_split(p, b.B, cap * lm::kGroups, normalize != 0, &k.split, &k.tiles_per_chunk);
     if (k.split > 1 && normalize) {
         unsigned char* blk = p->d_split + static_cast<size_t>(seq % kCounters) * (kMaxSplitClips * 20);
         k.clip_stats = reinterpret_cast<unsigned long long*>(blk);
         k.clip_cnt = reinterpret_cast<int*>(blk + kMaxSplitClips * 16);
         // zero at plan creation; the group that completes a clip resets its entries
     }
-    const int grid = std::min<int>(B * k.split, cap);
-    const bool extra = (out_db != nullptr) || (out_melpow != nullptr);
-    const bool device_noise = (aug != nullptr) && (noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
-    // pcm16: `wave` holds 16-bit samples (lm_forward_pcm16), expanded inside the staging, no decode kernel
-    if (pcm16 && extra) return LM_ERR_UNSUPPORTED;
+    const int grid = std::min<int>(b.B * k.split, cap);
+    const bool extra = (o.db != nullptr) || (o.melpow != nullptr);
+    const bool device_noise = (b.aug != nullptr) && (b.noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
+    if (b.pcm16 && extra) return LM_ERR_UNSUPPORTED;
     if (resampled && extra) return LM_ERR_UNSUPPORTED;
-    const Variant v = resampled ? kResampled : pcm16 ? kPcm16 : extra ? kExtraOut : device_noise ? kDeviceNoise : kPlain;
+    const Variant v = resampled ? kResampled : b.pcm16 ? kPcm16 : extra ? kExtraOut : device_noise ? kDeviceNoise : kPlain;
     p->kernels[v]<<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
     LM_CUDA(cudaGetLastError());
     return LM_OK;
+}
+
+// The common tail of the device-input entry points, after their argument checks: an NVTX range named after the entry
+// point, the plan's device made current, one launch.
+int forward_on_device(const char* name, lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, void* stream) {
+    NvtxRange nvtx(name);
+    DeviceOf on(p->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
+    return launch(p, b, o, normalize, static_cast<cudaStream_t>(stream));
 }
 
 int ensure_slots(lm_plan* p) {
@@ -432,6 +452,88 @@ int upload_tables(lm_plan* p, const float* window, const std::vector<float2>& tw
     return LM_OK;
 }
 
+// lm_forward_host and lm_forward_host_pcm16: `wave` holds fp32 samples, or 16-bit PCM when pcm16.
+int forward_host_impl(lm_plan* plan, const void* wave, bool pcm16, int64_t total_samples, const int64_t* offset,
+                      const int32_t* length, int32_t B, const lm_aug* aug, const float* noise, float* out, int32_t normalize) {
+    if (!plan || B < 0 || total_samples < 0) return LM_ERR_INVALID_ARG;
+    if (B == 0) return LM_OK;
+    if (!wave || !offset || !length || !out) return LM_ERR_INVALID_ARG;
+    for (int i = 0; i < B; ++i)
+        if (length[i] < 0 || offset[i] < 0 || offset[i] + length[i] > total_samples) return LM_ERR_INVALID_ARG;
+    NvtxRange nvtx(pcm16 ? "lm_forward_host_pcm16" : "lm_forward_host");
+    std::lock_guard<std::mutex> one_caller(plan->host_mu);   // the staging slots belong to the plan
+    DeviceOf on(plan->device);
+    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
+    int rc = ensure_slots(plan);
+    if (rc) return rc;
+
+    const size_t clip_elems = static_cast<size_t>(plan->n_mels) * plan->frames;
+    const size_t sample_bytes = pcm16 ? sizeof(int16_t) : sizeof(float);
+    // chunk so that a few chunks are in flight: ~64 MB of waveform, at least 2 SM-waves of clips
+    const int auto_chunk = std::max(2 * plan->sm_count, static_cast<int>((64u << 20) / (4u * static_cast<size_t>(plan->T))));
+    const int chunk = std::max(1, std::min<int>(B, plan->host_chunk_clips > 0 ? plan->host_chunk_clips : auto_chunk));
+    int slot_i = 0;
+    for (int c0 = 0; c0 < B && rc == LM_OK; c0 += chunk, slot_i = (slot_i + 1) % kSlots) {
+        const int n = std::min(chunk, B - c0);
+        HostSlot& s = plan->slots[slot_i];
+        if ((rc = cudaStreamSynchronize(s.stream) == cudaSuccess ? LM_OK : cuda_fail(cudaGetLastError(), "slot sync"))) break;
+        int64_t lo = INT64_MAX, hi = 0;
+        for (int i = c0; i < c0 + n; ++i) {
+            if (length[i] == 0) continue;
+            lo = std::min(lo, offset[i]);
+            hi = std::max(hi, offset[i] + length[i]);
+        }
+        if (lo == INT64_MAX) { lo = 0; hi = 0; }
+        lo &= ~int64_t(7);   // keep 16-byte alignment of clip starts (TMA staging path; 8 PCM samples per int4)
+        const size_t n_wave = static_cast<size_t>(hi - lo);
+        constexpr size_t kMetaPerClip = sizeof(long long) + sizeof(lm_aug) + sizeof(int);
+        if (n > s.cap_clips) {
+            cudaFree(s.d_meta);
+            if (s.h_meta) cudaFreeHost(s.h_meta);
+            s.d_meta = nullptr; s.h_meta = nullptr; s.cap_clips = 0;
+            if (cudaMalloc(&s.d_meta, kMetaPerClip * n) != cudaSuccess || cudaMallocHost(&s.h_meta, kMetaPerClip * n) != cudaSuccess) {
+                rc = cuda_fail(cudaGetLastError(), "slot metadata alloc");
+                break;
+            }
+            s.cap_clips = n;
+        }
+        // the blocks are laid out for the slot's capacity so that the three arrays keep their alignment
+        const size_t cap = static_cast<size_t>(s.cap_clips);
+        long long* h_off = reinterpret_cast<long long*>(s.h_meta);
+        lm_aug* h_aug = reinterpret_cast<lm_aug*>(s.h_meta + sizeof(long long) * cap);
+        int* h_len = reinterpret_cast<int*>(s.h_meta + (sizeof(long long) + sizeof(lm_aug)) * cap);
+        const long long* d_off = reinterpret_cast<const long long*>(s.d_meta);
+        const lm_aug* d_aug = reinterpret_cast<const lm_aug*>(s.d_meta + sizeof(long long) * cap);
+        const int* d_len = reinterpret_cast<const int*>(s.d_meta + (sizeof(long long) + sizeof(lm_aug)) * cap);
+        if ((rc = grow(&s.d_wave, &s.cap_wave, sample_bytes * std::max<size_t>(n_wave + 8, 16)))) break;
+        if ((rc = grow(&s.d_out, &s.cap_out, clip_elems * n))) break;
+        if (noise && (rc = grow(&s.d_noise, &s.cap_noise, static_cast<size_t>(plan->T) * n))) break;
+        for (int i = 0; i < n; ++i) h_off[i] = length[c0 + i] ? offset[c0 + i] - lo : 0;
+        memcpy(h_len, length + c0, sizeof(int) * n);
+        if (aug) memcpy(h_aug, aug + c0, sizeof(lm_aug) * n);
+
+        cudaError_t e = cudaMemcpyAsync(s.d_meta, s.h_meta, kMetaPerClip * cap, cudaMemcpyHostToDevice, s.stream);
+        if (e != cudaSuccess) { rc = cuda_fail(e, "H2D copy (metadata)"); break; }
+        if (n_wave)
+            e = cudaMemcpyAsync(s.d_wave, static_cast<const unsigned char*>(wave) + sample_bytes * lo, sample_bytes * n_wave,
+                                cudaMemcpyHostToDevice, s.stream);
+        if (e == cudaSuccess && noise)
+            e = cudaMemcpyAsync(s.d_noise, noise + static_cast<size_t>(c0) * plan->T, sizeof(float) * plan->T * n,
+                                cudaMemcpyHostToDevice, s.stream);
+        if (e != cudaSuccess) { rc = cuda_fail(e, "H2D copy"); break; }
+        rc = launch(plan, {s.d_wave, pcm16, reinterpret_cast<const int64_t*>(d_off), d_len, n, aug ? d_aug : nullptr,
+                           noise ? s.d_noise : nullptr}, {s.d_out}, normalize, s.stream);
+        if (rc) break;
+        e = cudaMemcpyAsync(out + clip_elems * c0, s.d_out, sizeof(float) * clip_elems * n, cudaMemcpyDeviceToHost, s.stream);
+        if (e != cudaSuccess) { rc = cuda_fail(e, "D2H copy"); break; }
+    }
+    for (auto& s : plan->slots) {
+        const cudaError_t e = cudaStreamSynchronize(s.stream);
+        if (e != cudaSuccess && rc == LM_OK) rc = cuda_fail(e, "pipeline drain");
+    }
+    return rc;
+}
+
 }  // namespace
 
 extern "C" {
@@ -539,11 +641,8 @@ int lm_forward(lm_plan* plan, const float* wave, const int64_t* offset, const in
     if (!plan || B < 0) return LM_ERR_INVALID_ARG;
     if (B == 0) return LM_OK;
     if (!wave || !offset || !length || !out_norm) return LM_ERR_INVALID_ARG;
-    NvtxRange nvtx("lm_forward");
-    DeviceOf on(plan->device);
-    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
-    return launch(plan, wave, offset, length, B, aug, noise, out_norm, out_db, out_melpow, normalize,
-                  static_cast<cudaStream_t>(cuda_stream));
+    return forward_on_device("lm_forward", plan, {wave, false, offset, length, B, aug, noise}, {out_norm, out_db, out_melpow},
+                             normalize, cuda_stream);
 }
 
 int lm_forward_pcm16(lm_plan* plan, const int16_t* pcm, const int64_t* offset, const int32_t* length, int32_t B,
@@ -551,11 +650,7 @@ int lm_forward_pcm16(lm_plan* plan, const int16_t* pcm, const int64_t* offset, c
     if (!plan || B < 0) return LM_ERR_INVALID_ARG;
     if (B == 0) return LM_OK;
     if (!pcm || !offset || !length || !out_norm) return LM_ERR_INVALID_ARG;
-    NvtxRange nvtx("lm_forward_pcm16");
-    DeviceOf on(plan->device);
-    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
-    return launch(plan, reinterpret_cast<const float*>(pcm), offset, length, B, aug, noise, out_norm, nullptr, nullptr, normalize,
-                  static_cast<cudaStream_t>(cuda_stream), nullptr, 0, nullptr, true);
+    return forward_on_device("lm_forward_pcm16", plan, {pcm, true, offset, length, B, aug, noise}, {out_norm}, normalize, cuda_stream);
 }
 
 int lm_forward_gather(lm_plan* plan, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
@@ -569,10 +664,8 @@ int lm_forward_gather(lm_plan* plan, const float* wave, const int64_t* offset, c
     if ((reinterpret_cast<uintptr_t>(out_slice) & 15u) || (reinterpret_cast<uintptr_t>(mc_slice) & 15u)) return LM_ERR_INVALID_ARG;
     for (int r = 0; r < n_peers; ++r)
         if (!peer_slices[r] || (reinterpret_cast<uintptr_t>(peer_slices[r]) & 15u)) return LM_ERR_INVALID_ARG;
-    DeviceOf on(plan->device);
-    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
-    return launch(plan, wave, offset, length, B, aug, noise, out_slice, nullptr, nullptr, 1,
-                  static_cast<cudaStream_t>(cuda_stream), peer_slices, n_peers, mc_slice);
+    return forward_on_device("lm_forward_gather", plan, {wave, false, offset, length, B, aug, noise},
+                             {out_slice, nullptr, nullptr, peer_slices, n_peers, mc_slice}, 1, cuda_stream);
 }
 
 int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, int32_t n_resamplers, const void* wave,
@@ -588,11 +681,9 @@ int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, i
     if (!wave || !offset || !length || !source || !out_norm) return LM_ERR_INVALID_ARG;
     for (int r = 0; r < n_resamplers; ++r)
         if (resamplers[r]->device != plan->device) return LM_ERR_INVALID_ARG;
-    NvtxRange nvtx("lm_forward_resampled");
-    DeviceOf on(plan->device);
-    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
-    return launch(plan, static_cast<const float*>(wave), offset, length, B, aug, noise, out_norm, nullptr, nullptr, normalize,
-                  static_cast<cudaStream_t>(cuda_stream), nullptr, 0, nullptr, pcm16 != 0, source, resamplers, n_resamplers);
+    return forward_on_device("lm_forward_resampled", plan,
+                             {wave, pcm16 != 0, offset, length, B, aug, noise, source, resamplers, n_resamplers}, {out_norm},
+                             normalize, cuda_stream);
 }
 
 int lm_resize_finish(const float* in, int32_t B, int32_t n_mels, int32_t frames_in, int32_t frames_out,
@@ -767,10 +858,6 @@ int lm_pcm16_decode(const int16_t* in, float* out, int64_t n, void* cuda_stream)
     return LM_OK;
 }
 
-static int forward_host_impl(lm_plan* plan, const void* wave_any, bool pcm16, int64_t total_samples, const int64_t* offset,
-                             const int32_t* length, int32_t B, const lm_aug* aug, const float* noise, float* out,
-                             int32_t normalize);
-
 int lm_forward_host(lm_plan* plan, const float* wave, int64_t total_samples, const int64_t* offset,
                     const int32_t* length, int32_t B, const lm_aug* aug, const float* noise, float* out,
                     int32_t normalize) {
@@ -781,90 +868,6 @@ int lm_forward_host_pcm16(lm_plan* plan, const int16_t* pcm, int64_t total_sampl
                           const int32_t* length, int32_t B, const lm_aug* aug, const float* noise, float* out,
                           int32_t normalize) {
     return forward_host_impl(plan, pcm, true, total_samples, offset, length, B, aug, noise, out, normalize);
-}
-
-static int forward_host_impl(lm_plan* plan, const void* wave_any, bool pcm16, int64_t total_samples, const int64_t* offset,
-                             const int32_t* length, int32_t B, const lm_aug* aug, const float* noise, float* out,
-                             int32_t normalize) {
-    const float* wave = static_cast<const float*>(wave_any);
-    const int16_t* pcm = static_cast<const int16_t*>(wave_any);
-    if (!plan || B < 0 || total_samples < 0) return LM_ERR_INVALID_ARG;
-    if (B == 0) return LM_OK;
-    if (!wave || !offset || !length || !out) return LM_ERR_INVALID_ARG;
-    for (int i = 0; i < B; ++i)
-        if (length[i] < 0 || offset[i] < 0 || offset[i] + length[i] > total_samples) return LM_ERR_INVALID_ARG;
-    NvtxRange nvtx(pcm16 ? "lm_forward_host_pcm16" : "lm_forward_host");
-    std::lock_guard<std::mutex> one_caller(plan->host_mu);   // the staging slots belong to the plan
-    DeviceOf on(plan->device);
-    if (on.err) return cuda_fail(on.err, "cudaSetDevice");
-    int rc = ensure_slots(plan);
-    if (rc) return rc;
-
-    const size_t clip_elems = static_cast<size_t>(plan->n_mels) * plan->frames;
-    // chunk so that a few chunks are in flight: ~64 MB of waveform, at least 2 SM-waves of clips
-    const int auto_chunk = std::max(2 * plan->sm_count, static_cast<int>((64u << 20) / (4u * static_cast<size_t>(plan->T))));
-    const int chunk = std::max(1, std::min<int>(B, plan->host_chunk_clips > 0 ? plan->host_chunk_clips : auto_chunk));
-    int slot_i = 0;
-    for (int c0 = 0; c0 < B && rc == LM_OK; c0 += chunk, slot_i = (slot_i + 1) % kSlots) {
-        const int n = std::min(chunk, B - c0);
-        HostSlot& s = plan->slots[slot_i];
-        if ((rc = cudaStreamSynchronize(s.stream) == cudaSuccess ? LM_OK : cuda_fail(cudaGetLastError(), "slot sync"))) break;
-        int64_t lo = INT64_MAX, hi = 0;
-        for (int i = c0; i < c0 + n; ++i) {
-            if (length[i] == 0) continue;
-            lo = std::min(lo, offset[i]);
-            hi = std::max(hi, offset[i] + length[i]);
-        }
-        if (lo == INT64_MAX) { lo = 0; hi = 0; }
-        lo &= ~int64_t(7);   // keep 16-byte alignment of clip starts (TMA staging path; 8 PCM samples per int4)
-        const size_t n_wave = static_cast<size_t>(hi - lo);
-        constexpr size_t kMetaPerClip = sizeof(long long) + sizeof(lm_aug) + sizeof(int);
-        if (n > s.cap_clips) {
-            cudaFree(s.d_meta);
-            if (s.h_meta) cudaFreeHost(s.h_meta);
-            s.d_meta = nullptr; s.h_meta = nullptr; s.cap_clips = 0;
-            if (cudaMalloc(&s.d_meta, kMetaPerClip * n) != cudaSuccess || cudaMallocHost(&s.h_meta, kMetaPerClip * n) != cudaSuccess) {
-                rc = cuda_fail(cudaGetLastError(), "slot metadata alloc");
-                break;
-            }
-            s.cap_clips = n;
-        }
-        // the blocks are laid out for the slot's capacity so that the three arrays keep their alignment
-        const size_t cap = static_cast<size_t>(s.cap_clips);
-        long long* h_off = reinterpret_cast<long long*>(s.h_meta);
-        lm_aug* h_aug = reinterpret_cast<lm_aug*>(s.h_meta + sizeof(long long) * cap);
-        int* h_len = reinterpret_cast<int*>(s.h_meta + (sizeof(long long) + sizeof(lm_aug)) * cap);
-        const long long* d_off = reinterpret_cast<const long long*>(s.d_meta);
-        const lm_aug* d_aug = reinterpret_cast<const lm_aug*>(s.d_meta + sizeof(long long) * cap);
-        const int* d_len = reinterpret_cast<const int*>(s.d_meta + (sizeof(long long) + sizeof(lm_aug)) * cap);
-        if (!pcm16 && (rc = grow(&s.d_wave, &s.cap_wave, std::max<size_t>(n_wave + 8, 16)))) break;
-        if (pcm16 && (rc = grow(&s.d_pcm, &s.cap_pcm, std::max<size_t>(n_wave + 8, 16)))) break;
-        if ((rc = grow(&s.d_out, &s.cap_out, clip_elems * n))) break;
-        if (noise && (rc = grow(&s.d_noise, &s.cap_noise, static_cast<size_t>(plan->T) * n))) break;
-        for (int i = 0; i < n; ++i) h_off[i] = length[c0 + i] ? offset[c0 + i] - lo : 0;
-        memcpy(h_len, length + c0, sizeof(int) * n);
-        if (aug) memcpy(h_aug, aug + c0, sizeof(lm_aug) * n);
-
-        cudaError_t e = cudaMemcpyAsync(s.d_meta, s.h_meta, kMetaPerClip * cap, cudaMemcpyHostToDevice, s.stream);
-        if (e != cudaSuccess) { rc = cuda_fail(e, "H2D copy (metadata)"); break; }
-        if (n_wave && !pcm16) e = cudaMemcpyAsync(s.d_wave, wave + lo, sizeof(float) * n_wave, cudaMemcpyHostToDevice, s.stream);
-        if (n_wave && pcm16) e = cudaMemcpyAsync(s.d_pcm, pcm + lo, sizeof(int16_t) * n_wave, cudaMemcpyHostToDevice, s.stream);
-        if (e == cudaSuccess && noise)
-            e = cudaMemcpyAsync(s.d_noise, noise + static_cast<size_t>(c0) * plan->T, sizeof(float) * plan->T * n,
-                                cudaMemcpyHostToDevice, s.stream);
-        if (e != cudaSuccess) { rc = cuda_fail(e, "H2D copy"); break; }
-        rc = launch(plan, pcm16 ? reinterpret_cast<const float*>(s.d_pcm) : s.d_wave, reinterpret_cast<const int64_t*>(d_off), d_len, n,
-                    aug ? d_aug : nullptr, noise ? s.d_noise : nullptr, s.d_out, nullptr, nullptr, normalize, s.stream, nullptr, 0, nullptr,
-                    pcm16);
-        if (rc) break;
-        e = cudaMemcpyAsync(out + clip_elems * c0, s.d_out, sizeof(float) * clip_elems * n, cudaMemcpyDeviceToHost, s.stream);
-        if (e != cudaSuccess) { rc = cuda_fail(e, "D2H copy"); break; }
-    }
-    for (auto& s : plan->slots) {
-        const cudaError_t e = cudaStreamSynchronize(s.stream);
-        if (e != cudaSuccess && rc == LM_OK) rc = cuda_fail(e, "pipeline drain");
-    }
-    return rc;
 }
 
 }  // extern "C"

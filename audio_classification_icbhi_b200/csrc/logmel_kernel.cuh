@@ -18,8 +18,9 @@
 //           every sample feeds 4 frames.  The contiguous interior of a plain clip is one
 //           cp.async.bulk (TMA, 1-D) completing on an mbarrier; whatever is left -- torch.stft's
 //           reflect padding, zero padding, and whole tiles of augmented clips -- goes through the
-//           gather path that does pad/crop (R/src/data/preprocessing.py:70-83), noise and roll
-//           (:85-93) as index arithmetic.
+//           gather path, one loop (stage_slots) that does pad/crop (R/src/data/preprocessing.py:70-83),
+//           noise and roll (:85-93) as index arithmetic for every sample source: an fp32 or 16-bit
+//           sample of the clip, or one computed by the resampler (lm_forward_resampled).
 //   FFT     x Hann fused with the first butterfly stage (hann[n + n_fft/2] = 1 - hann[n]: one
 //           window load per two samples), 2048 real -> 1024 complex points held as 32
 //           registers/lane; register radix-32 FFT over the lane-local index, twiddle, 32x32
@@ -102,7 +103,7 @@ struct MelTable {                             // lives in global memory, copied 
 
 struct KParams {
     // batch
-    const float* __restrict__ wave;       // PCM16 instantiation: const int16_t* in disguise (offsets count samples either way)
+    const void* __restrict__ wave;        // fp32 samples, int16 for PCM16 and for RESAMPLE with pcm16 (offsets count samples)
     const long long* __restrict__ offset;
     const int* __restrict__ length;
     const lm_aug* __restrict__ aug;
@@ -358,7 +359,7 @@ __device__ __forceinline__ void philox_normal4(uint64_t seed, uint32_t blk, floa
 }
 
 struct ClipCtx;
-// Staging of one tile of a clip with on-device Philox noise (gain, roll, reflect padding as in stage_gather): four
+// Staging of one tile of a clip with on-device Philox noise (gain, roll, reflect padding as in stage_slots): four
 // consecutive slots per thread, so one Philox block serves up to four samples.  Kept out of line: it is the rare
 // path and must not change the register allocation or the code layout of the kernel's main loop.
 __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restrict__ sb, int ns, int need, int j0, int T, int gtid);
@@ -407,7 +408,7 @@ struct Smem {
 // in shared memory (clip ordinal & 1: staging runs one item ahead of the epilogue) so that none of
 // it occupies registers across the FFT.
 struct alignas(16) ClipCtx {
-    const float* src;    // first sample after the centre crop (PCM16: a const short* in disguise)
+    const void* src;     // first sample after the centre crop (fp32, or int16: see KParams::wave)
     const float* nz;     // host-drawn noise row or nullptr
     uint64_t seed;
     int lc;              // valid samples after pad/crop
@@ -419,7 +420,7 @@ struct alignas(16) ClipCtx {
     int t_begin, t_end;  // tile range of this virtual clip
 };
 __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restrict__ sb, int ns, int need, int j0, int T, int gtid) {
-    const float* __restrict__ src = c.src;
+    const float* __restrict__ src = static_cast<const float*>(c.src);
     const int shift = c.shift, lc = c.lc;
     const float gain = c.gain, nscale = c.nscale;
     const uint64_t seed = c.seed;
@@ -450,6 +451,44 @@ __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restric
 }
 constexpr int kCtxSlot = 80;
 static_assert(sizeof(ClipCtx) <= kCtxSlot && kCtxSlot % 16 == 0, "ClipCtx slot size");
+
+// Sample k of clip samples x (fp32, or 16-bit PCM when PCM): its address, and its value as fp32 (x / 32768 for 16-bit
+// PCM, as lm_pcm16_decode).
+template <bool PCM>
+__device__ __forceinline__ const void* sample_addr(const void* x, long long k) {
+    return PCM ? static_cast<const void*>(static_cast<const short*>(x) + k) : static_cast<const float*>(x) + k;
+}
+template <bool PCM>
+__device__ __forceinline__ float clip_sample(const void* x, long long k) {
+    return PCM ? static_cast<float>(__ldg(static_cast<const short*>(x) + k)) * (1.0f / 32768.0f) : __ldg(static_cast<const float*>(x) + k);
+}
+
+// The staging of a tile, slot by slot, for the slots [0, e_lo) and [e_lo + cnt, ns) that the bulk copy does not cover
+// (rest = ns - cnt of them): reflect (torch.stft center=True) -> roll -> pad/crop -> gain, + noise; slots past `need`
+// feed only frames >= `frames` and are zeroed.  `sample(i)` is clip sample i after the crop (i < lc).
+template <class Sample>
+__device__ __forceinline__ void stage_slots(const ClipCtx& c, float* __restrict__ sb, int rest, int e_lo, int cnt, int need, int j0,
+                                            int T, int gtid, Sample sample) {
+    const int shift = c.shift, lc = c.lc;
+    for (int idx = gtid; idx < rest; idx += kGroupThreads) {
+        const int e = idx < e_lo ? idx : idx + cnt;
+        int j = j0 + e;
+        if (j < 0) j = -j;
+        else if (j >= T) j = 2 * (T - 1) - j;
+        float v = 0.0f;
+        if (e < need && j >= 0 && j < T) {
+            int i = j - shift;               // torch.roll: out[j] = in[(j - shift) mod T]
+            if (i < 0) i += T;
+            else if (i >= T) i -= T;
+            if (i < lc) v = sample(i) * c.gain;
+            if (c.nscale != 0.0f) {
+                const float z = c.nz ? __ldg(c.nz + i) : philox_normal(c.seed, static_cast<uint32_t>(i));
+                v = fmaf(z, c.nscale, v);
+            }
+        }
+        sb[e] = v;
+    }
+}
 
 // ---------------------------------------------------------------------------------------
 // Resampling inside the staging (RESAMPLE instantiation, lm_forward_resampled).  Clip i holds len native samples;
@@ -482,10 +521,6 @@ __device__ __forceinline__ RsClip rs_clip(const KParams& p, int clip) {
     return r;
 }
 template <bool PCM>
-__device__ __forceinline__ float rs_in(const void* x, long long k) {
-    return PCM ? static_cast<float>(__ldg(static_cast<const short*>(x) + k)) * (1.0f / 32768.0f) : __ldg(static_cast<const float*>(x) + k);
-}
-template <bool PCM>
 __device__ __forceinline__ float rs_sample(const RsClip& r, const void* x, long long mp) {
     const long long m = mp / r.q;
     const int ph = static_cast<int>(mp - m * r.q);
@@ -496,13 +531,13 @@ __device__ __forceinline__ float rs_sample(const RsClip& r, const void* x, long 
         for (int t = 0; t < r.nt4; ++t) {
             const float4 wv = __ldg(w + t);
             const long long k = base + 4 * t;
-            acc = fmaf(wv.x, rs_in<PCM>(x, k), acc);
-            acc = fmaf(wv.y, rs_in<PCM>(x, k + 1), acc);
-            acc = fmaf(wv.z, rs_in<PCM>(x, k + 2), acc);
-            acc = fmaf(wv.w, rs_in<PCM>(x, k + 3), acc);
+            acc = fmaf(wv.x, clip_sample<PCM>(x, k), acc);
+            acc = fmaf(wv.y, clip_sample<PCM>(x, k + 1), acc);
+            acc = fmaf(wv.z, clip_sample<PCM>(x, k + 2), acc);
+            acc = fmaf(wv.w, clip_sample<PCM>(x, k + 3), acc);
         }
     } else {
-        auto at = [&](long long k) { return (k >= 0 && k < r.len) ? rs_in<PCM>(x, k) : 0.0f; };
+        auto at = [&](long long k) { return (k >= 0 && k < r.len) ? clip_sample<PCM>(x, k) : 0.0f; };
         for (int t = 0; t < r.nt4; ++t) {
             const float4 wv = __ldg(w + t);
             const long long k = base + 4 * t;
@@ -514,30 +549,14 @@ __device__ __forceinline__ float rs_sample(const RsClip& r, const void* x, long 
     }
     return acc;
 }
-// One tile of a clip of lm_forward_resampled: the steps of stage_gather (reflect, roll, i < lc, gain, noise), with the
-// source value computed by rs_sample.  Kept out of line like stage_noisy_tile.
+// One tile of a clip of lm_forward_resampled: stage_slots with the sample computed by rs_sample.  Kept out of line like
+// stage_noisy_tile.
 template <bool PCM>
 __device__ __forceinline__ void stage_resampled_impl(const ClipCtx& c, const RsClip& r, float* __restrict__ sb, int ns, int need,
                                                      int j0, int T, int gtid) {
     const void* x = c.src;
-    const int shift = c.shift, lc = c.lc;
-    for (int e = gtid; e < ns; e += kGroupThreads) {
-        int j = j0 + e;
-        if (j < 0) j = -j;
-        else if (j >= T) j = 2 * (T - 1) - j;
-        float v = 0.0f;
-        if (e < need && j >= 0 && j < T) {
-            int i = j - shift;               // torch.roll: out[j] = in[(j - shift) mod T]
-            if (i < 0) i += T;
-            else if (i >= T) i -= T;
-            if (i < lc) v = (r.q ? rs_sample<PCM>(r, x, r.crop + i) : rs_in<PCM>(x, i)) * c.gain;
-            if (c.nscale != 0.0f) {
-                const float z = c.nz ? __ldg(c.nz + i) : philox_normal(c.seed, static_cast<uint32_t>(i));
-                v = fmaf(z, c.nscale, v);
-            }
-        }
-        sb[e] = v;
-    }
+    stage_slots(c, sb, ns, 0, 0, need, j0, T, gtid,
+                [&](int i) { return r.q ? rs_sample<PCM>(r, x, r.crop + i) : clip_sample<PCM>(x, i); });
 }
 __device__ __noinline__ void stage_resampled_tile(const ClipCtx& c, const RsClip r, int pcm16, float* __restrict__ sb, int ns,
                                                   int need, int j0, int T, int gtid) {
@@ -559,12 +578,12 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     const int crop = len > p.T ? (len - p.T) / 2 : 0;       // centre crop
     c->clip = clip;
     c->lc = len < p.T ? len : p.T;
-    c->src = PCM16 ? reinterpret_cast<const float*>(reinterpret_cast<const short*>(p.wave) + off + crop) : p.wave + off + crop;
+    c->src = sample_addr<PCM16>(p.wave, off + crop);
     if (RESAMPLE) {   // overrides the lines above rather than replacing them: an if / else moved the register allocation of every other instantiation
         const RsClip r = rs_clip(p, clip);
         const long long start = off + (r.q ? 0 : r.crop);
         c->lc = r.lp < p.T ? static_cast<int>(r.lp) : p.T;
-        c->src = p.pcm16 ? reinterpret_cast<const float*>(reinterpret_cast<const short*>(p.wave) + start) : p.wave + start;
+        c->src = p.pcm16 ? sample_addr<true>(p.wave, start) : sample_addr<false>(p.wave, start);
     }
     int shift = 0, f0 = 0, f1 = 0, t0 = 0, t1 = 0;
     float nscale = 0.0f, gain = 1.0f;
@@ -610,6 +629,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
     using G = Geo<NFFT>;
     constexpr int TILE_F = G::TILE_F;
     constexpr int HALF = NFFT / 2;
+    constexpr int ES = PCM16 ? 2 : 4;               // bytes per sample on the bulk-copy path (RESAMPLE never takes it)
     constexpr int NBC = G::NB < 4 ? G::NB : 4;   // MMA column blocks per walk of a mel tile's band
     constexpr int DUNROLL = G::NB > 2 ? 1 : 2;     // unroll of the band walk (n_fft <= 512: 4 blocks per step are enough)
 
@@ -682,15 +702,9 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
         int hi = c->lc - j0;
         if (hi > need) hi = need;
         if (hi <= lo) return;
-        if (PCM16) {   // 16 bytes = 8 samples
-            if ((reinterpret_cast<uintptr_t>(reinterpret_cast<const short*>(c->src) + j0 + lo) & 15u) != 0 || (lo & 3) != 0) return;
-            e_lo = lo;
-            cnt = (hi - lo) & ~7;
-            return;
-        }
-        if ((reinterpret_cast<uintptr_t>(c->src + j0 + lo) & 15u) != 0 || (lo & 3) != 0) return;
+        if ((reinterpret_cast<uintptr_t>(sample_addr<PCM16>(c->src, j0 + lo)) & 15u) != 0 || (lo & 3) != 0) return;
         e_lo = lo;
-        cnt = (hi - lo) & ~3;
+        cnt = (hi - lo) & ~(16 / ES - 1);   // whole 16-byte units
     };
     auto tile_silent = [&](const ClipCtx* __restrict__ c, int tile_) -> bool {   // group-uniform
         return tile_ >= c->silent_from;
@@ -700,15 +714,12 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
         bulk_range(c, tile_, e_lo, cnt);
         if (cnt != 0) {
             const int j0 = tile_ * TILE_F * hop - HALF;
+            const uint32_t bytes = static_cast<uint32_t>(cnt) * ES;
+            // PCM16: raw samples to the end of the buffer; stage_gather expands them in place
+            void* const dst = PCM16 ? static_cast<void*>(reinterpret_cast<unsigned char*>(sb) + 4 * p.ns - bytes) : sb + e_lo;
             fence_proxy_async();
-            if (PCM16) {   // raw samples to the end of the buffer; stage_gather expands them in place
-                mbar_expect_tx(mbar, static_cast<uint32_t>(cnt) * 2u);
-                bulk_g2s(reinterpret_cast<unsigned char*>(sb) + 4 * p.ns - 2 * cnt, reinterpret_cast<const short*>(c->src) + j0 + e_lo,
-                         static_cast<uint32_t>(cnt) * 2u, mbar);
-            } else {
-                mbar_expect_tx(mbar, static_cast<uint32_t>(cnt) * 4u);
-                bulk_g2s(sb + e_lo, c->src + j0 + e_lo, static_cast<uint32_t>(cnt) * 4u, mbar);
-            }
+            mbar_expect_tx(mbar, bytes);
+            bulk_g2s(dst, sample_addr<PCM16>(c->src, j0 + e_lo), bytes, mbar);
         }
         *s_pend = (cnt != 0 ? 1 : 0) | (tile_silent(c, tile_) ? 2 : 0);   // bit 0: bulk copy pending, bit 1: silent tile
     };
@@ -761,31 +772,11 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
             stage_resampled_tile(*cc, rs_clip(p, c.clip), p.pcm16, sb, p.ns, need, j0, T, gtid);
             return true;
         }
-        // reflect (torch.stft center=True) -> roll -> pad/crop -> gain, + noise; slots past `need`
-        // feed only frames >= `frames` and are zeroed
         if (FASTNOISE && c.nscale != 0.0f && c.nz == nullptr && cnt == 0) {   // on-device noise (training batches): out of line
             stage_noisy_tile(*cc, sb, p.ns, need, j0, T, gtid);   // the context in shared memory, not the register copy
             return true;
         }
-        for (int idx = gtid; idx < rest; idx += kGroupThreads) {
-            const int e = idx < e_lo ? idx : idx + cnt;
-            int j = j0 + e;
-            if (j < 0) j = -j;
-            else if (j >= T) j = 2 * (T - 1) - j;
-            float v = 0.0f;
-            if (e < need && j >= 0 && j < T) {
-                int i = j - c.shift;               // torch.roll: out[j] = in[(j - shift) mod T]
-                if (i < 0) i += T;
-                else if (i >= T) i -= T;
-                if (i < c.lc)
-                    v = (PCM16 ? static_cast<float>(__ldg(reinterpret_cast<const short*>(c.src) + i)) * (1.0f / 32768.0f) : __ldg(c.src + i)) * c.gain;
-                if (c.nscale != 0.0f) {
-                    const float z = c.nz ? __ldg(c.nz + i) : philox_normal(c.seed, static_cast<uint32_t>(i));
-                    v = fmaf(z, c.nscale, v);
-                }
-            }
-            sb[e] = v;
-        }
+        stage_slots(c, sb, rest, e_lo, cnt, need, j0, T, gtid, [&](int i) { return clip_sample<PCM16>(c.src, i); });
         return true;
     };
 

@@ -12,6 +12,7 @@ global numpy / torch generators, in the same order, as the reference (see augmen
 """
 from __future__ import annotations
 
+from functools import partial
 from typing import List, Optional, Sequence, Union
 
 import numpy as np
@@ -264,12 +265,16 @@ class AudioPreprocessor:
             noise_d.index_copy_(0, ix.to(plan.device), noise.index_select(0, ix).to(plan.device, non_blocking=True))
         return noise_d
 
-    def _finish(self, plan: LogMelPlan, wave, offset, length, aug, noise, B: int, forward=None) -> torch.Tensor:
-        """Runs the kernel(s).  Overridden by FlexibleAudioPreprocessor when a resize is needed.  `forward` is
-        `plan.forward` or a stand-in with its signature (`plan.forward_resampled` with the rate pairs bound)."""
-        forward = plan.forward if forward is None else forward
-        aug_d = plan.upload_aug(aug) if aug is not None else None
-        return forward(wave, offset, length, aug=aug_d, noise=self._upload_noise(plan, aug, noise))
+    def _upload(self, plan: LogMelPlan, aug, noise):
+        """Host-drawn augmentation records and noise -> device tensors for the kernel (None where there are none)."""
+        return (plan.upload_aug(aug) if aug is not None else None), self._upload_noise(plan, aug, noise)
+
+    def _finish(self, plan: LogMelPlan, forward, aug, noise) -> torch.Tensor:
+        """Runs the kernel(s).  `forward(aug=, noise=, normalize=)` is one kernel call on the packed batch
+        (`plan.forward` or `plan.forward_resampled` with the clips bound).  Overridden by FlexibleAudioPreprocessor
+        when a resize is needed."""
+        aug_d, noise_d = self._upload(plan, aug, noise)
+        return forward(aug=aug_d, noise=noise_d)
 
     def preprocess_batch(self, waveforms: Union[Sequence[Wave], torch.Tensor],
                          lengths: Optional[Sequence[int]] = None, fast_augment: bool = False,
@@ -280,24 +285,37 @@ class AudioPreprocessor:
         log-mel kernel (`LogMelPlan.forward_resampled`, at most LM_MAX_RESAMPLERS distinct foreign rates per batch),
         with the same result as `resample_to_target` on each of them first.
         Returns `[B, 1, n_mels, frames]` float32 on the GPU."""
-        if sample_rates is not None and any(int(r) != int(self.sample_rate) for r in sample_rates):
-            return self._preprocess_resampled(waveforms, lengths, fast_augment, sample_rates)
         plan = self.plan
-        dev = plan.device
-        if isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2:
+        rate = int(self.sample_rate)
+        rates = [] if sample_rates is None else [int(r) for r in sample_rates]
+        foreign = sorted({r for r in rates if r != rate})
+        dense = isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2
+        if dense:
             B, n = waveforms.shape
-            wave = waveforms.to(device=dev, dtype=torch.float32).contiguous().view(-1)
-            offset = torch.arange(B, device=dev, dtype=torch.int64) * n
             lens = torch.full((B,), n, dtype=torch.int32) if lengths is None else torch.as_tensor(lengths, dtype=torch.int32)
             if int(lens.max()) > n:
                 raise ValueError("lengths exceed the row length")
-            length = lens.to(dev)
+        if dense and not foreign:   # the rows are the packed clips: no copy
+            wave = waveforms.to(device=plan.device, dtype=torch.float32).contiguous().view(-1)
+            offset = torch.arange(B, device=plan.device, dtype=torch.int64) * n
+            length = lens.to(plan.device)
         else:
-            clips = [_as_mono_1d(w) for w in waveforms]
+            keep = lens.tolist() if dense else None
+            clips = [waveforms[i, :keep[i]].to(torch.float32) for i in range(B)] if dense else [_as_mono_1d(w) for w in waveforms]
             B = len(clips)
             wave, offset, length = self._pack(clips)
+        forward = partial(plan.forward, wave, offset, length)
+        if foreign:
+            if len(rates) != B:
+                raise ValueError("sample_rates must give one rate per waveform")
+            if len(foreign) > _lib.LM_MAX_RESAMPLERS:
+                raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} sample rates other than {self.sample_rate} per batch")
+            from .resample import get_resampler
+            source = torch.tensor([foreign.index(r) if r != rate else -1 for r in rates], dtype=torch.int32)
+            forward = partial(plan.forward_resampled, wave, offset, length, source=source,
+                              resamplers=[get_resampler(r, rate, plan.device) for r in foreign])
         aug, noise = self._draw(B, fast_augment)
-        return self._finish(plan, wave, offset, length, aug, noise, B)
+        return self._finish(plan, forward, aug, noise)
 
     def _pack(self, clips: List[torch.Tensor]):
         """1-D fp32 clips (host or device) -> (packed device samples, offset int64, length int32) on the plan's device."""
@@ -326,34 +344,6 @@ class AudioPreprocessor:
         offset = torch.tensor(starts, dtype=torch.int64).to(dev, non_blocking=True)
         length = torch.tensor(lens, dtype=torch.int32).to(dev, non_blocking=True)
         return packed, offset, length
-
-    def _preprocess_resampled(self, waveforms, lengths, fast_augment: bool, sample_rates) -> torch.Tensor:
-        """`preprocess_batch` for a batch with clips at other rates: native-rate clips packed as usual, then ONE
-        `forward_resampled` launch (through `_finish`, so the flexible resize path applies too)."""
-        from functools import partial
-        from .resample import get_resampler
-        plan = self.plan
-        if isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2:
-            n = waveforms.shape[1]
-            lens = [n] * waveforms.shape[0] if lengths is None else [int(x) for x in lengths]
-            if max(lens, default=0) > n:
-                raise ValueError("lengths exceed the row length")
-            clips = [waveforms[i, :lens[i]].to(torch.float32) for i in range(waveforms.shape[0])]
-        else:
-            clips = [_as_mono_1d(w) for w in waveforms]
-        B = len(clips)
-        rates = [int(r) for r in sample_rates]
-        if len(rates) != B:
-            raise ValueError("sample_rates must give one rate per waveform")
-        foreign = sorted({r for r in rates if r != int(self.sample_rate)})
-        if len(foreign) > _lib.LM_MAX_RESAMPLERS:
-            raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} sample rates other than {self.sample_rate} per batch")
-        resamplers = [get_resampler(r, int(self.sample_rate), plan.device) for r in foreign]
-        source = torch.tensor([foreign.index(r) if r != int(self.sample_rate) else -1 for r in rates], dtype=torch.int32)
-        wave, offset, length = self._pack(clips)
-        aug, noise = self._draw(B, fast_augment)
-        forward = partial(plan.forward_resampled, source=source, resamplers=resamplers)
-        return self._finish(plan, wave, offset, length, aug, noise, B, forward=forward)
 
     def preprocess_waveform(self, waveform: Wave) -> torch.Tensor:
         """One in-memory waveform -> `[1, n_mels, frames]` float32 CPU tensor (what `preprocess`

@@ -73,18 +73,16 @@ class FlexibleAudioPreprocessor(AudioPreprocessor):
                                         1 if normalize else 0, 1e-8, C.c_void_p(stream)))
         return out
 
-    def _finish(self, plan: LogMelPlan, wave, offset, length, aug, noise, B: int, forward=None) -> torch.Tensor:
+    def _finish(self, plan: LogMelPlan, forward, aug, noise) -> torch.Tensor:
         fout = self.target_time_steps()
         if plan.frames == fout:
-            return super()._finish(plan, wave, offset, length, aug, noise, B, forward=forward)
-        forward = plan.forward if forward is None else forward
+            return super()._finish(plan, forward, aug, noise)
         # fused kernel up to dB with the waveform augmentation only; masks act on the resized map
-        aug_d = plan.upload_aug(aug) if aug is not None else None
-        wave_aug_d = None
+        aug_d = wave_aug = None
         if aug is not None:
-            wa = aug.copy()
-            wa["f0"] = wa["f1"] = wa["t0"] = wa["t1"] = 0
-            wave_aug_d = plan.upload_aug(wa)
-        noise_d = self._upload_noise(plan, aug, noise)
-        db = forward(wave, offset, length, aug=wave_aug_d, noise=noise_d, normalize=False)
+            aug_d = plan.upload_aug(aug)
+            wave_aug = aug.copy()
+            wave_aug["f0"] = wave_aug["f1"] = wave_aug["t0"] = wave_aug["t1"] = 0
+        wave_aug_d, noise_d = self._upload(plan, wave_aug, noise)
+        db = forward(aug=wave_aug_d, noise=noise_d, normalize=False)
         return self._resize_finish(db, fout, aug_d, normalize=True)

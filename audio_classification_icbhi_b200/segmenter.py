@@ -12,6 +12,7 @@ pairs into the one uploaded recording, with no intermediate files.
 from __future__ import annotations
 
 import json
+from functools import partial
 from pathlib import Path
 from typing import List, Tuple
 
@@ -127,7 +128,7 @@ class ICBHISegmenter:
         rec = torch.from_numpy(audio).to(plan.device)
         offset = torch.tensor([t[1] for t in table], dtype=torch.int64, device=plan.device)
         length = torch.tensor([t[2] for t in table], dtype=torch.int32, device=plan.device)
-        feats = preprocessor._finish(plan, rec, offset, length, None, None, len(table))
+        feats = preprocessor._finish(plan, partial(plan.forward, rec, offset, length), None, None)
         return feats, [t[3] for t in table]
 
     def process_all(self):
