@@ -6,10 +6,10 @@ segmenter callers).  All arithmetic of the path runs in hand-written CUDA behind
 (include/logmel_b200.h); there is no CPU fallback.  `compat/` at the repository root holds import
 shims under the reference's own module paths.
 """
-from .plan import LogMelPlan, make_aug_array, reference_filterbank, reference_window
+from .plan import LogMelPlan, clip_span, make_aug_array, reference_filterbank, reference_window
 from .preprocessing import AudioPreprocessor
 from .preprocessing_flexible import FlexibleAudioPreprocessor
-from .dataset import GpuCollate, GpuLoader, ICBHIDataset, ICBHISegmentedDataset, raw_collate
+from .dataset import GpuCollate, GpuLoader, ICBHIDataset, ICBHISegmentedDataset, SpanItem, raw_collate
 from .analyzer import SlidingWindowLogMel, segment_offsets
 from .segmenter import ICBHISegmenter
 from .sharding import FusedGather, ShardedLogMel, shard_bounds, shard_size
@@ -17,9 +17,9 @@ from .augment import draw_fast_augmentation, draw_reference_augmentation
 from .resample import Resampler, get_resampler
 
 __all__ = [
-    "LogMelPlan", "make_aug_array", "reference_filterbank", "reference_window",
+    "LogMelPlan", "clip_span", "make_aug_array", "reference_filterbank", "reference_window",
     "AudioPreprocessor", "FlexibleAudioPreprocessor",
-    "ICBHIDataset", "ICBHISegmentedDataset", "GpuCollate", "GpuLoader", "raw_collate",
+    "ICBHIDataset", "ICBHISegmentedDataset", "GpuCollate", "GpuLoader", "raw_collate", "SpanItem",
     "SlidingWindowLogMel", "segment_offsets", "ICBHISegmenter",
     "ShardedLogMel", "FusedGather", "shard_bounds", "shard_size",
     "draw_fast_augmentation", "draw_reference_augmentation",

@@ -78,6 +78,10 @@ EXPORTS = {
                                    C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
     "lm_forward_resampled": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
                                        C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p]),
+    "lm_clip_span": (C.c_int, [C.c_int32, C.c_int32, C.c_int32, C.c_int64, C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "lm_forward_spans": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p,
+                                   C.c_int32, C.c_void_p]),
 }
 
 _lib = None

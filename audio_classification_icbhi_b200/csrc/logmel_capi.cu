@@ -224,11 +224,13 @@ void choose_split(const lm_plan* p, int B, int groups, bool normalize, int* spli
 // A batch as the kernel reads it: clip i is samples [offset[i], offset[i] + length[i]), fp32 or, when pcm16, 16-bit PCM
 // expanded to x / 32768 inside the staging (no decode kernel).  lm_forward_resampled adds the rate of each clip: that of
 // resamplers[source[i]], or the plan's rate for -1.
+// lm_forward_spans adds the stored span of each clip: native samples [first[i], first[i] + stored[i]) from offset[i] on.
 struct Batch {
     const void* samples; bool pcm16;
     const int64_t* offset; const int32_t* length; int32_t B;
     const lm_aug* aug; const float* noise;
     const int32_t* source = nullptr; const lm_resampler* const* resamplers = nullptr; int n_resamplers = 0;
+    const int64_t* first = nullptr; const int32_t* stored = nullptr;
 };
 
 // Where the features go: `norm` always, dB and mel power when given.  lm_forward_gather also stores the normalised
@@ -254,6 +256,7 @@ int launch(lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, cuda
         k.rs_taps4[r] = rs->d_taps4; k.rs_k0[r] = rs->d_k0;
         k.rs_o[r] = rs->orig; k.rs_q[r] = rs->neu; k.rs_nt4[r] = rs->nt4; k.rs_width[r] = rs->width;
     }
+    k.first = reinterpret_cast<const long long*>(b.first); k.stored = b.stored;
     const long long seq = p->launches.fetch_add(1);
     k.work_counter = p->d_counters + 2 * (seq % kCounters);   // zero now, left at zero by the kernel (no memset per launch)
     const int cap = p->max_ctas > 0 ? p->max_ctas : p->sm_count;
@@ -534,6 +537,59 @@ int forward_host_impl(lm_plan* plan, const void* wave, bool pcm16, int64_t total
     return rc;
 }
 
+// The polyphase taps of one rate pair and their geometry: rates divided by their gcd (o -> q), `width`, per phase the
+// first kept tap k0 and ntaps taps (nt4 float4 once padded).  Host arithmetic only: lm_resampler_create uploads the
+// tables, lm_clip_span derives the samples a clip's features read from the same k0 / width / nt4.
+struct RsDesign {
+    int o = 1, q = 1, width = 0, ntaps = 1, nt4 = 1;
+    std::vector<float> taps;   // [q][ntaps]
+    std::vector<int> k0;       // [q]
+};
+
+RsDesign rs_design(int orig_freq, int new_freq) {
+    RsDesign d;
+    int a = orig_freq, b = new_freq;
+    while (b) { const int t = a % b; a = b; b = t; }
+    const int o = orig_freq / a, q = new_freq / a;
+    // TA/functional/functional.py _get_sinc_resample_kernel with lowpass_filter_width = 6, rolloff = 0.99,
+    // sinc_interp_hann, float64 index arithmetic, kernel rounded to float32 at the end
+    const int lpw = 6;
+    const double base_freq = std::min(o, q) * 0.99;
+    const int width = static_cast<int>(ceil(lpw * o / base_freq));
+    const int K = 2 * width + o;
+    const double pi = 3.14159265358979323846;
+    std::vector<float> dense(static_cast<size_t>(q) * K);
+    for (int p = 0; p < q; ++p)
+        for (int k = 0; k < K; ++k) {
+            double t = (static_cast<double>(-p) / q + static_cast<double>(k - width) / o) * base_freq;
+            t = std::min(std::max(t, -static_cast<double>(lpw)), static_cast<double>(lpw));
+            const double c = cos(t * pi / lpw / 2.0);
+            const double window = c * c;
+            const double tp = t * pi;
+            const double sinc = (tp == 0.0) ? 1.0 : sin(tp) / tp;
+            dense[static_cast<size_t>(p) * K + k] = static_cast<float>(sinc * window * (base_freq / o));
+        }
+    // per phase keep the taps that are not negligible (|w| > 1e-12: the clamped tails are ~1e-33)
+    int ntaps = 1;
+    std::vector<int> k0(q), k1(q);
+    for (int p = 0; p < q; ++p) {
+        int lo = K, hi = -1;
+        for (int k = 0; k < K; ++k)
+            if (fabsf(dense[static_cast<size_t>(p) * K + k]) > 1e-12f) { lo = std::min(lo, k); hi = k; }
+        if (hi < 0) { lo = 0; hi = 0; }
+        k0[p] = lo; k1[p] = hi;
+        ntaps = std::max(ntaps, hi - lo + 1);
+    }
+    std::vector<float> taps(static_cast<size_t>(q) * ntaps, 0.0f);
+    for (int p = 0; p < q; ++p) {
+        if (k0[p] + ntaps > K) k0[p] = std::max(0, K - ntaps);
+        for (int i = 0; i < ntaps && k0[p] + i < K; ++i) taps[static_cast<size_t>(p) * ntaps + i] = dense[static_cast<size_t>(p) * K + k0[p] + i];
+    }
+    d.o = o; d.q = q; d.width = width; d.ntaps = ntaps; d.nt4 = (ntaps + 3) / 4;
+    d.taps = std::move(taps); d.k0 = std::move(k0);
+    return d;
+}
+
 }  // namespace
 
 extern "C" {
@@ -686,6 +742,44 @@ int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, i
                              normalize, cuda_stream);
 }
 
+int lm_clip_span(int32_t orig_freq, int32_t new_freq, int32_t target_len, int64_t length, int64_t* first, int64_t* count) {
+    if (orig_freq < 1 || new_freq < 1 || target_len < 1 || length < 0 || !first || !count) return LM_ERR_INVALID_ARG;
+    long long lo = 0, hi = 0;
+    if (orig_freq == new_freq) {   // no resampling: the pad / centre-crop span
+        lo = length > target_len ? (length - target_len) / 2 : 0;
+        hi = lo + std::min<int64_t>(length, target_len);
+    } else {
+        // a worker asks once per item: keep each rate pair's design (per thread, so no lock is held across a fork)
+        thread_local std::map<std::pair<int, int>, RsDesign> designs;
+        auto it = designs.find(std::make_pair(orig_freq, new_freq));
+        if (it == designs.end()) it = designs.emplace(std::make_pair(orig_freq, new_freq), rs_design(orig_freq, new_freq)).first;
+        const RsDesign& d = it->second;
+        lm::rs_read_span(d.k0.data(), d.o, d.q, d.width, d.nt4, length, target_len, &lo, &hi);
+    }
+    *first = lo;
+    *count = hi - lo;
+    return LM_OK;
+}
+
+int lm_forward_spans(lm_plan* plan, const lm_resampler* const* resamplers, int32_t n_resamplers, const void* wave,
+                     int32_t pcm16, const int64_t* offset, const int64_t* first, const int32_t* stored,
+                     const int32_t* length, const int32_t* source, int32_t B, const lm_aug* aug, const float* noise,
+                     float* out_norm, int32_t normalize, void* cuda_stream) {
+    // the checks and their order are lm_forward_resampled's
+    if (!plan || B < 0 || n_resamplers < 0 || n_resamplers > LM_MAX_RESAMPLERS || (n_resamplers > 0 && !resamplers) ||
+        (pcm16 != 0 && pcm16 != 1))
+        return LM_ERR_INVALID_ARG;
+    for (int r = 0; r < n_resamplers; ++r)
+        if (!resamplers[r]) return LM_ERR_INVALID_ARG;
+    if (B == 0) return LM_OK;
+    if (!wave || !offset || !first || !stored || !length || !source || !out_norm) return LM_ERR_INVALID_ARG;
+    for (int r = 0; r < n_resamplers; ++r)
+        if (resamplers[r]->device != plan->device) return LM_ERR_INVALID_ARG;
+    Batch b{wave, pcm16 != 0, offset, length, B, aug, noise, source, resamplers, n_resamplers};
+    b.first = first; b.stored = stored;
+    return forward_on_device("lm_forward_spans", plan, b, {out_norm}, normalize, cuda_stream);
+}
+
 int lm_resize_finish(const float* in, int32_t B, int32_t n_mels, int32_t frames_in, int32_t frames_out,
                      const lm_aug* aug, float* out, int32_t normalize, float norm_eps, void* cuda_stream) {
     if (B < 0 || n_mels < 1 || frames_in < 1 || frames_out < 1) return LM_ERR_INVALID_ARG;
@@ -719,47 +813,14 @@ int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resa
     }
     DeviceOf on(device);
     if (on.err) return cuda_fail(on.err, "cudaSetDevice");
-    int a = orig_freq, b = new_freq;
-    while (b) { const int t = a % b; a = b; b = t; }
-    const int o = orig_freq / a, q = new_freq / a;
-    // TA/functional/functional.py _get_sinc_resample_kernel with lowpass_filter_width = 6, rolloff = 0.99,
-    // sinc_interp_hann, float64 index arithmetic, kernel rounded to float32 at the end
-    const int lpw = 6;
-    const double base_freq = std::min(o, q) * 0.99;
-    const int width = static_cast<int>(ceil(lpw * o / base_freq));
-    const int K = 2 * width + o;
-    const double pi = 3.14159265358979323846;
-    std::vector<float> dense(static_cast<size_t>(q) * K);
-    for (int p = 0; p < q; ++p)
-        for (int k = 0; k < K; ++k) {
-            double t = (static_cast<double>(-p) / q + static_cast<double>(k - width) / o) * base_freq;
-            t = std::min(std::max(t, -static_cast<double>(lpw)), static_cast<double>(lpw));
-            const double c = cos(t * pi / lpw / 2.0);
-            const double window = c * c;
-            const double tp = t * pi;
-            const double sinc = (tp == 0.0) ? 1.0 : sin(tp) / tp;
-            dense[static_cast<size_t>(p) * K + k] = static_cast<float>(sinc * window * (base_freq / o));
-        }
-    // per phase keep the taps that are not negligible (|w| > 1e-12: the clamped tails are ~1e-33)
-    int ntaps = 1;
-    std::vector<int> k0(q), k1(q);
-    for (int p = 0; p < q; ++p) {
-        int lo = K, hi = -1;
-        for (int k = 0; k < K; ++k)
-            if (fabsf(dense[static_cast<size_t>(p) * K + k]) > 1e-12f) { lo = std::min(lo, k); hi = k; }
-        if (hi < 0) { lo = 0; hi = 0; }
-        k0[p] = lo; k1[p] = hi;
-        ntaps = std::max(ntaps, hi - lo + 1);
-    }
-    std::vector<float> taps(static_cast<size_t>(q) * ntaps, 0.0f);
-    for (int p = 0; p < q; ++p) {
-        if (k0[p] + ntaps > K) k0[p] = std::max(0, K - ntaps);
-        for (int i = 0; i < ntaps && k0[p] + i < K; ++i) taps[static_cast<size_t>(p) * ntaps + i] = dense[static_cast<size_t>(p) * K + k0[p] + i];
-    }
+    const RsDesign d = rs_design(orig_freq, new_freq);
+    const int o = d.o, q = d.q, ntaps = d.ntaps;
+    const std::vector<float>& taps = d.taps;
+    const std::vector<int>& k0 = d.k0;
     lm_resampler* r = new (std::nothrow) lm_resampler();
     if (!r) return LM_ERR_INVALID_ARG;
-    r->device = device; r->orig = o; r->neu = q; r->width = width; r->ntaps = ntaps;
-    r->nt4 = (ntaps + 3) / 4;
+    r->device = device; r->orig = o; r->neu = q; r->width = d.width; r->ntaps = ntaps;
+    r->nt4 = d.nt4;
     r->k0max = *std::max_element(k0.begin(), k0.end());
     std::vector<float> taps4(static_cast<size_t>(q) * r->nt4 * 4, 0.0f);
     for (int p = 0; p < q; ++p)

@@ -20,7 +20,8 @@
 //           reflect padding, zero padding, and whole tiles of augmented clips -- goes through the
 //           gather path, one loop (stage_slots) that does pad/crop (R/src/data/preprocessing.py:70-83),
 //           noise and roll (:85-93) as index arithmetic for every sample source: an fp32 or 16-bit
-//           sample of the clip, or one computed by the resampler (lm_forward_resampled).
+//           sample of the clip, or one computed by the resampler (lm_forward_resampled; lm_forward_spans when only the
+//           native samples a clip's features read are stored: rs_read_span is that set, the same code on host and device).
 //   FFT     x Hann fused with the first butterfly stage (hann[n + n_fft/2] = 1 - hann[n]: one
 //           window load per two samples), 2048 real -> 1024 complex points held as 32
 //           registers/lane; register radix-32 FFT over the lane-local index, twiddle, 32x32
@@ -155,6 +156,10 @@ struct KParams {
     const float4* rs_taps4[LM_MAX_RESAMPLERS];
     const int* rs_k0[LM_MAX_RESAMPLERS];
     int rs_o[LM_MAX_RESAMPLERS], rs_q[LM_MAX_RESAMPLERS], rs_nt4[LM_MAX_RESAMPLERS], rs_width[LM_MAX_RESAMPLERS];
+    // lm_forward_spans (RESAMPLE instantiation): clip i stores only its native samples [first[i], first[i] + stored[i]),
+    // starting at wave + offset[i]; length[i] is still the whole clip's.  Null for lm_forward_resampled.
+    const long long* __restrict__ first;
+    const int* __restrict__ stored;
 };
 
 // ---------------------------------------------------------------------------------------
@@ -497,6 +502,9 @@ __device__ __forceinline__ void stage_slots(const ClipCtx& c, float* __restrict_
 // is the tiled resampler's chain: acc = fmaf(taps4[ph][t], x[m o + k0[ph] - width + t], acc) for t < 4 nt4, x = 0
 // outside [0, len) -- the same taps, the same order and the same zero-padded tail, hence bit-identical to lm_resample.
 // ClipCtx has no room for the rate pair: the staging reads source / length / offset of the clip again per tile.
+// lm_forward_spans stores only native samples [first, first + stored) of a clip: ClipCtx::src is then wave + offset - first
+// (+ crop for a clip at the plan's rate), so x[k] is read where it is stored; lc, the crop, L' and the silent tiles still
+// come from the whole clip's length.
 // ---------------------------------------------------------------------------------------
 struct RsClip {
     const float4* taps4;
@@ -549,6 +557,47 @@ __device__ __forceinline__ float rs_sample(const RsClip& r, const void* x, long 
     }
     return acc;
 }
+// The native samples [*lo, *hi) that the staging of a resampled clip of len samples reads (lm_clip_span): every x[k],
+// 0 <= k < len, that the chain of an output y[crop + i], i < lc, touches, zero padding taps included (a non-finite sample
+// under a zero tap still poisons the sum).  Empty: *lo == *hi == 0.  For one phase the tap window moves right with m, so
+// the lowest index comes from the first q outputs of the crop and the highest from the last q; the windows of
+// neighbouring outputs overlap, so the indices in between are all read.  Host (lm_clip_span) and device (the
+// lm_forward_spans check) run this same code on the same k0 table.
+__host__ __device__ inline void rs_read_span(const int* k0, int o, int q, int width, int nt4, long long len, int T,
+                                             long long* lo, long long* hi) {
+    const long long lp = (static_cast<long long>(q) * len + o - 1) / o;
+    const long long lc = lp < T ? lp : T, crop = lp > T ? (lp - T) / 2 : 0;
+    *lo = 0; *hi = 0;
+    if (lc <= 0) return;
+    const int n = lc < q ? static_cast<int>(lc) : q;
+    long long a = 0, b = 0;
+    for (int side = 0; side < 2; ++side) {
+        const long long mp0 = side ? crop + lc - n : crop;
+        long long m = mp0 / q;
+        int ph = static_cast<int>(mp0 - m * q);
+        for (int j = 0; j < n; ++j) {
+            const long long base = m * o + k0[ph] - width;
+            if (side == 0 && (j == 0 || base < a)) a = base;
+            if (side == 1 && (j == 0 || base + 4 * nt4 > b)) b = base + 4 * nt4;
+            if (++ph == q) { ph = 0; ++m; }
+        }
+    }
+    if (a < 0) a = 0;
+    if (b > len) b = len;
+    if (b > a) { *lo = a; *hi = b; }
+}
+
+// lm_forward_spans: whether the stored span [f, f + stored) holds every native sample the staging of a clip reads: the
+// resampler's read set (rs_read_span), or for a clip at the plan's rate (q == 0) its lc samples from the crop on.  Once
+// per clip, by one thread.  Inline: as an out-of-line call from load_clip it cost the RESAMPLE instantiations 32-56 bytes
+// of stack and spills across the call.
+__device__ __forceinline__ bool span_stored(const int* k0, int o, int q, int width, int nt4, long long len, long long crop,
+                                         int lc, int T, long long f, int stored) {
+    long long lo = crop, hi = crop + lc;
+    if (q) rs_read_span(k0, o, q, width, nt4, len, T, &lo, &hi);
+    return hi <= lo || (f <= lo && hi <= f + stored);
+}
+
 // One tile of a clip of lm_forward_resampled: stage_slots with the sample computed by rs_sample.  Kept out of line like
 // stage_noisy_tile.
 template <bool PCM>
@@ -567,7 +616,8 @@ __device__ __noinline__ void stage_resampled_tile(const ClipCtx& c, const RsClip
 // `nfft` is NFFT passed as a value: with the compile-time constant in the padded-signal bounds below, the compiler
 // reassociates them and the churn that follows through the whole kernel measured 0.1-0.2 % slower at n_fft = 512.
 // RESAMPLE: lc = min(L', T) and src is the clip's first native sample, or its first sample after the crop for a clip at
-// the plan's rate (rs_clip); `plain` then only decides silent tiles, the staging never takes the bulk-copy path.
+// the plan's rate (rs_clip); `plain` then only decides silent tiles, the staging never takes the bulk-copy path.  With
+// stored spans (lm_forward_spans) a clip whose span misses a sample the staging reads gets lc = 0: a zero-length clip.
 template <int NFFT, bool PCM16, bool RESAMPLE = false>
 __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* __restrict__ c, int nfft) {
     const int clip = vclip / p.split, chunk = vclip - clip * p.split;
@@ -581,8 +631,14 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     c->src = sample_addr<PCM16>(p.wave, off + crop);
     if (RESAMPLE) {   // overrides the lines above rather than replacing them: an if / else moved the register allocation of every other instantiation
         const RsClip r = rs_clip(p, clip);
-        const long long start = off + (r.q ? 0 : r.crop);
+        long long start = off + (r.q ? 0 : r.crop);
         c->lc = r.lp < p.T ? static_cast<int>(r.lp) : p.T;
+        if (p.first != nullptr) {   // lm_forward_spans: native sample k sits at wave[offset + k - first]
+            const long long f = p.first[clip];
+            if (!span_stored(r.k0, r.o, r.q, r.width, r.nt4, r.len, r.crop, c->lc, p.T, f, p.stored[clip]))
+                c->lc = 0;   // a sample the staging needs is not stored: a zero-length clip, nothing is read
+            start -= f;
+        }
         c->src = p.pcm16 ? sample_addr<true>(p.wave, start) : sample_addr<false>(p.wave, start);
     }
     int shift = 0, f0 = 0, f1 = 0, t0 = 0, t1 = 0;

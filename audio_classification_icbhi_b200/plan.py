@@ -18,7 +18,7 @@ import torch
 
 from . import _lib
 
-__all__ = ["LogMelPlan", "reference_window", "reference_filterbank", "make_aug_array"]
+__all__ = ["LogMelPlan", "reference_window", "reference_filterbank", "make_aug_array", "clip_span"]
 
 
 def reference_window(n_fft: int) -> torch.Tensor:
@@ -55,6 +55,16 @@ def make_aug_array(n: int) -> np.ndarray:
     a = np.zeros(n, dtype=_lib.AUG_DTYPE)
     a["gain"] = 1.0
     return a
+
+
+def clip_span(orig_freq: int, new_freq: int, target_len: int, length: int) -> Tuple[int, int]:
+    """(first, count): the native samples [first, first + count) that the features of a clip of `length` samples at
+    `orig_freq` read when a plan at `new_freq` crops to `target_len` (`lm_clip_span`).  Host arithmetic only -- no
+    GPU, no CUDA call -- so DataLoader workers can read just those samples from a file for `forward_spans`."""
+    first, count = C.c_int64(), C.c_int64()
+    _lib.check(_lib.load().lm_clip_span(int(orig_freq), int(new_freq), int(target_len), int(length),
+                                        C.byref(first), C.byref(count)))
+    return first.value, count.value
 
 
 def _ptr(t: Optional[torch.Tensor]) -> Optional[int]:
@@ -193,6 +203,39 @@ class LogMelPlan:
         index into `resamplers` (`Resampler(clip_rate, plan.sample_rate)`, at most LM_MAX_RESAMPLERS), or -1 for a clip
         already at the plan's rate.  Bit-identical to resampling each clip with its `Resampler`, packing the results
         and calling `forward` (`forward_pcm16` for int16 clips with source -1)."""
+        B, (handles, n_rs), source, out = self._check_resampled_inputs(wave, offset, length, source, resamplers, aug, noise,
+                                                                      out)
+        s = torch.cuda.current_stream(self.device) if stream is None else stream
+        _lib.check(self._lib.lm_forward_resampled(self._h, handles, n_rs, wave.data_ptr(),
+                                                  1 if wave.dtype == torch.int16 else 0, offset.data_ptr(), length.data_ptr(),
+                                                  source.data_ptr(), B, _ptr(aug), _ptr(noise), out.data_ptr(),
+                                                  1 if normalize else 0, C.c_void_p(s.cuda_stream)))
+        return out
+
+    def forward_spans(self, wave: torch.Tensor, offset: torch.Tensor, first: torch.Tensor, stored: torch.Tensor,
+                      length: torch.Tensor, source: torch.Tensor, resamplers: Sequence["Resampler"],
+                      aug: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None, normalize: bool = True,
+                      out: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """`forward_resampled` on clips of which only a span of native samples is stored: clip i has `length[i]`
+        samples, of which [first[i], first[i] + stored[i]) sit at wave[offset[i] ...].  `first` int64 [B] and `stored`
+        int32 [B] live on the plan's device.  When every stored span contains `clip_span(clip rate, plan rate,
+        target_length, length[i])`, the output is bit-identical to `forward_resampled` on the whole clips; a clip whose
+        stored span misses a sample it needs comes out as a zero-length clip, and nothing outside the spans is read."""
+        B, (handles, n_rs), source, out = self._check_resampled_inputs(wave, offset, length, source, resamplers, aug, noise,
+                                                                      out)
+        for name, t, dt in (("first", first, torch.int64), ("stored", stored, torch.int32)):
+            if t.device != self.device or t.dtype != dt or not t.is_contiguous() or t.numel() != B:
+                raise ValueError(f"{name} must be a contiguous {dt} [B] tensor on {self.device}")
+        s = torch.cuda.current_stream(self.device) if stream is None else stream
+        _lib.check(self._lib.lm_forward_spans(self._h, handles, n_rs, wave.data_ptr(),
+                                              1 if wave.dtype == torch.int16 else 0, offset.data_ptr(), first.data_ptr(),
+                                              stored.data_ptr(), length.data_ptr(), source.data_ptr(), B, _ptr(aug),
+                                              _ptr(noise), out.data_ptr(), 1 if normalize else 0, C.c_void_p(s.cuda_stream)))
+        return out
+
+    def _check_resampled_inputs(self, wave, offset, length, source, resamplers, aug, noise, out):
+        """The checks of `forward_resampled` / `forward_spans` (ValueError); returns B, (resampler handles, their number),
+        `source` on the device and the output tensor."""
         if wave.dtype not in (torch.float32, torch.int16):
             raise ValueError("wave must be fp32 samples or int16 PCM")
         B = self._check_device_inputs(("wave", wave, wave.dtype), offset, length, aug, noise, (("out", out),))
@@ -215,12 +258,7 @@ class LogMelPlan:
         if out is None:
             out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
         handles = (C.c_void_p * max(len(resamplers), 1))(*[r._h.value for r in resamplers])
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
-        _lib.check(self._lib.lm_forward_resampled(self._h, handles, len(resamplers), wave.data_ptr(),
-                                                  1 if wave.dtype == torch.int16 else 0, offset.data_ptr(), length.data_ptr(),
-                                                  source.data_ptr(), B, _ptr(aug), _ptr(noise), out.data_ptr(),
-                                                  1 if normalize else 0, C.c_void_p(s.cuda_stream)))
-        return out
+        return B, (handles, len(resamplers)), source, out
 
     def forward_gather(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor, out_slice_ptr: int,
                        peer_slice_ptrs=(), mc_slice_ptr: int = 0, aug: Optional[torch.Tensor] = None,

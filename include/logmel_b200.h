@@ -216,6 +216,36 @@ int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, i
                          float* out_norm, int32_t normalize, void* cuda_stream);
 
 /*
+ * Training batches need not carry whole recordings: which native samples a clip's features read is fixed by its length,
+ * its rate pair and target_len (roll, noise, gain, reflect padding and masks all act inside the crop).  A data-loading
+ * worker asks lm_clip_span for that span, reads only those samples from the file and ships them; lm_forward_spans
+ * turns a batch of such spans into the features lm_forward_resampled gives for the whole clips.
+ *
+ * lm_clip_span: the native-sample span [*first, *first + *count) that the features of a clip of `length` samples at
+ * orig_freq read when the plan runs at new_freq with target_len (orig == new: the pad / centre-crop span).  Every index
+ * the resampler's fmaf chain touches inside [0, length) counts, zero padding taps included, so the span covers
+ * non-finite samples exactly as the full clip would.  A clip of length 0 gives (0, 0).  Pure host arithmetic: no
+ * device, no CUDA call, safe in forked workers.  LM_ERR_INVALID_ARG for rates or target_len < 1, length < 0 or NULL
+ * outputs.
+ */
+int lm_clip_span(int32_t orig_freq, int32_t new_freq, int32_t target_len, int64_t length, int64_t* first,
+                 int64_t* count);
+
+/*
+ * lm_forward_resampled on clips of which only a span is stored: clip i has length[i] native samples, and samples
+ * [first[i], first[i] + stored[i]) sit at wave[offset[i] ...].  first (int64) / stored (int32) are [B] DEVICE arrays.
+ * When the stored span contains lm_clip_span's span, the output is bit-identical to lm_forward_resampled on the full
+ * clips.  A clip whose stored span does not contain it becomes a zero-length clip: nothing outside the stored span is
+ * ever read.  Argument checks and status codes are those of lm_forward_resampled, with first and stored checked
+ * for NULL with the other arrays.
+ */
+int lm_forward_spans(lm_plan* plan, const lm_resampler* const* resamplers, int32_t n_resamplers,
+                     const void* wave, int32_t pcm16, const int64_t* offset, const int64_t* first,
+                     const int32_t* stored, const int32_t* length, const int32_t* source, int32_t B,
+                     const lm_aug* aug, const float* noise, float* out_norm, int32_t normalize,
+                     void* cuda_stream);
+
+/*
  * T.AmplitudeToDB() as a stand-alone transform (R/src/data/preprocessing.py:46; torchaudio/functional/functional.py:390-391,
  * stype "power", top_db None): out = multiplier * log10(max(in, amin)) - db_offset, element-wise.  Device pointers, in == out
  * allowed.  Serves the `amplitude_to_db` attribute of the drop-in AudioPreprocessor.
