@@ -10,7 +10,6 @@ intended use on a B200 is the raw mode: workers (or the main process) hand back 
 from __future__ import annotations
 
 import random
-from functools import partial
 from pathlib import Path
 from typing import List, NamedTuple, Sequence, Tuple
 
@@ -18,7 +17,6 @@ import numpy as np
 import torch
 from torch.utils.data import Dataset
 
-from . import _lib
 from .plan import clip_span
 from .preprocessing import AudioPreprocessor
 from .wavio import read_wav_span, wav_info
@@ -92,103 +90,55 @@ class RawView(Dataset):
 
 class GpuCollate:
     """collate_fn for raw items: list of (waveform, sample_rate, label) -- or (waveform, label) for waveforms already
-    at the target rate -- -> (features [B,1,n_mels,frames] on the GPU, labels int64 on the GPU).  The whole batch is
-    ONE log-mel launch; recordings at other rates are resampled inside it (`lm_forward_resampled`).  A batch with more
-    than LM_MAX_RESAMPLERS distinct foreign rates is resampled item by item first (`lm_resample`), then packed.
+    at the target rate -- -> (features [B,1,n_mels,frames] on the GPU, labels int64 on the GPU).  The batch is packed
+    into one pinned buffer, uploaded with one copy and turned into features by ONE log-mel launch
+    (`AudioPreprocessor.preprocess_batch`); recordings at other rates are resampled inside it (`lm_forward_resampled`).
     It must run in the process that owns the CUDA context.  A DataLoader calls its collate_fn INSIDE the worker
     processes, so with `num_workers > 0` give the loader `raw_collate` (workers hand back plain lists) and wrap it in
     `GpuLoader(loader, GpuCollate(...))`, which collates in the training process; with `num_workers=0` it can be
     the collate_fn itself.
 
-    Items of `raw(spans=True)` (`SpanItem`s) carry only the native samples their features read: they are packed into
-    one pinned buffer (int16 when every item is, else fp32 with int16 as x / 32768), uploaded with one copy and turned
-    into features by `LogMelPlan.forward_spans` -- the same features as the whole recordings give.  A batch with more
-    than LM_MAX_RESAMPLERS foreign rates makes one launch per group of at most that many rates, each filling its own
-    rows of the output.  A span item that misses samples this preprocessor's features read (cut for another rate or
-    target length) raises ValueError."""
+    Items of `raw(spans=True)` (`SpanItem`s) carry only the native samples their features read.  They are packed the
+    same way (int16 when every item is, else fp32 with int16 as x / 32768) and turned into features by
+    `LogMelPlan.forward_spans` -- the same features as the whole recordings give.  A span item that misses samples this
+    preprocessor's features read (cut for another rate or target length) raises ValueError before CUDA is touched.
+
+    For either kind of item, a batch with more than LM_MAX_RESAMPLERS foreign rates makes one launch per group of at
+    most that many rates, each filling its own rows of the output."""
 
     def __init__(self, preprocessor: AudioPreprocessor, fast_augment: bool = False):
         self.preprocessor = preprocessor
         self.fast_augment = fast_augment
 
     def __call__(self, batch: Sequence[tuple]):
+        pre = self.preprocessor
         spans = [isinstance(item, SpanItem) for item in batch]
         if any(spans):
             if not all(spans):
                 raise ValueError("a batch mixes SpanItems with whole-recording items")
-            return self._collate_spans(batch)
-        pre = self.preprocessor
-        waves, rates, labels = [], [], []
-        for item in batch:
-            w, sr, y = item if len(item) == 3 else (item[0], pre.sample_rate, item[1])
-            waves.append(w)
-            rates.append(int(sr))
-            labels.append(int(y))
-        if len({r for r in rates if r != int(pre.sample_rate)}) > _lib.LM_MAX_RESAMPLERS:
-            waves = [pre.resample_to_target(w, sr) for w, sr in zip(waves, rates)]
-            rates = None
-        feats = pre.preprocess_batch(waves, fast_augment=self.fast_augment, sample_rates=rates)
+            rate = int(pre.sample_rate)
+            # An item cut for another rate or target length would come out of the kernel as a silent clip: refuse it
+            # here, before anything touches CUDA.
+            for it in batch:
+                c = int(it.samples.shape[0])
+                first, count = clip_span(int(it.rate), rate, pre.target_length, int(it.length))
+                if count and not (it.first <= first and first + count <= it.first + c):
+                    raise ValueError(f"span item [{it.first}, {it.first + c}) of a {it.length}-sample {it.rate} Hz "
+                                     f"recording misses samples [{first}, {first + count}) that {rate} Hz features of "
+                                     f"{pre.target_length} samples read")
+            feats = pre._features([it.samples for it in batch], [it.rate for it in batch],
+                                  first=[int(it.first) for it in batch], length=[int(it.length) for it in batch],
+                                  fast_augment=self.fast_augment)
+            labels = [int(it.label) for it in batch]
+        else:
+            waves, rates, labels = [], [], []
+            for item in batch:
+                w, sr, y = item if len(item) == 3 else (item[0], pre.sample_rate, item[1])
+                waves.append(w)
+                rates.append(int(sr))
+                labels.append(int(y))
+            feats = pre.preprocess_batch(waves, fast_augment=self.fast_augment, sample_rates=rates)
         return feats, torch.tensor(labels, dtype=torch.int64).to(feats.device, non_blocking=True)
-
-    def _collate_spans(self, items: Sequence[SpanItem]):
-        from .resample import get_resampler
-        pre = self.preprocessor
-        rate, B = int(pre.sample_rate), len(items)
-        counts = [int(it.samples.shape[0]) for it in items]
-        # An item cut for another rate or target length would come out of the kernel as a silent clip: refuse it here.
-        for it, c in zip(items, counts):
-            first, count = clip_span(int(it.rate), rate, pre.target_length, int(it.length))
-            if count and not (it.first <= first and first + count <= it.first + c):
-                raise ValueError(f"span item [{it.first}, {it.first + c}) of a {it.length}-sample {it.rate} Hz recording "
-                                 f"misses samples [{first}, {first + count}) that {rate} Hz features of "
-                                 f"{pre.target_length} samples read")
-        plan = pre.plan
-        dev = plan.device
-        offsets = np.concatenate([[0], np.cumsum(counts)[:-1]]).astype(np.int64)
-        n = int(sum(counts))
-        pcm16 = all(it.samples.dtype == np.int16 for it in items)
-        stage = pre._pinned_stage((n + 1) // 2 if pcm16 else n)
-        host = stage.view(torch.int16)[:n] if pcm16 else stage[:n]
-        for it, o, c in zip(items, offsets.tolist(), counts):
-            x = torch.from_numpy(it.samples)
-            if not pcm16 and x.dtype == torch.int16:
-                x = x.to(torch.float32) / 32768.0   # exact: what the kernel's int16 staging computes
-            host[o:o + c].copy_(x)
-        wave = torch.empty(max(n, 1), dtype=host.dtype, device=dev)
-        if n:
-            wave[:n].copy_(host, non_blocking=True)
-        pre._stage_release()
-        # one upload of [B] int64 offset, [B] int64 first, then [B] int32 stored and [B] int32 length (B int64 slots)
-        meta = np.zeros(3 * B, dtype=np.int64)
-        meta[:B], meta[B:2 * B] = offsets, [int(it.first) for it in items]
-        meta[2 * B:].view(np.int32)[:] = counts + [int(it.length) for it in items]
-        meta_d = torch.from_numpy(meta).to(dev, non_blocking=True)
-        i32 = meta_d[2 * B:].view(torch.int32)
-        offset, first, stored, length = meta_d[:B], meta_d[B:2 * B], i32[:B], i32[B:]
-        labels = torch.tensor([int(it.label) for it in items], dtype=torch.int64).to(dev, non_blocking=True)
-
-        aug, noise = pre._draw(B, self.fast_augment)
-        foreign = sorted({int(it.rate) for it in items if int(it.rate) != rate})
-        k = _lib.LM_MAX_RESAMPLERS
-        groups = [foreign[i:i + k] for i in range(0, len(foreign), k)] or [[]]
-        feats = None
-        for gi, g in enumerate(groups):
-            rows = [i for i, it in enumerate(items) if int(it.rate) in g or (gi == 0 and int(it.rate) == rate)]
-            source = torch.tensor([g.index(int(items[i].rate)) if int(items[i].rate) != rate else -1 for i in rows],
-                                  dtype=torch.int32)
-            resamplers = [get_resampler(r, rate, dev) for r in g]
-            if len(groups) == 1:
-                forward = partial(plan.forward_spans, wave, offset, first, stored, length, source=source,
-                                  resamplers=resamplers)
-                return pre._finish(plan, forward, aug, noise), labels
-            ix = torch.tensor(rows, dtype=torch.int64, device=dev)
-            forward = partial(plan.forward_spans, wave, offset[ix], first[ix], stored[ix], length[ix], source=source,
-                              resamplers=resamplers)
-            part = pre._finish(plan, forward, None if aug is None else aug[rows], None if noise is None else noise[rows])
-            if feats is None:
-                feats = torch.empty((B,) + tuple(part.shape[1:]), dtype=part.dtype, device=dev)
-            feats.index_copy_(0, ix, part)
-        return feats, labels
 
 
 def raw_collate(batch):

@@ -196,46 +196,17 @@ class LogMelPlan:
     def forward_resampled(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor, source: torch.Tensor,
                           resamplers: Sequence["Resampler"], aug: Optional[torch.Tensor] = None,
                           noise: Optional[torch.Tensor] = None, normalize: bool = True, out: Optional[torch.Tensor] = None,
-                          stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+                          stream: Optional[torch.cuda.Stream] = None, *, first: Optional[torch.Tensor] = None,
+                          stored: Optional[torch.Tensor] = None) -> torch.Tensor:
         """`forward` on clips at their own sample rates, resampled to the plan's rate inside the kernel: one launch for
         a batch that mixes rates.  `wave` is fp32 or int16 (x / 32768) packed samples; `offset` / `length` count
         samples at the clip's own rate; `source` int32 [B] (on the host or on the plan's device) holds each clip's
         index into `resamplers` (`Resampler(clip_rate, plan.sample_rate)`, at most LM_MAX_RESAMPLERS), or -1 for a clip
         already at the plan's rate.  Bit-identical to resampling each clip with its `Resampler`, packing the results
-        and calling `forward` (`forward_pcm16` for int16 clips with source -1)."""
-        B, (handles, n_rs), source, out = self._check_resampled_inputs(wave, offset, length, source, resamplers, aug, noise,
-                                                                      out)
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
-        _lib.check(self._lib.lm_forward_resampled(self._h, handles, n_rs, wave.data_ptr(),
-                                                  1 if wave.dtype == torch.int16 else 0, offset.data_ptr(), length.data_ptr(),
-                                                  source.data_ptr(), B, _ptr(aug), _ptr(noise), out.data_ptr(),
-                                                  1 if normalize else 0, C.c_void_p(s.cuda_stream)))
-        return out
-
-    def forward_spans(self, wave: torch.Tensor, offset: torch.Tensor, first: torch.Tensor, stored: torch.Tensor,
-                      length: torch.Tensor, source: torch.Tensor, resamplers: Sequence["Resampler"],
-                      aug: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None, normalize: bool = True,
-                      out: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
-        """`forward_resampled` on clips of which only a span of native samples is stored: clip i has `length[i]`
-        samples, of which [first[i], first[i] + stored[i]) sit at wave[offset[i] ...].  `first` int64 [B] and `stored`
-        int32 [B] live on the plan's device.  When every stored span contains `clip_span(clip rate, plan rate,
-        target_length, length[i])`, the output is bit-identical to `forward_resampled` on the whole clips; a clip whose
-        stored span misses a sample it needs comes out as a zero-length clip, and nothing outside the spans is read."""
-        B, (handles, n_rs), source, out = self._check_resampled_inputs(wave, offset, length, source, resamplers, aug, noise,
-                                                                      out)
-        for name, t, dt in (("first", first, torch.int64), ("stored", stored, torch.int32)):
-            if t.device != self.device or t.dtype != dt or not t.is_contiguous() or t.numel() != B:
-                raise ValueError(f"{name} must be a contiguous {dt} [B] tensor on {self.device}")
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
-        _lib.check(self._lib.lm_forward_spans(self._h, handles, n_rs, wave.data_ptr(),
-                                              1 if wave.dtype == torch.int16 else 0, offset.data_ptr(), first.data_ptr(),
-                                              stored.data_ptr(), length.data_ptr(), source.data_ptr(), B, _ptr(aug),
-                                              _ptr(noise), out.data_ptr(), 1 if normalize else 0, C.c_void_p(s.cuda_stream)))
-        return out
-
-    def _check_resampled_inputs(self, wave, offset, length, source, resamplers, aug, noise, out):
-        """The checks of `forward_resampled` / `forward_spans` (ValueError); returns B, (resampler handles, their number),
-        `source` on the device and the output tensor."""
+        and calling `forward` (`forward_pcm16` for int16 clips with source -1).
+        With `first` and `stored` (both or neither) only a span of each clip is stored: see `forward_spans`."""
+        if (first is None) != (stored is None):
+            raise ValueError("first and stored must be given together")
         if wave.dtype not in (torch.float32, torch.int16):
             raise ValueError("wave must be fp32 samples or int16 PCM")
         B = self._check_device_inputs(("wave", wave, wave.dtype), offset, length, aug, noise, (("out", out),))
@@ -252,13 +223,37 @@ class LogMelPlan:
             raise ValueError(f"source must be an int32 [B] tensor on the host or on {self.device}")
         if B and (int(source.min()) < -1 or int(source.max()) >= len(resamplers)):
             raise ValueError(f"source values must lie in [-1, {len(resamplers)})")
+        spans = ()
+        if first is not None:
+            for name, t, dt in (("first", first, torch.int64), ("stored", stored, torch.int32)):
+                if t.device != self.device or t.dtype != dt or not t.is_contiguous() or t.numel() != B:
+                    raise ValueError(f"{name} must be a contiguous {dt} [B] tensor on {self.device}")
+            spans = (first.data_ptr(), stored.data_ptr())
         if not source.is_cuda:
             source = source.contiguous().to(self.device, non_blocking=True)
         source = source.contiguous()
         if out is None:
             out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
         handles = (C.c_void_p * max(len(resamplers), 1))(*[r._h.value for r in resamplers])
-        return B, (handles, len(resamplers)), source, out
+        s = torch.cuda.current_stream(self.device) if stream is None else stream
+        # lm_forward_spans is lm_forward_resampled's argument list with first / stored after offset
+        fn = self._lib.lm_forward_spans if spans else self._lib.lm_forward_resampled
+        _lib.check(fn(self._h, handles, len(resamplers), wave.data_ptr(), 1 if wave.dtype == torch.int16 else 0,
+                      offset.data_ptr(), *spans, length.data_ptr(), source.data_ptr(), B, _ptr(aug), _ptr(noise),
+                      out.data_ptr(), 1 if normalize else 0, C.c_void_p(s.cuda_stream)))
+        return out
+
+    def forward_spans(self, wave: torch.Tensor, offset: torch.Tensor, first: torch.Tensor, stored: torch.Tensor,
+                      length: torch.Tensor, source: torch.Tensor, resamplers: Sequence["Resampler"],
+                      aug: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None, normalize: bool = True,
+                      out: Optional[torch.Tensor] = None, stream: Optional[torch.cuda.Stream] = None) -> torch.Tensor:
+        """`forward_resampled` on clips of which only a span of native samples is stored: clip i has `length[i]`
+        samples, of which [first[i], first[i] + stored[i]) sit at wave[offset[i] ...].  `first` int64 [B] and `stored`
+        int32 [B] live on the plan's device.  When every stored span contains `clip_span(clip rate, plan rate,
+        target_length, length[i])`, the output is bit-identical to `forward_resampled` on the whole clips; a clip whose
+        stored span misses a sample it needs comes out as a zero-length clip, and nothing outside the spans is read."""
+        return self.forward_resampled(wave, offset, length, source, resamplers, aug, noise, normalize, out, stream,
+                                      first=first, stored=stored)
 
     def forward_gather(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor, out_slice_ptr: int,
                        peer_slice_ptrs=(), mc_slice_ptr: int = 0, aug: Optional[torch.Tensor] = None,

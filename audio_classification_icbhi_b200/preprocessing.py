@@ -21,6 +21,7 @@ import torch
 from . import _lib
 from .augment import draw_fast_augmentation, draw_reference_augmentation
 from .plan import LogMelPlan
+from .resample import get_resampler
 from .wavio import read_wav
 
 __all__ = ["AudioPreprocessor"]
@@ -177,7 +178,6 @@ class AudioPreprocessor:
         device tensor when it resamples, the input unchanged when the rates agree."""
         if int(sr) == int(self.sample_rate):
             return waveform
-        from .resample import get_resampler
         return get_resampler(int(sr), int(self.sample_rate), self.plan.device)(waveform.float())
 
     def load_audio(self, audio_path):
@@ -234,18 +234,20 @@ class AudioPreprocessor:
                                            freq_mask_param=self.freq_mask_param,
                                            time_mask_param=self.time_mask_param)
 
-    def _pinned_stage(self, n: int) -> torch.Tensor:
-        """One of two grow-only pinned host buffers for packing a batch.  Each carries an event recorded after the copy
-        out of it (`_stage_release`); the buffer is reused only once that copy is done, so packing batch k+1 overlaps the
-        GPU work of batch k and never scribbles over a copy in flight."""
+    def _pinned_stage(self, n: int, dtype: torch.dtype) -> torch.Tensor:
+        """n elements of `dtype` in one of two grow-only pinned host buffers for packing a batch.  Each carries an event
+        recorded after the copy out of it (`_stage_release`); the buffer is reused only once that copy is done, so
+        packing batch k+1 overlaps the GPU work of batch k and never scribbles over a copy in flight."""
         slots = self.__dict__.setdefault("_stages", [None, None])
         self._stage_ix = 1 - getattr(self, "_stage_ix", 1)
         slot = slots[self._stage_ix]
         if slot is not None:
             slot[1].synchronize()
-        if slot is None or slot[0].numel() < n:
-            slot = slots[self._stage_ix] = [torch.empty(max(n, 1 << 16), dtype=torch.float32).pin_memory(), torch.cuda.Event()]
-        return slot[0]
+        nbytes = n * dtype.itemsize
+        if slot is None or slot[0].numel() < nbytes:
+            slot = slots[self._stage_ix] = [torch.empty(max(nbytes, 1 << 18), dtype=torch.uint8).pin_memory(),
+                                            torch.cuda.Event()]
+        return slot[0][:nbytes].view(dtype)
 
     def _stage_release(self) -> None:
         self._stages[self._stage_ix][1].record(torch.cuda.current_stream(self.plan.device))
@@ -282,68 +284,109 @@ class AudioPreprocessor:
         """Batched hot path.  `waveforms`: list of 1-D / [C, len] waveforms of any lengths (host
         or device), or a dense `[B, len]` tensor (optionally with per-row `lengths`).
         `sample_rates`: optional rate of each clip.  Clips at other rates than `sample_rate` are resampled inside the
-        log-mel kernel (`LogMelPlan.forward_resampled`, at most LM_MAX_RESAMPLERS distinct foreign rates per batch),
-        with the same result as `resample_to_target` on each of them first.
+        log-mel kernel (`LogMelPlan.forward_resampled`), with the same result as `resample_to_target` on each of them
+        first.  Any number of rates may be mixed: one launch serves up to 8 foreign rates, and a batch with more makes
+        one launch per group of 8, each filling its own rows of the output.
         Returns `[B, 1, n_mels, frames]` float32 on the GPU."""
-        plan = self.plan
         rate = int(self.sample_rate)
-        rates = [] if sample_rates is None else [int(r) for r in sample_rates]
-        foreign = sorted({r for r in rates if r != rate})
-        dense = isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2
-        if dense:
+        if isinstance(waveforms, torch.Tensor) and waveforms.dim() == 2:
             B, n = waveforms.shape
             lens = torch.full((B,), n, dtype=torch.int32) if lengths is None else torch.as_tensor(lengths, dtype=torch.int32)
             if int(lens.max()) > n:
                 raise ValueError("lengths exceed the row length")
-        if dense and not foreign:   # the rows are the packed clips: no copy
-            wave = waveforms.to(device=plan.device, dtype=torch.float32).contiguous().view(-1)
-            offset = torch.arange(B, device=plan.device, dtype=torch.int64) * n
-            length = lens.to(plan.device)
+            if sample_rates is None or all(int(r) == rate for r in sample_rates):   # the rows are the packed clips: no copy
+                plan = self.plan
+                wave = waveforms.to(device=plan.device, dtype=torch.float32).contiguous().view(-1)
+                offset = torch.arange(B, device=plan.device, dtype=torch.int64) * n
+                aug, noise = self._draw(B, fast_augment)
+                return self._finish(plan, partial(plan.forward, wave, offset, lens.to(plan.device)), aug, noise)
+            clips = [waveforms[i, :k].to(torch.float32) for i, k in enumerate(lens.tolist())]
         else:
-            keep = lens.tolist() if dense else None
-            clips = [waveforms[i, :keep[i]].to(torch.float32) for i in range(B)] if dense else [_as_mono_1d(w) for w in waveforms]
-            B = len(clips)
-            wave, offset, length = self._pack(clips)
-        forward = partial(plan.forward, wave, offset, length)
-        if foreign:
-            if len(rates) != B:
-                raise ValueError("sample_rates must give one rate per waveform")
-            if len(foreign) > _lib.LM_MAX_RESAMPLERS:
-                raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} sample rates other than {self.sample_rate} per batch")
-            from .resample import get_resampler
-            source = torch.tensor([foreign.index(r) if r != rate else -1 for r in rates], dtype=torch.int32)
-            forward = partial(plan.forward_resampled, wave, offset, length, source=source,
-                              resamplers=[get_resampler(r, rate, plan.device) for r in foreign])
-        aug, noise = self._draw(B, fast_augment)
-        return self._finish(plan, forward, aug, noise)
+            clips = [_as_mono_1d(w) for w in waveforms]
+        return self._features(clips, sample_rates, fast_augment=fast_augment)
 
-    def _pack(self, clips: List[torch.Tensor]):
-        """1-D fp32 clips (host or device) -> (packed device samples, offset int64, length int32) on the plan's device."""
+    def _features(self, clips: List[Wave], rates: Optional[Sequence[int]] = None, first: Optional[Sequence[int]] = None,
+                  length: Optional[Sequence[int]] = None, fast_augment: bool = False) -> torch.Tensor:
+        """1-D clips at their own rates (`rates`, default `sample_rate`) -> `[B, 1, n_mels, frames]` on the GPU.  With
+        `first` and `length`, clip i holds only the native samples [first[i], first[i] + len(clip i)) of a recording of
+        length[i] samples (span items, `LogMelPlan.forward_spans`).  The sorted foreign rates are cut into groups of at
+        most LM_MAX_RESAMPLERS, one kernel call per group; a clip's features do not depend on the rest of its batch."""
+        plan, rate, B = self.plan, int(self.sample_rate), len(clips)
+        rates = [rate] * B if rates is None else [int(r) for r in rates]
+        if len(rates) != B:
+            raise ValueError("sample_rates must give one rate per waveform")
+        wave, starts = self._pack(clips)
+        stored = [int(c.shape[0]) for c in clips]
+        spans = first is not None
+        # one upload of the per-clip metadata: int64 offset [and first], then int32 [stored and] length
+        k = 2 if spans else 1
+        meta = np.zeros(k * B + (k * B + 1) // 2, dtype=np.int64)
+        meta[:B] = starts
+        if spans:
+            meta[B:2 * B] = first
+        meta[k * B:].view(np.int32)[:k * B] = (stored if spans else []) + list(stored if length is None else length)
+        meta_d = torch.from_numpy(meta).to(plan.device, non_blocking=True)
+        i32 = meta_d[k * B:].view(torch.int32)
+        per_clip = dict(offset=meta_d[:B], length=i32[(k - 1) * B:k * B])
+        if spans:
+            per_clip.update(first=meta_d[B:2 * B], stored=i32[:B])
+
+        def kernel(group, rows, tensors):
+            """One kernel call on the clips `rows` (their per-clip tensors bound) for the foreign rates `group`."""
+            if not (spans or group):   # nothing to resample: the plain kernel, which stages aligned clips through TMA
+                return partial(plan.forward, wave, **tensors)
+            source = torch.tensor([group.index(rates[i]) if rates[i] != rate else -1 for i in rows], dtype=torch.int32)
+            return partial(plan.forward_resampled, wave, source=source,
+                           resamplers=[get_resampler(r, rate, plan.device) for r in group], **tensors)
+
+        aug, noise = self._draw(B, fast_augment)
+        foreign = sorted({r for r in rates if r != rate})
+        n = _lib.LM_MAX_RESAMPLERS
+        groups = [foreign[i:i + n] for i in range(0, len(foreign), n)] or [[]]
+        if len(groups) == 1:
+            return self._finish(plan, kernel(groups[0], range(B), per_clip), aug, noise)
+        feats = None
+        for gi, group in enumerate(groups):   # clips at the plan's rate ride with group 0
+            rows = [i for i, r in enumerate(rates) if r in group or (gi == 0 and r == rate)]
+            ix = torch.tensor(rows, dtype=torch.int64, device=plan.device)
+            part = self._finish(plan, kernel(group, rows, {name: t[ix] for name, t in per_clip.items()}),
+                                None if aug is None else aug[rows], None if noise is None else noise[rows])
+            if feats is None:
+                feats = torch.empty((B,) + tuple(part.shape[1:]), dtype=part.dtype, device=plan.device)
+            feats.index_copy_(0, ix, part)
+        return feats
+
+    def _pack(self, clips: List[Wave]):
+        """1-D clips (torch or numpy, host or device, fp32 or int16) -> (packed device samples, start of each clip).  The
+        samples are int16 when every clip is, else fp32 with int16 clips as x / 32768 (exact: what the kernel's int16
+        staging computes)."""
         dev = self.plan.device
+        clips = [torch.as_tensor(c) for c in clips]
+        dtype = torch.int16 if clips and all(c.dtype == torch.int16 for c in clips) else torch.float32
+        clips = [c.to(torch.float32) / 32768.0 if c.dtype == torch.int16 and dtype == torch.float32 else c for c in clips]
+        align = 16 // dtype.itemsize   # 16-byte aligned clip starts: interior tiles of `plan.forward` go through TMA
         lens = [int(c.numel()) for c in clips]
         starts, pos = [], 0
-        for n in lens:           # 16-byte aligned clip starts: interior tiles go through TMA
+        for n in lens:
             starts.append(pos)
-            pos += (n + 3) & ~3
-        packed = torch.empty(max(pos, 4), dtype=torch.float32, device=dev)   # alignment gaps are never read
+            pos += (n + align - 1) & ~(align - 1)
+        packed = torch.empty(max(pos, align), dtype=dtype, device=dev)   # alignment gaps are never read
         # host clips: packed into ONE pinned staging buffer (kept on the object, grow-only) and sent with ONE
-        # asynchronous copy; clips that already live on the device (e.g. resampled by GpuCollate) are copied in place
+        # asynchronous copy; clips that already live on the device are copied in place
         host_ix = [i for i, c in enumerate(clips) if not c.is_cuda]
         if host_ix:
             lo, hi = starts[host_ix[0]], starts[host_ix[-1]] + lens[host_ix[-1]]
-            stage = self._pinned_stage(hi - lo)
+            stage = self._pinned_stage(hi - lo, dtype)
             for i in host_ix:
                 if lens[i]:
                     stage[starts[i] - lo:starts[i] - lo + lens[i]].copy_(clips[i])
             if hi > lo:
-                packed[lo:hi].copy_(stage[:hi - lo], non_blocking=True)
+                packed[lo:hi].copy_(stage, non_blocking=True)
             self._stage_release()
         for i, c in enumerate(clips):        # after the block copy: it also covered their (stale) slots
             if c.is_cuda and lens[i]:
                 packed[starts[i]:starts[i] + lens[i]].copy_(c, non_blocking=True)
-        offset = torch.tensor(starts, dtype=torch.int64).to(dev, non_blocking=True)
-        length = torch.tensor(lens, dtype=torch.int32).to(dev, non_blocking=True)
-        return packed, offset, length
+        return packed, starts
 
     def preprocess_waveform(self, waveform: Wave) -> torch.Tensor:
         """One in-memory waveform -> `[1, n_mels, frames]` float32 CPU tensor (what `preprocess`

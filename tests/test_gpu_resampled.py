@@ -258,18 +258,31 @@ def test_gpu_collate_one_launch_per_batch_equals_per_item_path(tmp_path):
         assert_bytes_equal(feats, _old_collate(pre, batch))
 
 
-def test_gpu_collate_falls_back_beyond_max_resamplers():
+def test_gpu_collate_groups_beyond_max_resamplers(monkeypatch):
     pre = A.AudioPreprocessor()
     rs = np.random.RandomState(22)
     rates = [8000, 11025, 12000, 22050, 24000, 32000, 44100, 48000, 10000, 16000]
     assert len(set(rates) - {16000}) > _lib.LM_MAX_RESAMPLERS
     batch = [(torch.from_numpy((rs.standard_normal((1, int(r * 3.3))) * 0.1).astype(np.float32)), r, i % 4)
              for i, r in enumerate(rates)]
+    ref = _old_collate(pre, batch)
+
+    def no_per_item_resampling(*args):
+        raise AssertionError("resampled item by item")
+    monkeypatch.setattr(pre, "resample_to_target", no_per_item_resampling)
+    n0 = pre.plan.launches
     feats, _ = A.GpuCollate(pre)(batch)
-    assert_bytes_equal(feats, _old_collate(pre, batch))
+    assert pre.plan.launches == n0 + 2   # 9 foreign rates: two groups of at most 8, no lm_resample
+    assert_bytes_equal(feats, ref)
     # the same items split into batches of <= 8 foreign rates take the fused path, with the same features
     feats2 = torch.cat([A.GpuCollate(pre)(batch[:5])[0], A.GpuCollate(pre)(batch[5:])[0]])
     assert_bytes_equal(feats2, feats)
+    # preprocess_batch takes any number of rates, too
+    waves = [w for w, _, _ in batch]
+    assert_bytes_equal(pre.preprocess_batch(waves, sample_rates=rates), ref)
+    split = [pre.preprocess_batch(waves[:5], sample_rates=rates[:5]),
+             pre.preprocess_batch(waves[5:], sample_rates=rates[5:])]
+    assert_bytes_equal(torch.cat(split), ref)
 
 
 def test_flexible_8s_mixed_rates_equals_two_step():

@@ -287,3 +287,7 @@ def test_error_paths():
         plan.forward_spans(wave, off, first, stored, ln, src, [get_resampler(44100, 8000, DEV)])
     with pytest.raises(ValueError, match="at most 8"):
         plan.forward_spans(wave, off, first, stored, ln, src, [r] * 9)
+    with pytest.raises(ValueError, match="first and stored must be given together"):
+        plan.forward_resampled(wave, off, ln, src, [r], first=first)
+    with pytest.raises(ValueError, match="first and stored must be given together"):
+        plan.forward_resampled(wave, off, ln, src, [r], stored=stored)

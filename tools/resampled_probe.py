@@ -6,9 +6,9 @@ the same process, alternated, and their outputs are compared bit for bit.
   1. 4096 x 5 s clips resident in HBM at 44.1, 10 and 4 kHz, fp32 and int16, -> 16 kHz, n_fft 2048 / hop 512 / 128 mels.
      Two-step: one lm_resample_rows launch over the batch (all rows of one length) + one lm_forward.
   2. ICBHI-shaped: 20 s recordings at 44.1 kHz, 5 s centre crop.  The two-step path resamples whole recordings.
-  3. GpuCollate wall time for batches of 32 mixed-rate host items (ICBHI mix: 44.1 / 10 / 4 kHz, 20 s): the
-     per-item path (H2D + lm_resample per item, pack, lm_forward) against one lm_forward_resampled, with a
-     synchronise after each batch.
+  3. GpuCollate wall time for batches of 32 mixed-rate host items of 20 s: the per-item path (H2D + lm_resample per
+     item, pack, lm_forward) against GpuCollate, with a synchronise after each batch.  The ICBHI mix (44.1 / 10 / 4 kHz)
+     is one lm_forward_resampled; a mix of 10 foreign rates and 16 kHz is more than one launch takes.
 
 Every input set is larger than the 126 MB L2 (sizes printed).  Times: median of >= 20 launches per path.
     python tools/resampled_probe.py [--reps 21]
@@ -102,9 +102,8 @@ def resident(plan, sr, secs, B, pcm16, reps, name):
     return t_old, t_new, same
 
 
-def collate_wall(pre, reps):
+def collate_wall(pre, reps, rates, name):
     rs = np.random.RandomState(3)
-    rates = [44100] * 22 + [10000] * 5 + [4000] * 5   # ICBHI: most recordings at 44.1 kHz
     batches = []
     for k in range(4):
         items = []
@@ -133,7 +132,7 @@ def collate_wall(pre, reps):
         t_old.append((t1 - t0) * 1e3); t_new.append((t2 - t1) * 1e3)
         same &= torch.equal(fo.view(torch.int32), fn.view(torch.int32))
     a, b = float(np.median(t_old)), float(np.median(t_new))
-    print(f"{'GpuCollate, 32 x 20 s host items':34s} B={32:5d} in={mb:8.0f} MB  per-item {a:8.3f} ms/batch  "
+    print(f"{name:34s} B={len(rates):5d} in={mb:8.0f} MB  per-item {a:8.3f} ms/batch  "
           f"fused {b:8.3f} ms/batch  x{a / b:5.2f}  bit-identical={same}  (4 distinct batches, wall clock + sync)",
           flush=True)
 
@@ -155,7 +154,10 @@ def main():
     resident(plan, 44100, 20, args.batch // 2, False, args.reps, "44100 Hz fp32, 20 s")
     torch.cuda.empty_cache()
     print("3. GpuCollate")
-    collate_wall(A.AudioPreprocessor(), args.reps)
+    icbhi = [44100] * 22 + [10000] * 5 + [4000] * 5   # ICBHI: most recordings at 44.1 kHz
+    collate_wall(A.AudioPreprocessor(), args.reps, icbhi, "GpuCollate, 32 x 20 s host items")
+    many = ([44100, 48000, 32000, 24000, 22050, 12000, 11025, 10000, 8000, 4000, 16000] * 3)[:32]
+    collate_wall(A.AudioPreprocessor(), args.reps, many, "GpuCollate, 32 x 20 s at 11 rates")
 
 
 if __name__ == "__main__":
