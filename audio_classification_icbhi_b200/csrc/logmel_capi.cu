@@ -83,8 +83,6 @@ struct HostSlot {
     int cap_clips = 0;
 };
 
-// The logmel_kernel instantiations a plan may launch, by what the call needs.
-enum Variant { kPlain, kExtraOut, kPcm16, kDeviceNoise, kResampled, kVariants };
 using KernelFn = void (*)(lm::KParams);
 
 // What a plan of one n_fft and hop needs from the kernel's compile-time layout (lm::Geo, lm::Smem).
@@ -94,20 +92,20 @@ struct Geometry {
     int row_cap;   // a mel band of the last frame of a warp row (at (FPW - 1) * OFF) must end before this row offset
     int nc;        // points of one complex FFT: the twiddle between its two stages is W_nc^(k1 n2)
     size_t (*smem_total)(int ns, int n_dk);
-    KernelFn kernels[kVariants];
+    KernelFn kernels[lm::kVariants];   // by lm::Variant
 };
 
 template <int NFFT>
 Geometry geometry(int hop) {
     using G = lm::Geo<NFFT>;
-    // Philox noise drawn in the kernel has its own staging instantiation (FASTNOISE) at n_fft = 2048 only; the other
-    // sizes stage it in the plain kernel.
-    KernelFn device_noise = lm::logmel_kernel<NFFT, false>;
-    if constexpr (NFFT == 2048) device_noise = lm::logmel_kernel<NFFT, false, true>;
+    using V = lm::Variant;
+    // Philox noise drawn in the kernel has its own staging instantiation (DeviceNoise) at n_fft = 2048 only; the other
+    // sizes stage it in the Plain kernel.
+    constexpr V device_noise = NFFT == 2048 ? V::DeviceNoise : V::Plain;
     return {G::TILE_F, ((G::TILE_F - 1) * hop + NFFT + 3) & ~3, lm::kRowFloats - (G::FPW - 1) * G::OFF, 32 * G::R,
             &lm::Smem<NFFT>::total,
-            {lm::logmel_kernel<NFFT, false>, lm::logmel_kernel<NFFT, true>, lm::logmel_kernel<NFFT, false, false, true>,
-             device_noise, lm::logmel_kernel<NFFT, false, false, false, true>}};
+            {lm::logmel_kernel<NFFT, V::Plain>, lm::logmel_kernel<NFFT, V::ExtraOut>, lm::logmel_kernel<NFFT, V::Pcm16>,
+             lm::logmel_kernel<NFFT, device_noise>, lm::logmel_kernel<NFFT, V::Resampled>}};
 }
 
 // The one place where a run-time n_fft (validated by lm_plan_create) becomes a compile-time size.
@@ -142,7 +140,7 @@ struct lm_plan {
     int sm_count = 0, max_ctas = 0, use_tma = 1, stagger_ns = 0;
     int host_chunk_clips = 0;   // lm_forward_host chunk size; 0 = automatic
     size_t smem_bytes = 0;
-    KernelFn kernels[kVariants] = {};
+    KernelFn kernels[lm::kVariants] = {};
     float db_mult = 10.f, amin = 1e-10f, db_offset = 0.f, floor_db = -100.f, norm_eps = 1e-8f;
     // device constants
     float* d_window = nullptr;
@@ -194,7 +192,7 @@ lm::KParams make_params(const lm_plan* p) {
 std::mutex g_smem_mu;
 std::map<std::pair<const void*, int>, size_t> g_smem_limit;   // (kernel, device) -> limit set so far
 
-cudaError_t set_smem_limit(const KernelFn (&kernels)[kVariants], int device, size_t bytes) {
+cudaError_t set_smem_limit(const KernelFn (&kernels)[lm::kVariants], int device, size_t bytes) {
     std::lock_guard<std::mutex> lock(g_smem_mu);
     for (KernelFn f : kernels) {
         size_t& cur = g_smem_limit[std::make_pair(reinterpret_cast<const void*>(f), device)];
@@ -226,7 +224,7 @@ void choose_split(const lm_plan* p, int B, int groups, bool normalize, int* spli
 // resamplers[source[i]], or the plan's rate for -1.
 // lm_forward_spans adds the stored span of each clip: native samples [first[i], first[i] + stored[i]) from offset[i] on.
 struct Batch {
-    const void* samples; bool pcm16;
+    const void* samples; int32_t pcm16;   // 0 or 1; lm_forward_resampled / lm_forward_spans take it from the caller
     const int64_t* offset; const int32_t* length; int32_t B;
     const lm_aug* aug; const float* noise;
     const int32_t* source = nullptr; const lm_resampler* const* resamplers = nullptr; int n_resamplers = 0;
@@ -240,8 +238,20 @@ struct Outputs {
     float* const* peers = nullptr; int n_peers = 0; float* mc = nullptr;
 };
 
+// The kernel instantiation of a launch: resampled and 16-bit batches have no dB / mel power outputs.
+int pick_variant(const Batch& b, const Outputs& o, lm::Variant* v) {
+    using V = lm::Variant;
+    const bool extra = (o.db != nullptr) || (o.melpow != nullptr);
+    if ((b.source != nullptr || b.pcm16) && extra) return LM_ERR_UNSUPPORTED;
+    const bool device_noise = (b.aug != nullptr) && (b.noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
+    *v = b.source ? V::Resampled : b.pcm16 ? V::Pcm16 : extra ? V::ExtraOut : device_noise ? V::DeviceNoise : V::Plain;
+    return LM_OK;
+}
+
 int launch(lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, cudaStream_t stream) {
     if (b.B == 0) return LM_OK;
+    lm::Variant v;
+    if (const int rc = pick_variant(b, o, &v)) return rc;
     lm::KParams k = make_params(p);
     for (int r = 0; r < o.n_peers; ++r) k.peer[r] = o.peers[r];
     k.n_peer = o.n_peers; k.mc_out = o.mc;
@@ -249,8 +259,7 @@ int launch(lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, cuda
     k.aug = b.aug; k.noise = b.noise; k.out_norm = o.norm; k.out_db = o.db; k.out_melpow = o.melpow;
     k.B = b.B; k.normalize = normalize;
     // lm_forward_resampled: every clip through the resampling staging, the sample format a run-time flag
-    const bool resampled = b.source != nullptr;
-    k.source = b.source; k.pcm16 = b.pcm16 ? 1 : 0; k.n_rs = b.n_resamplers;
+    k.source = b.source; k.pcm16 = b.pcm16; k.n_rs = b.n_resamplers;
     for (int r = 0; r < b.n_resamplers; ++r) {
         const lm_resampler* rs = b.resamplers[r];
         k.rs_taps4[r] = rs->d_taps4; k.rs_k0[r] = rs->d_k0;
@@ -268,19 +277,38 @@ int launch(lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, cuda
         // zero at plan creation; the group that completes a clip resets its entries
     }
     const int grid = std::min<int>(b.B * k.split, cap);
-    const bool extra = (o.db != nullptr) || (o.melpow != nullptr);
-    const bool device_noise = (b.aug != nullptr) && (b.noise == nullptr);   // clips may ask for Philox noise drawn in the kernel
-    if (b.pcm16 && extra) return LM_ERR_UNSUPPORTED;
-    if (resampled && extra) return LM_ERR_UNSUPPORTED;
-    const Variant v = resampled ? kResampled : b.pcm16 ? kPcm16 : extra ? kExtraOut : device_noise ? kDeviceNoise : kPlain;
-    p->kernels[v]<<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
+    p->kernels[static_cast<int>(v)]<<<grid, lm::kThreads, p->smem_bytes, stream>>>(k);
     LM_CUDA(cudaGetLastError());
     return LM_OK;
 }
 
-// The common tail of the device-input entry points, after their argument checks: an NVTX range named after the entry
-// point, the plan's device made current, one launch.
-int forward_on_device(const char* name, lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, void* stream) {
+// What an entry point needs beyond plan, clips and `norm`: `source` (Resampled, Spans), `first` / `stored` (Spans),
+// 16-byte aligned outputs (Gather).
+enum class Call { Plain, Gather, Resampled, Spans };
+
+// Every device-input entry point: the argument check, in the order its statuses are returned (device-free up to the
+// first plan dereference), then an NVTX range named after the entry point, the plan's device made current, one launch.
+int forward_on_device(const char* name, Call call, lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize,
+                      void* stream) {
+    if (!p || b.B < 0 || b.n_resamplers < 0 || b.n_resamplers > LM_MAX_RESAMPLERS || (b.n_resamplers > 0 && !b.resamplers) ||
+        (b.pcm16 != 0 && b.pcm16 != 1) || o.n_peers < 0 || o.n_peers > lm::kMaxPeers)
+        return LM_ERR_INVALID_ARG;
+    for (int r = 0; r < b.n_resamplers; ++r)
+        if (!b.resamplers[r]) return LM_ERR_INVALID_ARG;
+    if (b.B == 0) return LM_OK;
+    const bool resampled = call == Call::Resampled || call == Call::Spans;
+    if (!b.samples || !b.offset || !b.length || !o.norm || (resampled && !b.source) ||
+        (call == Call::Spans && (!b.first || !b.stored)) || (o.n_peers > 0 && !o.peers))
+        return LM_ERR_INVALID_ARG;
+    if (call == Call::Gather) {
+        // the gather rides on the 16-byte stores of the normalisation pass
+        if ((static_cast<size_t>(p->n_mels) * p->frames) % 4 != 0) return LM_ERR_UNSUPPORTED;
+        if ((reinterpret_cast<uintptr_t>(o.norm) & 15u) || (reinterpret_cast<uintptr_t>(o.mc) & 15u)) return LM_ERR_INVALID_ARG;
+        for (int r = 0; r < o.n_peers; ++r)
+            if (!o.peers[r] || (reinterpret_cast<uintptr_t>(o.peers[r]) & 15u)) return LM_ERR_INVALID_ARG;
+    }
+    for (int r = 0; r < b.n_resamplers; ++r)
+        if (b.resamplers[r]->device != p->device) return LM_ERR_INVALID_ARG;
     NvtxRange nvtx(name);
     DeviceOf on(p->device);
     if (on.err) return cuda_fail(on.err, "cudaSetDevice");
@@ -694,51 +722,28 @@ int64_t lm_plan_launch_count(const lm_plan* plan) { return plan ? plan->launches
 int lm_forward(lm_plan* plan, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
                const lm_aug* aug, const float* noise, float* out_norm, float* out_db, float* out_melpow,
                int32_t normalize, void* cuda_stream) {
-    if (!plan || B < 0) return LM_ERR_INVALID_ARG;
-    if (B == 0) return LM_OK;
-    if (!wave || !offset || !length || !out_norm) return LM_ERR_INVALID_ARG;
-    return forward_on_device("lm_forward", plan, {wave, false, offset, length, B, aug, noise}, {out_norm, out_db, out_melpow},
-                             normalize, cuda_stream);
+    return forward_on_device("lm_forward", Call::Plain, plan, {wave, 0, offset, length, B, aug, noise},
+                             {out_norm, out_db, out_melpow}, normalize, cuda_stream);
 }
 
 int lm_forward_pcm16(lm_plan* plan, const int16_t* pcm, const int64_t* offset, const int32_t* length, int32_t B,
                      const lm_aug* aug, const float* noise, float* out_norm, int32_t normalize, void* cuda_stream) {
-    if (!plan || B < 0) return LM_ERR_INVALID_ARG;
-    if (B == 0) return LM_OK;
-    if (!pcm || !offset || !length || !out_norm) return LM_ERR_INVALID_ARG;
-    return forward_on_device("lm_forward_pcm16", plan, {pcm, true, offset, length, B, aug, noise}, {out_norm}, normalize, cuda_stream);
+    return forward_on_device("lm_forward_pcm16", Call::Plain, plan, {pcm, 1, offset, length, B, aug, noise}, {out_norm},
+                             normalize, cuda_stream);
 }
 
 int lm_forward_gather(lm_plan* plan, const float* wave, const int64_t* offset, const int32_t* length, int32_t B,
                       const lm_aug* aug, const float* noise, float* out_slice, float* const* peer_slices,
                       int32_t n_peers, float* mc_slice, void* cuda_stream) {
-    if (!plan || B < 0 || n_peers < 0 || n_peers > lm::kMaxPeers) return LM_ERR_INVALID_ARG;
-    if (B == 0) return LM_OK;
-    if (!wave || !offset || !length || !out_slice || (n_peers > 0 && !peer_slices)) return LM_ERR_INVALID_ARG;
-    // the gather rides on the 16-byte stores of the normalisation pass
-    if ((static_cast<size_t>(plan->n_mels) * plan->frames) % 4 != 0) return LM_ERR_UNSUPPORTED;
-    if ((reinterpret_cast<uintptr_t>(out_slice) & 15u) || (reinterpret_cast<uintptr_t>(mc_slice) & 15u)) return LM_ERR_INVALID_ARG;
-    for (int r = 0; r < n_peers; ++r)
-        if (!peer_slices[r] || (reinterpret_cast<uintptr_t>(peer_slices[r]) & 15u)) return LM_ERR_INVALID_ARG;
-    return forward_on_device("lm_forward_gather", plan, {wave, false, offset, length, B, aug, noise},
+    return forward_on_device("lm_forward_gather", Call::Gather, plan, {wave, 0, offset, length, B, aug, noise},
                              {out_slice, nullptr, nullptr, peer_slices, n_peers, mc_slice}, 1, cuda_stream);
 }
 
 int lm_forward_resampled(lm_plan* plan, const lm_resampler* const* resamplers, int32_t n_resamplers, const void* wave,
                          int32_t pcm16, const int64_t* offset, const int32_t* length, const int32_t* source, int32_t B,
                          const lm_aug* aug, const float* noise, float* out_norm, int32_t normalize, void* cuda_stream) {
-    // every check that needs no device comes before the plan is dereferenced
-    if (!plan || B < 0 || n_resamplers < 0 || n_resamplers > LM_MAX_RESAMPLERS || (n_resamplers > 0 && !resamplers) ||
-        (pcm16 != 0 && pcm16 != 1))
-        return LM_ERR_INVALID_ARG;
-    for (int r = 0; r < n_resamplers; ++r)
-        if (!resamplers[r]) return LM_ERR_INVALID_ARG;
-    if (B == 0) return LM_OK;
-    if (!wave || !offset || !length || !source || !out_norm) return LM_ERR_INVALID_ARG;
-    for (int r = 0; r < n_resamplers; ++r)
-        if (resamplers[r]->device != plan->device) return LM_ERR_INVALID_ARG;
-    return forward_on_device("lm_forward_resampled", plan,
-                             {wave, pcm16 != 0, offset, length, B, aug, noise, source, resamplers, n_resamplers}, {out_norm},
+    return forward_on_device("lm_forward_resampled", Call::Resampled, plan,
+                             {wave, pcm16, offset, length, B, aug, noise, source, resamplers, n_resamplers}, {out_norm},
                              normalize, cuda_stream);
 }
 
@@ -765,19 +770,9 @@ int lm_forward_spans(lm_plan* plan, const lm_resampler* const* resamplers, int32
                      int32_t pcm16, const int64_t* offset, const int64_t* first, const int32_t* stored,
                      const int32_t* length, const int32_t* source, int32_t B, const lm_aug* aug, const float* noise,
                      float* out_norm, int32_t normalize, void* cuda_stream) {
-    // the checks and their order are lm_forward_resampled's
-    if (!plan || B < 0 || n_resamplers < 0 || n_resamplers > LM_MAX_RESAMPLERS || (n_resamplers > 0 && !resamplers) ||
-        (pcm16 != 0 && pcm16 != 1))
-        return LM_ERR_INVALID_ARG;
-    for (int r = 0; r < n_resamplers; ++r)
-        if (!resamplers[r]) return LM_ERR_INVALID_ARG;
-    if (B == 0) return LM_OK;
-    if (!wave || !offset || !first || !stored || !length || !source || !out_norm) return LM_ERR_INVALID_ARG;
-    for (int r = 0; r < n_resamplers; ++r)
-        if (resamplers[r]->device != plan->device) return LM_ERR_INVALID_ARG;
-    Batch b{wave, pcm16 != 0, offset, length, B, aug, noise, source, resamplers, n_resamplers};
-    b.first = first; b.stored = stored;
-    return forward_on_device("lm_forward_spans", plan, b, {out_norm}, normalize, cuda_stream);
+    return forward_on_device("lm_forward_spans", Call::Spans, plan,
+                             {wave, pcm16, offset, length, B, aug, noise, source, resamplers, n_resamplers, first, stored},
+                             {out_norm}, normalize, cuda_stream);
 }
 
 int lm_resize_finish(const float* in, int32_t B, int32_t n_mels, int32_t frames_in, int32_t frames_out,

@@ -47,7 +47,7 @@
 //           the same pass also stores the result into the other ranks' gathered buffers (multimem.st
 //           through the NVSwitch, or plain stores to peer-mapped memory).
 //
-//   pcm16   (PCM16 instantiation, lm_forward_pcm16) the clips are 16-bit PCM, the sample format of the ICBHI wav
+//   pcm16   (Pcm16 instantiation, lm_forward_pcm16) the clips are 16-bit PCM, the sample format of the ICBHI wav
 //           files (R/src/data/preprocessing.py:55-68 decodes them with torchaudio.load): the bulk copy brings the
 //           tile's raw samples (2 bytes each) to the END of the staging buffer and the group expands them in place to
 //           fp32 (x / 32768, as lm_pcm16_decode) before the FFT reads them; the gather path converts sample by sample.
@@ -94,6 +94,11 @@ constexpr int kMaxMelTiles = 32;              // n_mels <= 256
 constexpr int kMaxPeers = 7;                  // other GPUs of one NVSwitch domain
 constexpr int kTileSlots = kMaxMelTiles / kGroupWarps;   // mel tiles per warp, at most
 constexpr int kMaxDk = 96;                    // 16-bin steps of banded filterbank kept on chip (1 KB each)
+
+// What one logmel_kernel instantiation is built for: fp32 clips (Plain), + dB and mel power outputs (ExtraOut), 16-bit
+// PCM clips (Pcm16), on-device Philox noise (DeviceNoise), resampling in the staging (Resampled).  One per launch.
+enum class Variant { Plain, ExtraOut, Pcm16, DeviceNoise, Resampled };
+constexpr int kVariants = static_cast<int>(Variant::Resampled) + 1;
 
 struct MelTable {                             // lives in global memory, copied to shared
     int kb[kMaxMelTiles];                     // first bin of the tile's band (multiple of 4)
@@ -147,7 +152,7 @@ struct KParams {
     const float2* __restrict__ utw;     // [512]    (cos, sin)(2 pi k / 2048)
     const float4* __restrict__ melw;    // [n_dk][2 k-steps][32 lanes]: mma A fragments (head, residual, head, residual)
     const MelTable* __restrict__ mel_table;
-    // lm_forward_resampled (RESAMPLE instantiation): clip i is at the rate of rate pair source[i] (-1: the plan's rate)
+    // lm_forward_resampled (Resampled instantiation): clip i is at the rate of rate pair source[i] (-1: the plan's rate)
     // and is resampled inside the staging; `wave` holds int16 samples when pcm16 is set.  Per rate pair the tables of
     // the tiled resampler (logmel_aux.cuh resample_tiled_kernel): nt4 float4 taps per phase, first tap k0 per phase.
     const int* __restrict__ source;
@@ -156,7 +161,7 @@ struct KParams {
     const float4* rs_taps4[LM_MAX_RESAMPLERS];
     const int* rs_k0[LM_MAX_RESAMPLERS];
     int rs_o[LM_MAX_RESAMPLERS], rs_q[LM_MAX_RESAMPLERS], rs_nt4[LM_MAX_RESAMPLERS], rs_width[LM_MAX_RESAMPLERS];
-    // lm_forward_spans (RESAMPLE instantiation): clip i stores only its native samples [first[i], first[i] + stored[i]),
+    // lm_forward_spans (Resampled instantiation): clip i stores only its native samples [first[i], first[i] + stored[i]),
     // starting at wave + offset[i]; length[i] is still the whole clip's.  Null for lm_forward_resampled.
     const long long* __restrict__ first;
     const int* __restrict__ stored;
@@ -496,7 +501,7 @@ __device__ __forceinline__ void stage_slots(const ClipCtx& c, float* __restrict_
 }
 
 // ---------------------------------------------------------------------------------------
-// Resampling inside the staging (RESAMPLE instantiation, lm_forward_resampled).  Clip i holds len native samples;
+// Resampling inside the staging (Resampled instantiation, lm_forward_resampled).  Clip i holds len native samples;
 // its resampled signal y has L' = ceil(q len / o) samples and is padded / centre-cropped like any clip, so staged
 // sample i (after reflect and roll, i < lc = min(L', T)) is y[crop + i], crop = (L' - T) / 2 when L' > T.  y[m q + ph]
 // is the tiled resampler's chain: acc = fmaf(taps4[ph][t], x[m o + k0[ph] - width + t], acc) for t < 4 nt4, x = 0
@@ -589,7 +594,7 @@ __host__ __device__ inline void rs_read_span(const int* k0, int o, int q, int wi
 
 // lm_forward_spans: whether the stored span [f, f + stored) holds every native sample the staging of a clip reads: the
 // resampler's read set (rs_read_span), or for a clip at the plan's rate (q == 0) its lc samples from the crop on.  Once
-// per clip, by one thread.  Inline: as an out-of-line call from load_clip it cost the RESAMPLE instantiations 32-56 bytes
+// per clip, by one thread.  Inline: as an out-of-line call from load_clip it cost the Resampled instantiations 32-56 bytes
 // of stack and spills across the call.
 __device__ __forceinline__ bool span_stored(const int* k0, int o, int q, int width, int nt4, long long len, long long crop,
                                          int lc, int T, long long f, int stored) {
@@ -615,11 +620,12 @@ __device__ __noinline__ void stage_resampled_tile(const ClipCtx& c, const RsClip
 
 // `nfft` is NFFT passed as a value: with the compile-time constant in the padded-signal bounds below, the compiler
 // reassociates them and the churn that follows through the whole kernel measured 0.1-0.2 % slower at n_fft = 512.
-// RESAMPLE: lc = min(L', T) and src is the clip's first native sample, or its first sample after the crop for a clip at
+// Resampled: lc = min(L', T) and src is the clip's first native sample, or its first sample after the crop for a clip at
 // the plan's rate (rs_clip); `plain` then only decides silent tiles, the staging never takes the bulk-copy path.  With
 // stored spans (lm_forward_spans) a clip whose span misses a sample the staging reads gets lc = 0: a zero-length clip.
-template <int NFFT, bool PCM16, bool RESAMPLE = false>
+template <int NFFT, Variant V>
 __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* __restrict__ c, int nfft) {
+    constexpr bool PCM16 = V == Variant::Pcm16, RESAMPLE = V == Variant::Resampled;
     const int clip = vclip / p.split, chunk = vclip - clip * p.split;
     c->t_begin = chunk * p.tiles_per_chunk;
     c->t_end = (c->t_begin + p.tiles_per_chunk < p.n_tiles) ? c->t_begin + p.tiles_per_chunk : p.n_tiles;
@@ -673,15 +679,15 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     c->silent_from = silent_from;
 }
 
-// FASTNOISE: tiles of clips with on-device Philox noise are staged four samples per thread (stage_noisy_tile).  The call
+// DeviceNoise: tiles of clips with on-device Philox noise are staged four samples per thread (stage_noisy_tile).  The call
 // costs the main loop ~3 % (registers live across it), so the host launches this instantiation only when the batch can
-// contain such clips (augmentation records given, no host-drawn noise tensor); the headline path keeps FASTNOISE = false.
-// RESAMPLE: lm_forward_resampled.  Every tile goes through stage_resampled_tile (no bulk copy; fp32 or 16-bit samples by
+// contain such clips (augmentation records given, no host-drawn noise tensor); the headline path launches Plain.
+// Resampled: lm_forward_resampled.  Every tile goes through stage_resampled_tile (no bulk copy; fp32 or 16-bit samples by
 // p.pcm16 at run time, Philox noise drawn per sample); silent tiles still apply to un-augmented clips.
-template <int NFFT, bool EXTRA_OUT, bool FASTNOISE = false, bool PCM16 = false, bool RESAMPLE = false>
+template <int NFFT, Variant V>
 __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
-    static_assert(!(PCM16 && (FASTNOISE || EXTRA_OUT)), "the 16-bit instantiation is the plain one");
-    static_assert(!(RESAMPLE && (PCM16 || FASTNOISE || EXTRA_OUT)), "the resampling instantiation is the plain one");
+    constexpr bool EXTRA_OUT = V == Variant::ExtraOut, FASTNOISE = V == Variant::DeviceNoise;
+    constexpr bool PCM16 = V == Variant::Pcm16, RESAMPLE = V == Variant::Resampled;
     using G = Geo<NFFT>;
     constexpr int TILE_F = G::TILE_F;
     constexpr int HALF = NFFT / 2;
@@ -838,7 +844,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
 
     // ---- prologue: item 0 is staged before the loop; item it+1 is staged during item it ----------------
     if (gtid == 0) {
-        load_clip<NFFT, PCM16, RESAMPLE>(p, clip0, &s_ctx[0], NFFT);
+        load_clip<NFFT, V>(p, clip0, &s_ctx[0], NFFT);
         stage_bulk(&s_ctx[0], s_ctx[0].t_begin);
     }
     group_bar(group);
@@ -880,7 +886,7 @@ __global__ void __launch_bounds__(kThreads, 1) logmel_kernel(const KParams p) {
                 if (wrap) {   // fetch the group's next (virtual) clip
                     const int nxt = nv + atomicAdd(p.work_counter, 1);
                     if (nxt < n_virtual) {
-                        load_clip<NFFT, PCM16, RESAMPLE>(p, nxt, cn, NFFT);
+                        load_clip<NFFT, V>(p, nxt, cn, NFFT);
                         stage_bulk(cn, cn->t_begin);
                     } else {
                         cn->clip = -1;

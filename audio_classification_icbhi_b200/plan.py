@@ -137,9 +137,11 @@ class LogMelPlan:
     # -- device path -----------------------------------------------------------------------
     def _check_device_inputs(self, samples: Tuple[str, torch.Tensor, torch.dtype], offset: torch.Tensor,
                              length: torch.Tensor, aug: Optional[torch.Tensor], noise: Optional[torch.Tensor],
-                             outs=()) -> int:
+                             outs=(), resamplers: Optional[list] = None, source: Optional[torch.Tensor] = None,
+                             first: Optional[torch.Tensor] = None, stored: Optional[torch.Tensor] = None) -> int:
         """Raises ValueError unless the tensors of one device call fit this plan; returns the batch size B.
-        `samples` is (name, tensor, dtype) of the packed clips, `outs` (name, tensor or None) of the outputs."""
+        `samples` is (name, tensor, dtype) of the packed clips, `outs` (name, tensor or None) of the outputs;
+        `forward_resampled` adds its resamplers, per-clip `source` indices and optional stored spans."""
         B = int(offset.numel())
         for name, t, dt in (samples, ("offset", offset, torch.int64), ("length", length, torch.int32)):
             if t.device != self.device or t.dtype != dt or not t.is_contiguous():
@@ -155,7 +157,36 @@ class LogMelPlan:
         if noise is not None and (noise.device != self.device or noise.dtype != torch.float32
                                   or noise.numel() != B * self.target_length or not noise.is_contiguous()):
             raise ValueError("noise must be contiguous fp32 [B, target_length] on the plan's device")
+        if resamplers is None:
+            return B
+        if len(resamplers) > _lib.LM_MAX_RESAMPLERS:
+            raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} resamplers per call")
+        for r in resamplers:
+            if r.new_freq != self.sample_rate:
+                raise ValueError(f"resampler {r.orig_freq} -> {r.new_freq} Hz does not produce the plan's {self.sample_rate} Hz")
+            if torch.device("cuda", r.device.index or 0) != self.device:
+                raise ValueError(f"resampler on {r.device}, plan on {self.device}")
+        if source.dtype != torch.int32 or source.numel() != B or source.dim() != 1 or source.device.type not in ("cpu", "cuda") \
+                or (source.is_cuda and source.device != self.device):
+            raise ValueError(f"source must be an int32 [B] tensor on the host or on {self.device}")
+        if B and (int(source.min()) < -1 or int(source.max()) >= len(resamplers)):
+            raise ValueError(f"source values must lie in [-1, {len(resamplers)})")
+        for name, t, dt in (("first", first, torch.int64), ("stored", stored, torch.int32)):
+            if t is not None and (t.device != self.device or t.dtype != dt or not t.is_contiguous() or t.numel() != B):
+                raise ValueError(f"{name} must be a contiguous {dt} [B] tensor on {self.device}")
         return B
+
+    def _launch(self, fn, B: int, args: tuple, out: Optional[torch.Tensor], tail: tuple,
+                stream: Optional[torch.cuda.Stream]) -> torch.Tensor:
+        """The checked call fn(plan, *args, out, *tail, stream) of one device entry point.  Tensors are passed as their
+        data pointers; `out` is allocated as [B, 1, n_mels, frames] when None, `stream` defaults to the current stream
+        of the plan's device.  Returns `out`."""
+        if out is None:
+            out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
+        s = torch.cuda.current_stream(self.device) if stream is None else stream
+        ptrs = [a.data_ptr() if isinstance(a, torch.Tensor) else a for a in (*args, out, *tail)]
+        _lib.check(fn(self._h, *ptrs, C.c_void_p(s.cuda_stream)))
+        return out
 
     def forward(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor,
                 aug: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None,
@@ -169,13 +200,8 @@ class LogMelPlan:
         noise: fp32 [B, target_length].  Returns ``out`` = [B, 1, n_mels, frames] fp32."""
         B = self._check_device_inputs(("wave", wave, torch.float32), offset, length, aug, noise,
                                       (("out", out), ("out_db", out_db), ("out_melpow", out_melpow)))
-        if out is None:
-            out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
-        _lib.check(self._lib.lm_forward(self._h, wave.data_ptr(), offset.data_ptr(), length.data_ptr(), B,
-                                        _ptr(aug), _ptr(noise), out.data_ptr(), _ptr(out_db), _ptr(out_melpow),
-                                        1 if normalize else 0, C.c_void_p(s.cuda_stream)))
-        return out
+        return self._launch(self._lib.lm_forward, B, (wave, offset, length, B, aug, noise), out,
+                            (out_db, out_melpow, 1 if normalize else 0), stream)
 
     def forward_pcm16(self, pcm: torch.Tensor, offset: torch.Tensor, length: torch.Tensor,
                       aug: Optional[torch.Tensor] = None, noise: Optional[torch.Tensor] = None,
@@ -185,13 +211,8 @@ class LogMelPlan:
         torchaudio.load, i.e. x / 32768): one kernel, 2 bytes per sample across HBM, bit-identical to decoding
         first.  Clip starts that are multiples of 8 samples take the bulk-copy staging path."""
         B = self._check_device_inputs(("pcm", pcm, torch.int16), offset, length, aug, noise, (("out", out),))
-        if out is None:
-            out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
-        _lib.check(self._lib.lm_forward_pcm16(self._h, pcm.data_ptr(), offset.data_ptr(), length.data_ptr(), B,
-                                              _ptr(aug), _ptr(noise), out.data_ptr(), 1 if normalize else 0,
-                                              C.c_void_p(s.cuda_stream)))
-        return out
+        return self._launch(self._lib.lm_forward_pcm16, B, (pcm, offset, length, B, aug, noise), out,
+                            (1 if normalize else 0,), stream)
 
     def forward_resampled(self, wave: torch.Tensor, offset: torch.Tensor, length: torch.Tensor, source: torch.Tensor,
                           resamplers: Sequence["Resampler"], aug: Optional[torch.Tensor] = None,
@@ -209,39 +230,18 @@ class LogMelPlan:
             raise ValueError("first and stored must be given together")
         if wave.dtype not in (torch.float32, torch.int16):
             raise ValueError("wave must be fp32 samples or int16 PCM")
-        B = self._check_device_inputs(("wave", wave, wave.dtype), offset, length, aug, noise, (("out", out),))
         resamplers = list(resamplers)
-        if len(resamplers) > _lib.LM_MAX_RESAMPLERS:
-            raise ValueError(f"at most {_lib.LM_MAX_RESAMPLERS} resamplers per call")
-        for r in resamplers:
-            if r.new_freq != self.sample_rate:
-                raise ValueError(f"resampler {r.orig_freq} -> {r.new_freq} Hz does not produce the plan's {self.sample_rate} Hz")
-            if torch.device("cuda", r.device.index or 0) != self.device:
-                raise ValueError(f"resampler on {r.device}, plan on {self.device}")
-        if source.dtype != torch.int32 or source.numel() != B or source.dim() != 1 or source.device.type not in ("cpu", "cuda") \
-                or (source.is_cuda and source.device != self.device):
-            raise ValueError(f"source must be an int32 [B] tensor on the host or on {self.device}")
-        if B and (int(source.min()) < -1 or int(source.max()) >= len(resamplers)):
-            raise ValueError(f"source values must lie in [-1, {len(resamplers)})")
-        spans = ()
-        if first is not None:
-            for name, t, dt in (("first", first, torch.int64), ("stored", stored, torch.int32)):
-                if t.device != self.device or t.dtype != dt or not t.is_contiguous() or t.numel() != B:
-                    raise ValueError(f"{name} must be a contiguous {dt} [B] tensor on {self.device}")
-            spans = (first.data_ptr(), stored.data_ptr())
+        B = self._check_device_inputs(("wave", wave, wave.dtype), offset, length, aug, noise, (("out", out),),
+                                      resamplers, source, first, stored)
         if not source.is_cuda:
             source = source.contiguous().to(self.device, non_blocking=True)
         source = source.contiguous()
-        if out is None:
-            out = torch.empty(self.out_shape(B), dtype=torch.float32, device=self.device)
         handles = (C.c_void_p * max(len(resamplers), 1))(*[r._h.value for r in resamplers])
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
         # lm_forward_spans is lm_forward_resampled's argument list with first / stored after offset
+        spans = () if first is None else (first, stored)
         fn = self._lib.lm_forward_spans if spans else self._lib.lm_forward_resampled
-        _lib.check(fn(self._h, handles, len(resamplers), wave.data_ptr(), 1 if wave.dtype == torch.int16 else 0,
-                      offset.data_ptr(), *spans, length.data_ptr(), source.data_ptr(), B, _ptr(aug), _ptr(noise),
-                      out.data_ptr(), 1 if normalize else 0, C.c_void_p(s.cuda_stream)))
-        return out
+        return self._launch(fn, B, (handles, len(resamplers), wave, 1 if wave.dtype == torch.int16 else 0, offset, *spans,
+                                    length, source, B, aug, noise), out, (1 if normalize else 0,), stream)
 
     def forward_spans(self, wave: torch.Tensor, offset: torch.Tensor, first: torch.Tensor, stored: torch.Tensor,
                       length: torch.Tensor, source: torch.Tensor, resamplers: Sequence["Resampler"],
@@ -265,11 +265,8 @@ class LogMelPlan:
         B = self._check_device_inputs(("wave", wave, torch.float32), offset, length, aug, noise)
         peers = [int(x) for x in peer_slice_ptrs]
         arr = (C.c_void_p * max(len(peers), 1))(*peers) if peers else None
-        s = torch.cuda.current_stream(self.device) if stream is None else stream
-        _lib.check(self._lib.lm_forward_gather(self._h, wave.data_ptr(), offset.data_ptr(), length.data_ptr(), B,
-                                               _ptr(aug), _ptr(noise), C.c_void_p(int(out_slice_ptr)), arr, len(peers),
-                                               C.c_void_p(int(mc_slice_ptr)) if mc_slice_ptr else None,
-                                               C.c_void_p(s.cuda_stream)))
+        self._launch(self._lib.lm_forward_gather, B, (wave, offset, length, B, aug, noise), C.c_void_p(int(out_slice_ptr)),
+                     (arr, len(peers), C.c_void_p(int(mc_slice_ptr)) if mc_slice_ptr else None), stream)
 
     @property
     def launches(self) -> int:
