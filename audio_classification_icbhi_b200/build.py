@@ -13,7 +13,7 @@ PKG_DIR = os.path.dirname(os.path.abspath(__file__))
 CSRC = os.path.join(PKG_DIR, "csrc")
 LIB_PATH = os.path.join(PKG_DIR, "liblogmel_b200.so")
 SOURCES = ["logmel_capi.cu"]
-DEPS = ["logmel_capi.cu", "logmel_kernel.cuh", "logmel_aux.cuh", "lm_f2.cuh", "fft_gen.cuh", os.path.join("..", "..", "include", "logmel_b200.h")]
+DEPS = ["logmel_capi.cu", "logmel_kernel.cuh", "logmel_aux.cuh", "resample.cuh", "lm_f2.cuh", "fft_gen.cuh", os.path.join("..", "..", "include", "logmel_b200.h")]
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a",

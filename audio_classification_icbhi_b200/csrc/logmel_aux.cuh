@@ -121,76 +121,4 @@ __global__ void pcm16_decode_kernel(const int16_t* __restrict__ in, float* __res
     for (long long i = (n8 << 3) + tid; i < n; i += stride) out[i] = static_cast<float>(in[i]) * k;
 }
 
-// Polyphase sinc resampler = torchaudio.transforms.Resample(orig, new) with its defaults, the resampler of
-// AudioPreprocessor.load_audio (R/src/data/preprocessing.py:63-65; TA/functional/functional.py
-// _get_sinc_resample_kernel / _apply_sinc_resample_kernel).  With o = orig/gcd, q = new/gcd and
-// xpad = pad(x, (width, width + o)):   y[m q + p] = sum_k kernel[p][k] xpad[m o + k],  k < 2 width + o.
-// torchaudio runs that as a dense conv1d; all but ~2 width + 1 taps of a phase are (numerically) zero, so
-// the host keeps, per phase, the window of `ntaps` taps around the phase's centre and the kernel walks only
-// those.  One output sample per thread; a block's outputs share their input span through L1.
-// grid.y = row (channel / clip): rows of equal length `n_in`, `in_stride` / `out_stride` floats apart
-__global__ void resample_kernel(const float* __restrict__ x_all, long long n_in, long long in_stride,
-                                float* __restrict__ y_all, long long n_out, long long out_stride,
-                                const float* __restrict__ taps, const int* __restrict__ k0, int o, int q, int ntaps,
-                                int width) {
-    const long long j = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
-    if (j >= n_out) return;
-    const float* __restrict__ x = x_all + static_cast<long long>(blockIdx.y) * in_stride;
-    float* __restrict__ y = y_all + static_cast<long long>(blockIdx.y) * out_stride;
-    const long long m = j / q;
-    const int p = static_cast<int>(j - m * q);
-    const float* __restrict__ w = taps + static_cast<size_t>(p) * ntaps;
-    const long long base = m * o + k0[p] - width;   // index into x of tap 0
-    float acc = 0.0f;
-    for (int i = 0; i < ntaps; ++i) {
-        const long long xi = base + i;
-        const float v = (xi >= 0 && xi < n_in) ? __ldg(x + xi) : 0.0f;
-        acc = fmaf(w[i], v, acc);
-    }
-    y[j] = acc;
-}
-
-
-// The same resampler, tiled: a block produces kRsChunk consecutive outputs of one row from ONE copy of their input
-// span in shared memory (loaded coalesced, zero outside the row: each input sample feeds ~ntaps * q / o outputs), taps
-// padded to a multiple of four per phase and fetched as 128-bit read-only loads.  The taps are walked in the same
-// order with the same fmaf chain as resample_kernel (the padding adds fmaf(0, x, acc) = acc), so the result is
-// bit-identical to it.
-constexpr int kRsChunk = 1024, kRsThreads = 256;
-__global__ void __launch_bounds__(kRsThreads) resample_tiled_kernel(const float* __restrict__ x_all, long long n_in, long long in_stride,
-                                                                     float* __restrict__ y_all, long long n_out, long long out_stride,
-                                                                     const float4* __restrict__ taps4, const int* __restrict__ k0, int o,
-                                                                     int q, int nt4, int width, int k0max) {
-    extern __shared__ float sx[];
-    const float* __restrict__ x = x_all + static_cast<long long>(blockIdx.y) * in_stride;
-    float* __restrict__ y = y_all + static_cast<long long>(blockIdx.y) * out_stride;
-    const long long j0 = static_cast<long long>(blockIdx.x) * kRsChunk;
-    const int n_here = static_cast<int>((n_out - j0 < kRsChunk) ? (n_out - j0) : kRsChunk);
-    const long long m0 = j0 / q;
-    const unsigned p0 = static_cast<unsigned>(j0 - m0 * q);
-    const long long x_lo = m0 * o - width;                                             // tap 0 of the first output at the earliest
-    const int m_span = static_cast<int>((p0 + static_cast<unsigned>(n_here) - 1u) / static_cast<unsigned>(q));
-    const int span = m_span * o + k0max + 4 * nt4;                                     // covers the last output's last (padded) tap
-    for (int i = threadIdx.x; i < span; i += kRsThreads) {
-        const long long xi = x_lo + i;
-        sx[i] = (xi >= 0 && xi < n_in) ? __ldg(x + xi) : 0.0f;
-    }
-    __syncthreads();
-    for (int d = threadIdx.x; d < n_here; d += kRsThreads) {
-        const unsigned t = p0 + static_cast<unsigned>(d);
-        const unsigned dm = t / static_cast<unsigned>(q), p = t - dm * static_cast<unsigned>(q);
-        const float4* __restrict__ w = taps4 + static_cast<size_t>(p) * nt4;
-        const float* __restrict__ xs = sx + dm * o + k0[p];
-        float acc = 0.0f;
-        for (int i = 0; i < nt4; ++i) {
-            const float4 wv = __ldg(w + i);
-            acc = fmaf(wv.x, xs[4 * i], acc);
-            acc = fmaf(wv.y, xs[4 * i + 1], acc);
-            acc = fmaf(wv.z, xs[4 * i + 2], acc);
-            acc = fmaf(wv.w, xs[4 * i + 3], acc);
-        }
-        y[j0 + d] = acc;
-    }
-}
-
 }  // namespace lm

@@ -122,15 +122,11 @@ Geometry geometry(int n_fft, int hop) {
 
 // ---- polyphase sinc resampler (torchaudio.transforms.Resample defaults) ---------------------------------------
 struct lm_resampler {
-    int device = 0, orig = 1, neu = 1;   // after division by the gcd
-    int width = 0, ntaps = 0;
-    float* d_taps = nullptr;
-    int* d_k0 = nullptr;
-    // tiled kernel: taps padded to nt4 float4 per phase; shared memory for the widest input span of a 1024-output chunk
-    // (lm_forward_resampled walks the same padded taps inside the log-mel staging)
-    float4* d_taps4 = nullptr;
-    int nt4 = 0, k0max = 0;
-    size_t tile_smem = 0;     // 0 = the span does not fit: the untiled kernel is used
+    int device = 0;
+    lm::RsTaps rs{};          // device tables (rs_design), read by both lm_resample kernels and lm_forward_resampled
+    int k0max = 0;
+    size_t tile_smem = 0;     // tiled kernel: shared memory for the widest input span of a 1024-output chunk; 0 = the
+                              // span does not fit: the untiled kernel is used
 };
 
 struct lm_plan {
@@ -260,11 +256,7 @@ int launch(lm_plan* p, const Batch& b, const Outputs& o, int32_t normalize, cuda
     k.B = b.B; k.normalize = normalize;
     // lm_forward_resampled: every clip through the resampling staging, the sample format a run-time flag
     k.source = b.source; k.pcm16 = b.pcm16; k.n_rs = b.n_resamplers;
-    for (int r = 0; r < b.n_resamplers; ++r) {
-        const lm_resampler* rs = b.resamplers[r];
-        k.rs_taps4[r] = rs->d_taps4; k.rs_k0[r] = rs->d_k0;
-        k.rs_o[r] = rs->orig; k.rs_q[r] = rs->neu; k.rs_nt4[r] = rs->nt4; k.rs_width[r] = rs->width;
-    }
+    for (int r = 0; r < b.n_resamplers; ++r) k.rs[r] = b.resamplers[r]->rs;
     k.first = reinterpret_cast<const long long*>(b.first); k.stored = b.stored;
     const long long seq = p->launches.fetch_add(1);
     k.work_counter = p->d_counters + 2 * (seq % kCounters);   // zero now, left at zero by the kernel (no memset per launch)
@@ -566,12 +558,13 @@ int forward_host_impl(lm_plan* plan, const void* wave, bool pcm16, int64_t total
 }
 
 // The polyphase taps of one rate pair and their geometry: rates divided by their gcd (o -> q), `width`, per phase the
-// first kept tap k0 and ntaps taps (nt4 float4 once padded).  Host arithmetic only: lm_resampler_create uploads the
-// tables, lm_clip_span derives the samples a clip's features read from the same k0 / width / nt4.
+// first kept tap k0 and 4 nt4 taps (the widest phase's ntaps, zero-padded to whole float4).  Host arithmetic only:
+// lm_resampler_create uploads the tables, lm_clip_span derives the samples a clip's features read from view().
 struct RsDesign {
-    int o = 1, q = 1, width = 0, ntaps = 1, nt4 = 1;
-    std::vector<float> taps;   // [q][ntaps]
-    std::vector<int> k0;       // [q]
+    int o = 1, q = 1, width = 0, nt4 = 1;
+    std::vector<float> taps4;   // [q][4 nt4]
+    std::vector<int> k0;        // [q]
+    lm::RsTaps view() const { return {nullptr, k0.data(), o, q, nt4, width}; }
 };
 
 RsDesign rs_design(int orig_freq, int new_freq) {
@@ -599,22 +592,23 @@ RsDesign rs_design(int orig_freq, int new_freq) {
         }
     // per phase keep the taps that are not negligible (|w| > 1e-12: the clamped tails are ~1e-33)
     int ntaps = 1;
-    std::vector<int> k0(q), k1(q);
+    std::vector<int> k0(q);
     for (int p = 0; p < q; ++p) {
         int lo = K, hi = -1;
         for (int k = 0; k < K; ++k)
             if (fabsf(dense[static_cast<size_t>(p) * K + k]) > 1e-12f) { lo = std::min(lo, k); hi = k; }
         if (hi < 0) { lo = 0; hi = 0; }
-        k0[p] = lo; k1[p] = hi;
+        k0[p] = lo;
         ntaps = std::max(ntaps, hi - lo + 1);
     }
-    std::vector<float> taps(static_cast<size_t>(q) * ntaps, 0.0f);
+    const int row = 4 * ((ntaps + 3) / 4);
+    std::vector<float> taps4(static_cast<size_t>(q) * row, 0.0f);
     for (int p = 0; p < q; ++p) {
         if (k0[p] + ntaps > K) k0[p] = std::max(0, K - ntaps);
-        for (int i = 0; i < ntaps && k0[p] + i < K; ++i) taps[static_cast<size_t>(p) * ntaps + i] = dense[static_cast<size_t>(p) * K + k0[p] + i];
+        for (int i = 0; i < ntaps && k0[p] + i < K; ++i) taps4[static_cast<size_t>(p) * row + i] = dense[static_cast<size_t>(p) * K + k0[p] + i];
     }
-    d.o = o; d.q = q; d.width = width; d.ntaps = ntaps; d.nt4 = (ntaps + 3) / 4;
-    d.taps = std::move(taps); d.k0 = std::move(k0);
+    d.o = o; d.q = q; d.width = width; d.nt4 = row / 4;
+    d.taps4 = std::move(taps4); d.k0 = std::move(k0);
     return d;
 }
 
@@ -758,8 +752,7 @@ int lm_clip_span(int32_t orig_freq, int32_t new_freq, int32_t target_len, int64_
         thread_local std::map<std::pair<int, int>, RsDesign> designs;
         auto it = designs.find(std::make_pair(orig_freq, new_freq));
         if (it == designs.end()) it = designs.emplace(std::make_pair(orig_freq, new_freq), rs_design(orig_freq, new_freq)).first;
-        const RsDesign& d = it->second;
-        lm::rs_read_span(d.k0.data(), d.o, d.q, d.width, d.nt4, length, target_len, &lo, &hi);
+        lm::rs_read_span(it->second.view(), length, target_len, &lo, &hi);
     }
     *first = lo;
     *count = hi - lo;
@@ -809,19 +802,12 @@ int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resa
     DeviceOf on(device);
     if (on.err) return cuda_fail(on.err, "cudaSetDevice");
     const RsDesign d = rs_design(orig_freq, new_freq);
-    const int o = d.o, q = d.q, ntaps = d.ntaps;
-    const std::vector<float>& taps = d.taps;
-    const std::vector<int>& k0 = d.k0;
     lm_resampler* r = new (std::nothrow) lm_resampler();
     if (!r) return LM_ERR_INVALID_ARG;
-    r->device = device; r->orig = o; r->neu = q; r->width = d.width; r->ntaps = ntaps;
-    r->nt4 = d.nt4;
-    r->k0max = *std::max_element(k0.begin(), k0.end());
-    std::vector<float> taps4(static_cast<size_t>(q) * r->nt4 * 4, 0.0f);
-    for (int p = 0; p < q; ++p)
-        for (int i = 0; i < ntaps; ++i) taps4[(static_cast<size_t>(p) * r->nt4) * 4 + i] = taps[static_cast<size_t>(p) * ntaps + i];
+    r->device = device;
+    r->k0max = *std::max_element(d.k0.begin(), d.k0.end());
     {
-        const size_t span = static_cast<size_t>((lm::kRsChunk + q - 1) / q + 1) * o + r->k0max + 4 * r->nt4 + 8;
+        const size_t span = static_cast<size_t>((lm::kRsChunk + d.q - 1) / d.q + 1) * d.o + r->k0max + 4 * d.nt4 + 8;
         r->tile_smem = span * sizeof(float) <= 96 * 1024 ? span * sizeof(float) : 0;
         if (const char* e = getenv("LM_RESAMPLE_UNTILED")) { if (e[0] == '1') r->tile_smem = 0; }   // tests compare the two kernels
         if (r->tile_smem > 48 * 1024 &&
@@ -830,17 +816,18 @@ int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resa
             r->tile_smem = 0;
         }
     }
-    if (cudaMalloc(&r->d_taps4, sizeof(float) * taps4.size()) != cudaSuccess ||
-        cudaMemcpy(r->d_taps4, taps4.data(), sizeof(float) * taps4.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMalloc(&r->d_taps, sizeof(float) * taps.size()) != cudaSuccess ||
-        cudaMalloc(&r->d_k0, sizeof(int) * q) != cudaSuccess ||
-        cudaMemcpy(r->d_taps, taps.data(), sizeof(float) * taps.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
-        cudaMemcpy(r->d_k0, k0.data(), sizeof(int) * q, cudaMemcpyHostToDevice) != cudaSuccess) {
+    float4* taps4 = nullptr;
+    int* k0 = nullptr;
+    if (cudaMalloc(&taps4, sizeof(float) * d.taps4.size()) != cudaSuccess ||
+        cudaMalloc(&k0, sizeof(int) * d.q) != cudaSuccess ||
+        cudaMemcpy(taps4, d.taps4.data(), sizeof(float) * d.taps4.size(), cudaMemcpyHostToDevice) != cudaSuccess ||
+        cudaMemcpy(k0, d.k0.data(), sizeof(int) * d.q, cudaMemcpyHostToDevice) != cudaSuccess) {
         const int rc = cuda_fail(cudaGetLastError(), "resampler tables");
-        cudaFree(r->d_taps); cudaFree(r->d_k0); cudaFree(r->d_taps4);
+        cudaFree(taps4); cudaFree(k0);
         delete r;
         return rc;
     }
+    r->rs = {taps4, k0, d.o, d.q, d.nt4, d.width};
     *out = r;
     return LM_OK;
 }
@@ -848,14 +835,14 @@ int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resa
 int lm_resampler_destroy(lm_resampler* r) {
     if (!r) return LM_OK;
     DeviceOf on(r->device);
-    cudaFree(r->d_taps); cudaFree(r->d_k0); cudaFree(r->d_taps4);
+    cudaFree(const_cast<float4*>(r->rs.taps4)); cudaFree(const_cast<int*>(r->rs.k0));
     delete r;
     return LM_OK;
 }
 
 int64_t lm_resampler_out_len(const lm_resampler* r, int64_t in_len) {
     if (!r || in_len < 0) return LM_ERR_INVALID_ARG;
-    return (static_cast<int64_t>(r->neu) * in_len + r->orig - 1) / r->orig;   // ceil(new * len / orig)
+    return (static_cast<int64_t>(r->rs.q) * in_len + r->rs.o - 1) / r->rs.o;   // ceil(new * len / orig)
 }
 
 int lm_resample_rows(const lm_resampler* r, const float* in, int64_t in_len, int64_t in_stride, int32_t n_rows,
@@ -874,14 +861,14 @@ int lm_resample_rows(const lm_resampler* r, const float* in, int64_t in_len, int
         lm::resample_tiled_kernel<<<dim3(static_cast<unsigned>(tblocks), static_cast<unsigned>(nr)), lm::kRsThreads, r->tile_smem,
                                     static_cast<cudaStream_t>(cuda_stream)>>>(
             in + static_cast<int64_t>(r0) * in_stride, in_len, in_stride, out + static_cast<int64_t>(r0) * out_stride, n_out,
-            out_stride, r->d_taps4, r->d_k0, r->orig, r->neu, r->nt4, r->width, r->k0max);
+            out_stride, r->rs, r->k0max);
     }
     for (int32_t r0 = 0; r0 < n_rows && !r->tile_smem; r0 += 65535) {   // grid.y limit
         const int32_t nr = std::min<int32_t>(65535, n_rows - r0);
         lm::resample_kernel<<<dim3(static_cast<unsigned>(blocks), static_cast<unsigned>(nr)), threads, 0,
                               static_cast<cudaStream_t>(cuda_stream)>>>(
             in + static_cast<int64_t>(r0) * in_stride, in_len, in_stride, out + static_cast<int64_t>(r0) * out_stride, n_out,
-            out_stride, r->d_taps, r->d_k0, r->orig, r->neu, r->ntaps, r->width);
+            out_stride, r->rs);
     }
     LM_CUDA(cudaGetLastError());
     return LM_OK;

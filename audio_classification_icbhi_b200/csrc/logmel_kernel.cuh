@@ -60,6 +60,7 @@
 
 #include "../../include/logmel_b200.h"
 #include "fft_gen.cuh"
+#include "resample.cuh"
 
 // Build-time experiment switches (tools/build_variants.py); the shipped kernel is LM_EXP=0, LM_TIMING=0.
 //   LM_EXP     1: no mel phase (FFT only)   2: no FFT (mel phase on stale rows)   3: no FFT part 2
@@ -153,14 +154,12 @@ struct KParams {
     const float4* __restrict__ melw;    // [n_dk][2 k-steps][32 lanes]: mma A fragments (head, residual, head, residual)
     const MelTable* __restrict__ mel_table;
     // lm_forward_resampled (Resampled instantiation): clip i is at the rate of rate pair source[i] (-1: the plan's rate)
-    // and is resampled inside the staging; `wave` holds int16 samples when pcm16 is set.  Per rate pair the tables of
-    // the tiled resampler (logmel_aux.cuh resample_tiled_kernel): nt4 float4 taps per phase, first tap k0 per phase.
+    // and is resampled inside the staging; `wave` holds int16 samples when pcm16 is set.  rs[s]: rate pair s, the
+    // tables lm_resample reads (resample.cuh).
     const int* __restrict__ source;
     int pcm16;
     int n_rs;
-    const float4* rs_taps4[LM_MAX_RESAMPLERS];
-    const int* rs_k0[LM_MAX_RESAMPLERS];
-    int rs_o[LM_MAX_RESAMPLERS], rs_q[LM_MAX_RESAMPLERS], rs_nt4[LM_MAX_RESAMPLERS], rs_width[LM_MAX_RESAMPLERS];
+    RsTaps rs[LM_MAX_RESAMPLERS];
     // lm_forward_spans (Resampled instantiation): clip i stores only its native samples [first[i], first[i] + stored[i]),
     // starting at wave + offset[i]; length[i] is still the whole clip's.  Null for lm_forward_resampled.
     const long long* __restrict__ first;
@@ -462,15 +461,10 @@ __device__ __noinline__ void stage_noisy_tile(const ClipCtx& c, float* __restric
 constexpr int kCtxSlot = 80;
 static_assert(sizeof(ClipCtx) <= kCtxSlot && kCtxSlot % 16 == 0, "ClipCtx slot size");
 
-// Sample k of clip samples x (fp32, or 16-bit PCM when PCM): its address, and its value as fp32 (x / 32768 for 16-bit
-// PCM, as lm_pcm16_decode).
+// The address of sample k of clip samples x (fp32, or 16-bit PCM when PCM); its value as fp32 is clip_sample (resample.cuh).
 template <bool PCM>
 __device__ __forceinline__ const void* sample_addr(const void* x, long long k) {
     return PCM ? static_cast<const void*>(static_cast<const short*>(x) + k) : static_cast<const float*>(x) + k;
-}
-template <bool PCM>
-__device__ __forceinline__ float clip_sample(const void* x, long long k) {
-    return PCM ? static_cast<float>(__ldg(static_cast<const short*>(x) + k)) * (1.0f / 32768.0f) : __ldg(static_cast<const float*>(x) + k);
 }
 
 // The staging of a tile, slot by slot, for the slots [0, e_lo) and [e_lo + cnt, ns) that the bulk copy does not cover
@@ -504,102 +498,41 @@ __device__ __forceinline__ void stage_slots(const ClipCtx& c, float* __restrict_
 // Resampling inside the staging (Resampled instantiation, lm_forward_resampled).  Clip i holds len native samples;
 // its resampled signal y has L' = ceil(q len / o) samples and is padded / centre-cropped like any clip, so staged
 // sample i (after reflect and roll, i < lc = min(L', T)) is y[crop + i], crop = (L' - T) / 2 when L' > T.  y[m q + ph]
-// is the tiled resampler's chain: acc = fmaf(taps4[ph][t], x[m o + k0[ph] - width + t], acc) for t < 4 nt4, x = 0
-// outside [0, len) -- the same taps, the same order and the same zero-padded tail, hence bit-identical to lm_resample.
+// is rs_sample (resample.cuh): the chain of lm_resample's kernels over the same padded tap row and the same x values (0
+// outside [0, len)), hence bit-identical to lm_resample.
 // ClipCtx has no room for the rate pair: the staging reads source / length / offset of the clip again per tile.
 // lm_forward_spans stores only native samples [first, first + stored) of a clip: ClipCtx::src is then wave + offset - first
 // (+ crop for a clip at the plan's rate), so x[k] is read where it is stored; lc, the crop, L' and the silent tiles still
 // come from the whole clip's length.
 // ---------------------------------------------------------------------------------------
 struct RsClip {
-    const float4* taps4;
-    const int* k0;
+    RsTaps g;         // g.q == 0: the clip is at the plan's rate (src already points past its crop)
     long long len;    // native samples (0 for a source index outside [-1, n_rs))
     long long lp;     // L': samples of y (len when the clip is at the plan's rate)
     long long crop;   // first sample of y kept by the centre crop
-    int o, q, nt4, width;   // q == 0: the clip is at the plan's rate (src already points past its crop)
 };
 __device__ __forceinline__ RsClip rs_clip(const KParams& p, int clip) {
-    RsClip r{nullptr, nullptr, p.length[clip], 0, 0, 1, 0, 0, 0};
+    RsClip r{{nullptr, nullptr, 1, 0, 0, 0}, p.length[clip], 0, 0};
     const int s = p.source[clip];
     r.lp = r.len;
     if (s < -1 || s >= p.n_rs) {   // device data: an invalid index makes an empty clip, nothing is read
         r.len = 0; r.lp = 0;
     } else if (s >= 0) {
-        r.taps4 = p.rs_taps4[s]; r.k0 = p.rs_k0[s];
-        r.o = p.rs_o[s]; r.q = p.rs_q[s]; r.nt4 = p.rs_nt4[s]; r.width = p.rs_width[s];
-        r.lp = (static_cast<long long>(r.q) * r.len + r.o - 1) / r.o;   // 64-bit: q len overflows int for long recordings
+        r.g = p.rs[s];
+        r.lp = (static_cast<long long>(r.g.q) * r.len + r.g.o - 1) / r.g.o;   // 64-bit: q len overflows int for long recordings
     }
     r.crop = r.lp > p.T ? (r.lp - p.T) / 2 : 0;
     return r;
 }
-template <bool PCM>
-__device__ __forceinline__ float rs_sample(const RsClip& r, const void* x, long long mp) {
-    const long long m = mp / r.q;
-    const int ph = static_cast<int>(mp - m * r.q);
-    const long long base = m * r.o + __ldg(r.k0 + ph) - r.width;   // native index of tap 0
-    const float4* __restrict__ w = r.taps4 + static_cast<size_t>(ph) * r.nt4;
-    float acc = 0.0f;
-    if (base >= 0 && base + 4 * r.nt4 <= r.len) {   // the whole (padded) span inside the clip: no bounds checks
-        for (int t = 0; t < r.nt4; ++t) {
-            const float4 wv = __ldg(w + t);
-            const long long k = base + 4 * t;
-            acc = fmaf(wv.x, clip_sample<PCM>(x, k), acc);
-            acc = fmaf(wv.y, clip_sample<PCM>(x, k + 1), acc);
-            acc = fmaf(wv.z, clip_sample<PCM>(x, k + 2), acc);
-            acc = fmaf(wv.w, clip_sample<PCM>(x, k + 3), acc);
-        }
-    } else {
-        auto at = [&](long long k) { return (k >= 0 && k < r.len) ? clip_sample<PCM>(x, k) : 0.0f; };
-        for (int t = 0; t < r.nt4; ++t) {
-            const float4 wv = __ldg(w + t);
-            const long long k = base + 4 * t;
-            acc = fmaf(wv.x, at(k), acc);
-            acc = fmaf(wv.y, at(k + 1), acc);
-            acc = fmaf(wv.z, at(k + 2), acc);
-            acc = fmaf(wv.w, at(k + 3), acc);
-        }
-    }
-    return acc;
-}
-// The native samples [*lo, *hi) that the staging of a resampled clip of len samples reads (lm_clip_span): every x[k],
-// 0 <= k < len, that the chain of an output y[crop + i], i < lc, touches, zero padding taps included (a non-finite sample
-// under a zero tap still poisons the sum).  Empty: *lo == *hi == 0.  For one phase the tap window moves right with m, so
-// the lowest index comes from the first q outputs of the crop and the highest from the last q; the windows of
-// neighbouring outputs overlap, so the indices in between are all read.  Host (lm_clip_span) and device (the
-// lm_forward_spans check) run this same code on the same k0 table.
-__host__ __device__ inline void rs_read_span(const int* k0, int o, int q, int width, int nt4, long long len, int T,
-                                             long long* lo, long long* hi) {
-    const long long lp = (static_cast<long long>(q) * len + o - 1) / o;
-    const long long lc = lp < T ? lp : T, crop = lp > T ? (lp - T) / 2 : 0;
-    *lo = 0; *hi = 0;
-    if (lc <= 0) return;
-    const int n = lc < q ? static_cast<int>(lc) : q;
-    long long a = 0, b = 0;
-    for (int side = 0; side < 2; ++side) {
-        const long long mp0 = side ? crop + lc - n : crop;
-        long long m = mp0 / q;
-        int ph = static_cast<int>(mp0 - m * q);
-        for (int j = 0; j < n; ++j) {
-            const long long base = m * o + k0[ph] - width;
-            if (side == 0 && (j == 0 || base < a)) a = base;
-            if (side == 1 && (j == 0 || base + 4 * nt4 > b)) b = base + 4 * nt4;
-            if (++ph == q) { ph = 0; ++m; }
-        }
-    }
-    if (a < 0) a = 0;
-    if (b > len) b = len;
-    if (b > a) { *lo = a; *hi = b; }
-}
 
 // lm_forward_spans: whether the stored span [f, f + stored) holds every native sample the staging of a clip reads: the
-// resampler's read set (rs_read_span), or for a clip at the plan's rate (q == 0) its lc samples from the crop on.  Once
+// resampler's read set (rs_read_span), or for a clip at the plan's rate (g.q == 0) its lc samples from the crop on.  Once
 // per clip, by one thread.  Inline: as an out-of-line call from load_clip it cost the Resampled instantiations 32-56 bytes
 // of stack and spills across the call.
-__device__ __forceinline__ bool span_stored(const int* k0, int o, int q, int width, int nt4, long long len, long long crop,
-                                         int lc, int T, long long f, int stored) {
+__device__ __forceinline__ bool span_stored(const RsTaps& g, long long len, long long crop, int lc, int T, long long f,
+                                            int stored) {
     long long lo = crop, hi = crop + lc;
-    if (q) rs_read_span(k0, o, q, width, nt4, len, T, &lo, &hi);
+    if (g.q) rs_read_span(g, len, T, &lo, &hi);
     return hi <= lo || (f <= lo && hi <= f + stored);
 }
 
@@ -610,7 +543,7 @@ __device__ __forceinline__ void stage_resampled_impl(const ClipCtx& c, const RsC
                                                      int j0, int T, int gtid) {
     const void* x = c.src;
     stage_slots(c, sb, ns, 0, 0, need, j0, T, gtid,
-                [&](int i) { return r.q ? rs_sample<PCM>(r, x, r.crop + i) : clip_sample<PCM>(x, i); });
+                [&](int i) { return r.g.q ? rs_sample<PCM>(r.g, x, r.len, r.crop + i) : clip_sample<PCM>(x, i); });
 }
 __device__ __noinline__ void stage_resampled_tile(const ClipCtx& c, const RsClip r, int pcm16, float* __restrict__ sb, int ns,
                                                   int need, int j0, int T, int gtid) {
@@ -637,11 +570,11 @@ __device__ __forceinline__ void load_clip(const KParams& p, int vclip, ClipCtx* 
     c->src = sample_addr<PCM16>(p.wave, off + crop);
     if (RESAMPLE) {   // overrides the lines above rather than replacing them: an if / else moved the register allocation of every other instantiation
         const RsClip r = rs_clip(p, clip);
-        long long start = off + (r.q ? 0 : r.crop);
+        long long start = off + (r.g.q ? 0 : r.crop);
         c->lc = r.lp < p.T ? static_cast<int>(r.lp) : p.T;
         if (p.first != nullptr) {   // lm_forward_spans: native sample k sits at wave[offset + k - first]
             const long long f = p.first[clip];
-            if (!span_stored(r.k0, r.o, r.q, r.width, r.nt4, r.len, r.crop, c->lc, p.T, f, p.stored[clip]))
+            if (!span_stored(r.g, r.len, r.crop, c->lc, p.T, f, p.stored[clip]))
                 c->lc = 0;   // a sample the staging needs is not stored: a zero-length clip, nothing is read
             start -= f;
         }

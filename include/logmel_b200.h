@@ -179,7 +179,10 @@ int lm_forward_host(lm_plan* plan, const float* wave, int64_t total_samples, con
  * AudioPreprocessor.load_audio (R/src/data/preprocessing.py:63-65): ICBHI ships 4, 10 and 44.1 kHz
  * recordings.  Mono; `in` / `out` are device pointers; out holds lm_resampler_out_len(r, in_len) =
  * ceil(new_freq * in_len / orig_freq) samples.  Float arithmetic: agrees with torchaudio to ~1e-6 of
- * full scale (torchaudio sums the same products as a dense conv1d, in another order).
+ * full scale (torchaudio sums the same products as a dense conv1d, in another order).  Each output is one fmaf
+ * chain over its phase's taps, zero-padded to a multiple of four, whichever kernel runs (shared-memory tiles, or one
+ * output per thread for rate pairs whose tile span is over 96 KB): the bits do not depend on the kernel, non-finite
+ * input included (a zero padding tap over inf or NaN gives NaN).
  */
 typedef struct lm_resampler lm_resampler;
 int lm_resampler_create(int32_t orig_freq, int32_t new_freq, int device, lm_resampler** r);
@@ -206,7 +209,8 @@ int lm_resample_rows(const lm_resampler* r, const float* in, int64_t in_len, int
  *               extra outputs.  normalize == 0 leaves dB (the input of lm_resize_finish).
  * Output is bit-identical to: y_i = lm_resample(resamplers[source[i]], clip i) (ceil(q len / o) samples), the y_i
  * packed, then lm_forward (fp32) with the same aug, noise and normalize -- pad or centre crop, roll, gain and noise
- * act on y_i.  A clip with source -1 gives exactly what lm_forward (fp32) or lm_forward_pcm16 (pcm16) gives.
+ * act on y_i -- for every rate pair and any samples, non-finite ones included: the staging runs lm_resample's chain.
+ * A clip with source -1 gives exactly what lm_forward (fp32) or lm_forward_pcm16 (pcm16) gives.
  * Returns LM_ERR_INVALID_ARG for NULL pointers or handles, a bad n_resamplers or pcm16, or a resampler on
  * another device.
  */

@@ -356,14 +356,20 @@ def test_transform_attributes_of_the_reference_class(golden):
     assert not hasattr(A.AudioPreprocessor(augment=False), "freq_mask")       # as in the reference: only with augment
 
 
-@pytest.mark.parametrize("sr", [44100, 4000, 10000, 22050, 48000])
+@pytest.mark.parametrize("sr", [44100, 4000, 10000, 22050, 48000, 384000])
 def test_tiled_resampler_is_bit_identical_to_the_plain_kernel(sr, monkeypatch):
-    """The shared-memory tiled resampler walks the same taps in the same order as the one-output-per-thread kernel."""
+    """The shared-memory tiled resampler and the one-output-per-thread kernel run the same chain over the same padded
+    taps, so they agree bit for bit, on non-finite samples too (a zero padding tap over inf gives NaN in both).  384 kHz
+    takes the plain kernel by default (its tiled span is over 96 KB)."""
     from audio_classification_icbhi_b200.resample import Resampler
     x = torch.from_numpy(np.random.RandomState(sr).standard_normal((3, 2 * sr + 123)).astype(np.float32) * 0.1)
+    x[0, [7, sr // 3, sr + 1]] = float("inf")
+    x[0, sr // 2] = float("nan")
+    x[2, [0, sr - 2, 2 * sr + 122]] = float("-inf")
     tiled = Resampler(sr, 16000)(x)
     monkeypatch.setenv("LM_RESAMPLE_UNTILED", "1")
     plain = Resampler(sr, 16000)(x)
-    assert tiled.shape == plain.shape and torch.equal(tiled, plain)
+    assert tiled.shape == plain.shape and torch.equal(tiled.view(torch.int32), plain.view(torch.int32))
+    assert not torch.isfinite(tiled[0]).all() and not torch.isfinite(tiled[2]).all()
     ref = O.resample(x[1].numpy(), sr, 16000)
     assert np.abs(tiled[1].cpu().numpy() - ref).max() < 2e-6

@@ -17,6 +17,7 @@ from oracle import logmel_oracle as O
 pytestmark = pytest.mark.gpu
 DEV = "cuda:0"
 RATES = [44100, 10000, 4000, 8000, 22050, 48000]
+UNTILED_RATE = 384000   # its tiled span (99.6 KB) is over 96 KB: lm_resample runs the one-output-per-thread kernel
 GUARD_F32 = 1.0e6      # fills the gaps between packed clips: a read outside a clip would show up in every feature
 GUARD_I16 = 32767
 
@@ -126,7 +127,7 @@ def test_rate_pairs_and_edge_lengths_equal_two_step(n_fft, hop, n_mels, pcm16):
     plan = get_plan(16000, n_fft, hop, n_mels)
     rs = np.random.RandomState(11)
     lengths, rates = [], []
-    for sr in RATES:
+    for sr in RATES + [UNTILED_RATE]:
         ls = edge_lengths(sr, 16000, plan.target_length)
         lengths += ls
         rates += [sr] * len(ls)

@@ -1,12 +1,13 @@
 #!/usr/bin/env python3
-"""GPU box: throughput of the polyphase resampler, 5 s clips at the ICBHI rates -> 16 kHz."""
+"""GPU box: throughput of the polyphase resampler, 5 s clips at the ICBHI rates -> 16 kHz, and at 384 kHz, a rate pair
+whose tiled span is over 96 KB: lm_resample runs the one-output-per-thread kernel there."""
 import os, sys
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 sys.path.insert(0, ROOT)
 import torch
 from audio_classification_icbhi_b200 import get_resampler
 dev = torch.device("cuda:0")
-for sr in (44100, 10000, 4000):
+for sr in (44100, 10000, 4000, 384000):
     r = get_resampler(sr, 16000, dev)
     B = 512
     x = torch.randn(B, 5 * sr, device=dev) * 0.1

@@ -6,7 +6,8 @@
 For every kernel of either file: whether its instructions are byte-identical, the instruction counts, the number of
 differing lines when they are not, and the register / stack / spill figures ptxas reports (cuobjdump -res-usage).
 Instruction lines are compared with their addresses and encodings stripped, so a function that only moved in the
-file still counts as identical."""
+file still counts as identical.  A kernel whose parameter list changed is paired with its namesake when each file has one
+function of that name."""
 from __future__ import annotations
 
 import re
@@ -62,9 +63,20 @@ def main(old: str, new: str) -> int:
     ra, rb = resources(old), resources(new)
     names = sorted(set(a) | set(b))
     pretty = demangle(names)
+    base = lambda n: pretty[n].split("(")[0]
+    renamed = {}   # new name -> old name of the same kernel with another parameter list
+    for n in set(b) - set(a):
+        old_n = [m for m in set(a) - set(b) if base(m) == base(n)]
+        if len(old_n) == 1 and sum(base(m) == base(n) for m in b) == 1:
+            renamed[n] = old_n[0]
     same = 0
     for n in names:
-        fa, fb = a.get(n), b.get(n)
+        if n in renamed.values():
+            continue
+        fa, fb = a.get(renamed.get(n, n)), b.get(n)
+        if n in renamed:
+            ra[n] = ra[renamed[n]]
+            print(f"parameters changed: {pretty[renamed[n]]} -> {pretty[n]}")
         reg = f"regs {ra.get(n, ('-', '-'))[0]} -> {rb.get(n, ('-', '-'))[0]}, stack {ra.get(n, ('-', '-'))[1]} -> {rb.get(n, ('-', '-'))[1]}"
         if fa is None or fb is None:
             print(f"{'only in new' if fa is None else 'only in old'}: {pretty[n]}  ({reg})")
@@ -76,7 +88,7 @@ def main(old: str, new: str) -> int:
         diff = sum(max(i2 - i1, j2 - j1) for tag, i1, i2, j1, j2 in SequenceMatcher(None, fa, fb, autojunk=False).get_opcodes()
                    if tag != "equal")
         print(f"DIFFERS ({len(fa)} -> {len(fb)} instructions, {diff} lines differ, {reg}): {pretty[n]}")
-    print(f"{same} of {len(names)} functions identical")
+    print(f"{same} of {len(names) - len(renamed)} functions identical")
     return 0
 
 
